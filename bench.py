@@ -4,6 +4,7 @@ TTML overlay blend (config 3: 3840x2160 NV12, two full-width cue regions, 32 fra
 launch), with the reference's CPU blend timed beside it.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config 3]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
       --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -66,6 +67,7 @@ import __graft_entry__ as graft  # noqa: E402
 DST_SETS = 4
 METRIC = "frames/sec, 4K NV12 TTML overlay blend"
 UNIT = "frames/s"
+DUMP_BYTES = 60 << 20       # --dump-outputs: the .npy files stay below 64 MB in all
 
 
 def load_peaks():
@@ -200,10 +202,9 @@ def config_record(cfg, wl, fmt, world):
 # ---------------------------------------------------------------------------
 # CPU legs (the only places bench.py touches oracle/)
 
-def cpu_reference_setup(cfg, wl, n_frames):
+def cpu_frames(cfg, wl, n_frames):
+    """n_frames fresh source frames, the same as the GPU arm's (frame i rolled by 16 i pixels)."""
     from oracle import oracle
-    lib = oracle.load(native=True, out_dir=tempfile.mkdtemp(prefix="ttmlblend_oracle_"))
-    ov = wl.overlay_for(cfg)
     base = wl.frame_for(cfg, 0)
     keep = []
     arr = (oracle.RefFrame * n_frames)()
@@ -211,6 +212,14 @@ def cpu_reference_setup(cfg, wl, n_frames):
         planes = [np.roll(p, i * 16, axis=1).copy() for p in base]
         keep.append(planes)
         arr[i] = oracle.make_frame(cfg.fmt, cfg.width, cfg.height, planes)
+    return arr, keep
+
+
+def cpu_reference_setup(cfg, wl, n_frames):
+    from oracle import oracle
+    lib = oracle.load(native=True, out_dir=tempfile.mkdtemp(prefix="ttmlblend_oracle_"))
+    ov = wl.overlay_for(cfg)
+    arr, keep = cpu_frames(cfg, wl, n_frames)
     rects = oracle.make_rectangles(oracle.ttmlrender_rectangles(ov))
     return lib, arr, rects, keep, ov
 
@@ -246,6 +255,27 @@ def run_cpu_baseline(cfg, wl, target_s=12.0):
                       f"-O3 -march=native, {cores} pthreads, {t:.1f} s"}
 
 
+def dump_rows(wl, shapes, n_frames):
+    """Row numbers kept per plane by --dump-outputs: every row when the float32 copy of all
+    frames fits DUMP_BYTES, else the same seeded sample of rows in every frame."""
+    total = 4 * n_frames * sum(r * c for r, c in shapes)
+    frac = min(1.0, DUMP_BYTES / total)
+    rows = []
+    for i, (r, _) in enumerate(shapes):
+        k = max(1, int(r * frac))
+        rows.append(np.sort(np.argsort(wl.splitmix64(0x64756D70 + i, r), kind="stable")[:k]))
+    return rows
+
+
+def dump_outputs(out_dir, frames, rows):
+    """frames: per frame, the `rows` (dump_rows) of its planes as the caller receives them.
+    Writes plane<i>.npy, float32 [frame, row, byte], and plane<i>_rows.npy (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for i, keep in enumerate(rows):
+        np.save(os.path.join(out_dir, f"plane{i}.npy"), np.stack([f[i] for f in frames]).astype(np.float32))
+        np.save(os.path.join(out_dir, f"plane{i}_rows.npy"), keep.astype(np.float64))
+
+
 def run_reference_arm(args, cfg, wl, world, rank, real_stdout):
     """--impl reference: the reference's CPU implementation of the path (oracle port; GStreamer
     cannot be installed here) on all host threads, 32 frames per step like the GPU arm. Rank 0 only."""
@@ -260,6 +290,13 @@ def run_reference_arm(args, cfg, wl, world, rank, real_stdout):
     for _ in range(args.steps):
         t += cpu_blend_fps(lib, arr, rects, per_step, cores)[1]
     fps = per_step * args.steps / t
+    if args.dump_outputs:
+        # the timed frames have been blended in place warmup + steps times; one blend of fresh
+        # frames is what a caller of one step receives (and what the GPU arm dumps)
+        arr, keep = cpu_frames(cfg, wl, per_step)
+        lib.tbref_blend_many(arr, per_step, rects, 1, cores)
+        rows = dump_rows(wl, [p.shape for p in keep[0]], len(keep))
+        dump_outputs(args.dump_outputs, [[p[k] for p, k in zip(f, rows)] for f in keep], rows)
     line = {
         "impl": "reference", "metric": METRIC if args.config == 3 else f"frames/sec, TTML overlay blend ({cfg.name})",
         "value": fps, "unit": UNIT, "n_gpus": args.gpus,
@@ -330,18 +367,31 @@ class DeviceWorkload:
         self.tb = ctx.Batch(ids, fmt, W, H, [s.c for s in self.srcs], [d.c for d in self.dsts])
         self.tb_inplace = ctx.Batch(ids, fmt, W, H, [s.c for s in self.srcs], [s.c for s in self.srcs])
 
+    # submit_many_repeat keeps ONE step counter per context across calls and workloads: step k of
+    # the context writes destination set k % dst_sets. Every call here goes through steps(),
+    # which keeps the same count per context.
+    repeats = {}
+
     def steps(self, n, inplace=False):
         """n steps, each one submit_many of the whole batch + flush, issued by a native loop."""
         self.ctx.submit_many_repeat(self.tb_inplace if inplace else self.tb, n)
+        DeviceWorkload.repeats[self.ctx] = DeviceWorkload.repeats.get(self.ctx, 0) + n
+
+    def last_outputs(self, rows):
+        """The destination frames of the context's latest step, `rows` of each plane kept; that
+        step must be one of this workload's out-of-place steps."""
+        ofs = (DeviceWorkload.repeats[self.ctx] - 1) % self.dst_sets * self.batch
+        return [[p[keep] for p, keep in zip(d.download(), rows)] for d in self.dsts[ofs:ofs + self.batch]]
 
     def release(self, keep_srcs=False):
         for f in self.dsts + ([] if keep_srcs else self.srcs):
             f.release()
 
 
-def timed_region(ctx, work, steps, dist, device, pairs, inplace=False):
+def timed_region(ctx, work, steps, dist, device, pairs, inplace=False, after=None):
     """K steps between barriers: (device ms, stats of the region). Afterwards, outside the timed
-    region, `pairs` more launches each between its own CUDA-event pair: the duration of one
+    region, `after()` if given (while the frames still hold the last step's results), then
+    `pairs` more launches each between its own CUDA-event pair: the duration of one
     launch running alone (a timed launch neither overlaps its predecessor's tail nor lets its
     successor overlap its own), the cross-check of the region's mean."""
     ctx.sync()
@@ -353,6 +403,8 @@ def timed_region(ctx, work, steps, dist, device, pairs, inplace=False):
     ctx.sync()
     barrier(dist, device)
     st = ctx.stats()
+    if after is not None:
+        after()
     if pairs:
         ctx.stats_reset()
         ctx.set_profiling(1)
@@ -434,7 +486,14 @@ def main():
     ap.add_argument("--event-pairs", type=int, default=12,
                     help="launches timed one by one with a CUDA-event pair AFTER the timed region "
                          "(cross-check of launch_ms)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the frames of the last step (rank 0's) to DIR as "
+                         "plane<i>.npy, float32 [frame, row, byte], with the row numbers kept in "
+                         "plane<i>_rows.npy: all rows, or the same seeded sample of rows in every frame "
+                         "when the frames would exceed 60 MB as float32")
     args = ap.parse_args()
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs needs --steps >= 1")
     args.warmup = max(args.warmup, 3)
     profile_every = args.event_pairs
 
@@ -472,7 +531,12 @@ def main():
         work.steps(max(1, args.warmup))
         ctx.sync()
         warm_extra += max(1, args.warmup)
-    ms, st = timed_region(ctx, work, args.steps, dist, device, profile_every)
+    dump = None
+    if args.dump_outputs and rank == 0:
+        def dump():
+            rows = dump_rows(wl, [(r, rb) for rb, r in pkg.ttmlblend.plane_layout(fmt, W, H)], batch)
+            dump_outputs(args.dump_outputs, work.last_outputs(rows), rows)
+    ms, st = timed_region(ctx, work, args.steps, dist, device, profile_every, after=dump)
     worst_ms = sh.reduce_max(ms, dist, device)
     records = sh.gather_records((batch * args.steps, ms, st["kernel_ms"], st["kernel_ms_launches"]), dist, device)
     value = sh.aggregate_fps(records)

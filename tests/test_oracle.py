@@ -385,19 +385,23 @@ def test_scaled_rectangles_in_a_composition(fmt):
 
 
 # ---------------------------------------------------------------------------------------------
-# oracle/_ref: the reference's own gstttmlblur.c, compiled from /root/reference
+# oracle/_ref: the reference's own gstttmlblur.c, compiled from the reference tree. That tree is
+# not part of this repository, so these tests run only where it has been built and skip elsewhere.
+
+KERNEL_CASES = [(0, 0.7), (1, 0.5), (2, 1.0), (3, 1.5), (5, 2.5), (8, 4.0), (12, 3.3), (20, 10.0), (32, 8.0)]
+BLUR_CASES = [(1, 1, 0.8), (2, 2, 1.0), (3, 4, 2.0), (4, 7, 3.0)]
 
 needs_ref = pytest.mark.skipif(oracle.load_ref() is None,
-                               reason="oracle/_ref not built (needs /root/reference: make -C oracle ref)")
+                               reason="oracle/_ref not built: needs the reference's plugins/ttml/gstttmlblur.c "
+                                      "(make -C oracle ref REFERENCE=<reference tree>)")
 
 
 @needs_ref
-@pytest.mark.parametrize("radius,sigma", [(0, 0.7), (1, 0.5), (2, 1.0), (3, 1.5), (5, 2.5), (8, 4.0), (12, 3.3),
-                                          (20, 10.0), (32, 8.0)])
+@pytest.mark.parametrize("radius,sigma", KERNEL_CASES)
 def test_gaussian_kernel_equals_the_references_own_code(radius, sigma):
     """The taps the reference's gst_ttml_blur_create_gaussian_kernel hands to pixman
-    (/root/reference/plugins/ttml/gstttmlblur.c:28-67, executed) against the oracle's
-    restatement: bit for bit, every tap, plus the two size parameters."""
+    (gstttmlblur.c:28-67, executed) against the oracle's restatement: bit for bit, every tap,
+    plus the two size parameters."""
     img = np.zeros((3, 3, 4), np.uint8)
     _, params = oracle.ref_blur_argb32(img, radius, sigma)
     size = 2 * radius + 1
@@ -407,7 +411,7 @@ def test_gaussian_kernel_equals_the_references_own_code(radius, sigma):
 
 
 @needs_ref
-@pytest.mark.parametrize("seed,radius,sigma", [(1, 1, 0.8), (2, 2, 1.0), (3, 4, 2.0), (4, 7, 3.0)])
+@pytest.mark.parametrize("seed,radius,sigma", BLUR_CASES)
 def test_blur_through_the_references_call_sequence(seed, radius, sigma):
     """gst_ttml_blur_image_surface as the reference wrote it (surface -> pixman image, filter,
     PIXMAN_OP_SRC onto a cleared image of the same stride, new surface) with the convolution
@@ -417,6 +421,77 @@ def test_blur_through_the_references_call_sequence(seed, radius, sigma):
     img = np.concatenate([(r.integers(0, 256, (37, 53, 3)) * a // 255).astype(np.uint8), a], axis=2)
     got, _ = oracle.ref_blur_argb32(img, radius, sigma)
     assert np.array_equal(got, oracle.blur_argb32(img, radius, sigma))
+
+
+# ---------------------------------------------------------------------------------------------
+# golden/blur_oracle.npz: the ORACLE's taps and blurred images for the cases above, frozen by hash.
+# Not the reference's values (those need oracle/_ref, above); what is checked here is that the
+# oracle does not drift, and that the frozen values agree with independent numpy restatements of
+# the documented formulas (the Gaussian of gstttmlblur.c, pixman's convolution filter).
+
+BLUR_ORACLE = np.load(os.path.join(GOLDEN, "blur_oracle.npz"))
+BLUR_ORACLE_SHA256 = "ff08a88542170433b70a9b2b6cf0f72d07d4e9e16f492f57d47fa2113522e00a"
+
+
+def _blur_oracle_sha():
+    h = hashlib.sha256()
+    for k in sorted(BLUR_ORACLE.files):
+        h.update(k.encode())
+        h.update(np.ascontiguousarray(BLUR_ORACLE[k]).tobytes())
+    return h.hexdigest()
+
+
+def _blur_oracle_case(key, case):
+    cases = [tuple(c) for c in BLUR_ORACLE[key].tolist()]
+    assert case in cases, (key, case)
+    return cases.index(case)
+
+
+def _numpy_convolve(img, taps):
+    """pixman's convolution filter restated: window [x-r, x+r] x [y-r, y+r], outside the image
+    transparent (REPEAT_NONE), 16.16 taps, (sum + 0x8000) >> 16, clipped to 0..255."""
+    size = taps.shape[0]
+    r = (size - 1) // 2
+    h, w = img.shape[:2]
+    pad = np.zeros((h + 2 * r, w + 2 * r, 4), np.int64)
+    pad[r:r + h, r:r + w] = img
+    tot = np.zeros((h, w, 4), np.int64)
+    for i in range(size):
+        for j in range(size):
+            tot += int(taps[i, j]) * pad[i:i + h, j:j + w]
+    return np.clip((tot + 0x8000) >> 16, 0, 255).astype(np.uint8)
+
+
+def test_blur_oracle_vectors_are_frozen():
+    assert str(BLUR_ORACLE["source"]).startswith("oracle/ttmlblend_ref.c")
+    assert _blur_oracle_sha() == BLUR_ORACLE_SHA256
+
+
+@pytest.mark.parametrize("radius,sigma", KERNEL_CASES)
+def test_gaussian_kernel_matches_frozen_oracle_taps(radius, sigma):
+    """tbref_gaussian_kernel equals its frozen taps bit for bit; the frozen taps are the
+    normalised 2-D Gaussian in truncated 16.16 computed with numpy (up to the last ulp of exp())."""
+    import math
+    want = BLUR_ORACLE[f"taps{_blur_oracle_case('kernel_cases', (radius, sigma))}"].astype(np.int64)
+    size = 2 * radius + 1
+    assert want.shape == (size * size,)
+    assert np.array_equal(oracle.gaussian_kernel(radius, sigma).astype(np.int64).ravel(), want)
+    g = np.array([[math.exp(-(x * x + y * y) / (2 * sigma * sigma)) for y in range(-radius, radius + 1)]
+                  for x in range(-radius, radius + 1)])
+    assert np.abs(np.floor(g / g.sum() * 65536.0).astype(np.int64).ravel() - want).max() <= 1
+
+
+@pytest.mark.parametrize("seed,radius,sigma", BLUR_CASES)
+def test_blur_matches_frozen_oracle_images(seed, radius, sigma):
+    """tbref_blur_argb32 equals its frozen output bit for bit; the frozen output is the frozen
+    input convolved with the frozen taps by the numpy restatement of pixman's filter."""
+    k = _blur_oracle_case("blur_cases", (seed, radius, sigma))
+    img, taps, want = BLUR_ORACLE[f"blur_in{k}"], BLUR_ORACLE[f"blur_taps{k}"], BLUR_ORACLE[f"blur_out{k}"]
+    size = 2 * radius + 1
+    assert img.shape == want.shape == (37, 53, 4) and taps.shape == (size * size,)
+    assert np.array_equal(oracle.blur_argb32(img, radius, sigma), want)
+    assert np.array_equal(oracle.gaussian_kernel(radius, sigma).ravel(), taps)
+    assert np.array_equal(_numpy_convolve(img, taps.reshape(size, size)), want)
 
 
 @pytest.mark.parametrize("seed", range(24))
