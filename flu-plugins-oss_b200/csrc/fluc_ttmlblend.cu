@@ -151,12 +151,6 @@ destroy_cuda_objects (Ctx *c)
     if (e) { cudaEventDestroy (e); e = nullptr; }
   for (cudaEvent_t *e : { &c->timer0, &c->timer1 })
     if (*e) { cudaEventDestroy (*e); *e = nullptr; }
-  for (int i = 0; i < kLanes; i++) {
-    if (c->lanes[i].done) cudaEventDestroy (c->lanes[i].done);
-    if (c->lanes[i].stream) cudaStreamDestroy (c->lanes[i].stream);
-    c->lanes[i].done = nullptr;
-    c->lanes[i].stream = nullptr;
-  }
   for (cudaStream_t *st : { &c->blend_stream, &c->up_stream, &c->reaper, &c->table_stream, &c->dma_in, &c->dma_out })
     if (*st) { cudaStreamDestroy (*st); *st = nullptr; }
   if (c->mem_pool) { cudaMemPoolDestroy (c->mem_pool); c->mem_pool = nullptr; }
@@ -200,13 +194,8 @@ fluc_ttmlblend_new (int device, FlucTtmlBlend **out)
   ok &= cudaStreamCreateWithFlags (&c->table_stream, cudaStreamNonBlocking) == cudaSuccess;
   for (int i = 0; i < kDmaSets && ok; i++)
     ok &= cudaEventCreateWithFlags (&c->dma_sets[i].done, cudaEventDisableTiming) == cudaSuccess;
-  for (int i = 0; i < kLanes + 2 && ok; i++)
+  for (int i = 0; i < 2 && ok; i++)
     ok &= cudaEventCreateWithFlags (&c->ev_fence[i], cudaEventDisableTiming) == cudaSuccess;
-  for (int i = 0; i < kLanes && ok; i++) {
-    ok &= cudaStreamCreateWithFlags (&c->lanes[i].stream, cudaStreamNonBlocking) == cudaSuccess;
-    ok &= cudaEventCreateWithFlags (&c->lanes[i].done,
-        cudaEventDisableTiming | (c->blocking_sync ? cudaEventBlockingSync : 0)) == cudaSuccess;
-  }
   ok &= cudaEventCreate (&c->timer0) == cudaSuccess;
   ok &= cudaEventCreate (&c->timer1) == cudaSuccess;
   if (ok) {
@@ -251,13 +240,11 @@ fluc_ttmlblend_new (int device, FlucTtmlBlend **out)
     c->dma_piece = (uint32_t) std::max (0, std::min (1024, atoi (e)));
   c->stage_threads = (int) std::max (2u, std::min (12u, std::thread::hardware_concurrency () * 3 / 4));
   if ((e = getenv ("FLUC_TTMLBLEND_STAGE_THREADS")))
-    c->stage_threads = std::max (0, std::min (64, atoi (e)));
+    c->stage_threads = std::max (1, std::min (64, atoi (e)));
   if ((e = getenv ("FLUC_TTMLBLEND_STAGE_SLOTS")))
     c->stage_slots_max = std::max (1, std::min (4096, atoi (e)));
   if ((e = getenv ("FLUC_TTMLBLEND_AUTO_REGISTER")))
     c->auto_register = atoi (e) != 0;
-  if ((e = getenv ("FLUC_TTMLBLEND_HOST_MODE")))
-    c->host_mode = std::max (0, std::min (2, atoi (e)));
   if ((e = getenv ("FLUC_TTMLBLEND_LINGER_US")))
     c->linger_us = (uint32_t) std::max (0, atoi (e));
   find_numa_cpus (c);
@@ -296,8 +283,6 @@ fluc_ttmlblend_free (FlucTtmlBlend *thiz)
   /* our own streams only: other users of the device are none of our business */
   for (cudaStream_t st : { c->blend_stream, c->up_stream, c->table_stream, c->dma_in, c->dma_out })
     cudaStreamSynchronize (st);
-  for (int i = 0; i < kLanes; i++)
-    cudaStreamSynchronize (c->lanes[i].stream);
   {
     std::unique_lock<std::mutex> lk (c->mu);
     c->pending.clear ();
@@ -307,8 +292,6 @@ fluc_ttmlblend_free (FlucTtmlBlend *thiz)
       cudaEventDestroy (b.done);
     }
     c->batches.clear ();
-    for (int i = 0; i < kLanes; i++)
-      c->lanes[i].keep.reset ();
     c->overlays.clear ();       /* frees through the reaper stream */
     cudaStreamSynchronize (c->reaper);
     for (auto e : c->event_pool)
@@ -325,11 +308,6 @@ fluc_ttmlblend_free (FlucTtmlBlend *thiz)
     };
     for (auto &s : c->slots)
       free_slot (s);
-    for (int i = 0; i < kLanes; i++) {
-      free_slot (c->lanes[i].table[0]);
-      free_slot (c->lanes[i].table[1]);
-      if (c->lanes[i].dev) cudaFree (c->lanes[i].dev);
-    }
     stage_free_slots (c);
     for (auto &p : c->pool_free)
       if (!p.in_slab) {
@@ -600,29 +578,6 @@ fluc_ttmlblend_wait (FlucTtmlBlend *thiz, uint64_t ticket)
   int staged_rc = 0;
   if (stage_wait (c, lk, ticket, &staged_rc))
     return staged_rc;
-  auto lt = c->lane_tickets.find (ticket);
-  if (lt != c->lane_tickets.end ()) {
-    Lane &l = c->lanes[lt->second];
-    cudaEvent_t ev = l.done;
-    lk.unlock ();
-    cudaError_t e = cudaEventSynchronize (ev);
-    lk.lock ();
-    if (e != cudaSuccess) {
-      c->sticky = FLUC_TTMLBLEND_ERROR_CUDA;
-      c->cuda_error = std::string ("wait: ") + cudaGetErrorString (e);
-      return c->sticky;
-    }
-    auto again = c->lane_tickets.find (ticket);
-    if (again != c->lane_tickets.end ()) {
-      Lane &l2 = c->lanes[again->second];
-      if (l2.ticket == ticket) {
-        l2.busy = false;
-        l2.keep.reset ();
-      }
-      c->lane_tickets.erase (again);
-    }
-    return 0;
-  }
   if (!c->pending.empty () && ticket >= c->pending.front ().ticket) {
     /* The frame has not been launched yet. A lone stream launches now (lowest latency). When
      * several streams are active -- many elements calling blend + wait from their own
@@ -684,25 +639,12 @@ fluc_ttmlblend_sync (FlucTtmlBlend *thiz)
     return rc;
   /* what is in flight now, then wait for it with the context unlocked: other threads keep
    * submitting frames and changing cues meanwhile (their work is not waited for) */
-  uint64_t lane_ticket[kLanes];
-  bool lane_busy[kLanes];
-  for (int i = 0; i < kLanes; i++) {
-    lane_ticket[i] = c->lanes[i].ticket;
-    lane_busy[i] = c->lanes[i].busy;
-  }
-  cudaEvent_t ev[kLanes + 3];
+  const cudaStream_t streams[3] = { c->blend_stream, c->up_stream, c->dma_out };
+  cudaEvent_t ev[3];
   int n_ev = 0;
-  cudaStream_t streams[kLanes + 3];
-  int n_streams = 0;
-  streams[n_streams++] = c->blend_stream;
-  streams[n_streams++] = c->up_stream;
-  streams[n_streams++] = c->dma_out;
-  for (int i = 0; i < kLanes; i++)
-    if (lane_busy[i])
-      streams[n_streams++] = c->lanes[i].stream;
-  for (int i = 0; i < n_streams; i++) {
+  for (cudaStream_t st : streams) {
     cudaEvent_t e = event_get (c);
-    CU (c, cudaEventRecord (e, streams[i]));
+    CU (c, cudaEventRecord (e, st));
     ev[n_ev++] = e;
   }
   lk.unlock ();
@@ -719,12 +661,6 @@ fluc_ttmlblend_sync (FlucTtmlBlend *thiz)
     c->cuda_error = std::string ("sync: ") + cudaGetErrorString (err);
     return c->sticky;
   }
-  for (int i = 0; i < kLanes; i++)
-    if (lane_busy[i] && c->lanes[i].busy && c->lanes[i].ticket == lane_ticket[i]) {
-      c->lanes[i].busy = false;
-      c->lanes[i].keep.reset ();
-      c->lane_tickets.erase (lane_ticket[i]);
-    }
   reap_batches (c);
   stage_drain (c, lk, 1);       /* ... and has been copied back into the caller's frame */
   return c->sticky;
@@ -746,7 +682,7 @@ fluc_ttmlblend_set_batch (FlucTtmlBlend *thiz, uint32_t max_frames, uint32_t lin
 /* ---- host-resident frames -------------------------------------------- */
 
 /* Everything of ours that may still touch host memory has finished: queued frames launched,
- * blend stream and staging lanes drained. Needed before a registration goes away. */
+ * blend stream and host DMA copy streams drained. Needed before a registration goes away. */
 static void
 drain_host_users (Ctx *c)
 {
@@ -754,8 +690,6 @@ drain_host_users (Ctx *c)
   cudaStreamSynchronize (c->blend_stream);
   cudaStreamSynchronize (c->dma_in);
   cudaStreamSynchronize (c->dma_out);
-  for (int i = 0; i < kLanes; i++)
-    cudaStreamSynchronize (c->lanes[i].stream);
 }
 
 /* How many automatic plane registrations are kept: a pool's worth of buffers (16) times three
@@ -874,14 +808,6 @@ tbh::queue_mapped_frame (Ctx *c, uint64_t tk, uint32_t stream, const std::shared
   f.host_hi = xz.hull_hi ();
   if ((rc = order_against_pending (c, xz, xz, true)))
     return rc;
-  /* the same buffer still on its way through a staging lane (it was not device-accessible a
-   * moment ago): the blend stream waits for that lane */
-  for (int i = 0; i < kLanes; i++)
-    if (c->lanes[i].busy && xh.hull_lo () < c->lanes[i].host_hi && c->lanes[i].host_lo < xh.hull_hi ())
-    {
-      CU (c, cudaStreamWaitEvent (c->blend_stream, c->lanes[i].done, 0));
-      c->blend_stream_waits = true;
-    }
   f.layout = find_layout (c, prep, ov->lazy_inplace, fmt, W, H, frame_flags, &zf, &zf, true);
   for (int pl = 0; pl < 3; pl++) {
     f.src[pl] = static_cast<const uint8_t *> (zf.plane[pl]);
@@ -933,10 +859,10 @@ blend_host_locked (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, in
   /* Is the host frame device-accessible (pool frame / host_register)? Then the
    * kernel can reach it over PCIe itself. */
   const int n_planes = format_planes (fmt);
-  if (c->auto_register && c->host_mode != HM_STAGED)
+  if (c->auto_register)
     auto_register_frame (c, stream, fmt, W, H, hf);
   FlucTtmlBlendFrame zf = {};
-  bool mapped = c->host_mode != HM_STAGED;
+  bool mapped = true;
   for (int pl = 0; pl < n_planes && mapped; pl++) {
     /* pinned pool frames are known (cudaHostAlloc under UVA: device pointer == host pointer):
      * no driver call per plane per frame for them */
@@ -973,132 +899,19 @@ blend_host_locked (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, in
       zf.plane[pl] = attr.devicePointer;
       zf.stride[pl] = hf->stride[pl];
       /* byte-granular accesses to host memory would each cross PCIe: frames that are not
-       * 16-byte aligned go through the staging lanes (DMA, then the vector kernel) instead */
+       * 16-byte aligned go through the staging threads (copies into an aligned pinned frame) instead */
       if ((((uintptr_t) zf.plane[pl] | (uintptr_t) zf.stride[pl]) & 15u) != 0)
         mapped = false;
     }
   }
 
-  if (mapped && c->host_mode == HM_ZEROCOPY)
+  if (mapped)
     return queue_mapped_frame (c, tk, stream, ov, prep, fmt, W, H, frame_flags, &zf, hf);
 
   /* Not device-accessible (ordinary pageable memory, or not 16-byte aligned): worker threads copy
    * the rows under the cue into a pinned staging frame, that frame is blended zero copy like
    * any other, and the rows are copied back (staging.cu). */
-  if (c->host_mode == HM_ZEROCOPY && c->stage_threads > 0)
-    return stage_frame (c, lk, tk, stream, ov, prep, fmt, W, H, frame_flags, hf);
-
-  Lane &l = c->lanes[c->next_lane];
-  const int lane_idx = c->next_lane;
-  c->next_lane = (c->next_lane + 1) % kLanes;
-  if (l.busy) {
-    CU (c, cudaEventSynchronize (l.done));
-    c->lane_tickets.erase (l.ticket);
-    l.busy = false;
-    l.keep.reset ();
-  }
-  /* Ordering against other work on the same host buffer: two overlays on one frame through two
-   * lanes, or a zero-copy frame of this buffer that is queued or still running. */
-  const FrameExtent xh (fmt, W, H, hf);
-  const uintptr_t hull_lo = xh.hull_lo (), hull_hi = xh.hull_hi ();
-  if (xh.hits (c->pending_dst) && (rc = launch_pending (c)))
-    return rc;
-  if (xh.hits (c->inflight_host) && !c->batches.empty ())
-    CU (c, cudaStreamWaitEvent (l.stream, c->batches.back ().done, 0));
-  for (int i = 0; i < kLanes; i++)
-    if (i != lane_idx && c->lanes[i].busy && hull_lo < c->lanes[i].host_hi && c->lanes[i].host_lo < hull_hi)
-      CU (c, cudaStreamWaitEvent (l.stream, c->lanes[i].done, 0));
-
-  /* device staging frame: same strides as a pool frame */
-  FlucTtmlBlendFrame df = {};
-  size_t off = 0;
-  size_t plane_off[3];
-  for (int pl = 0; pl < n_planes; pl++) {
-    df.stride[pl] = (int32_t) align_up ((size_t) plane_row_bytes (fmt, pl, W), 256);
-    plane_off[pl] = off;
-    off += (size_t) df.stride[pl] * plane_rows (fmt, pl, H);
-  }
-  if ((rc = lane_reserve (c, l, off)))
-    return rc;
-  for (int pl = 0; pl < n_planes; pl++)
-    df.plane[pl] = l.dev + plane_off[pl];
-
-  /* HM_WRITEBACK: the copy engine brings the rows in, the kernel stores the
-   * result straight into the host frame (posted PCIe writes), no copy back */
-  const bool writeback = mapped && c->host_mode == HM_WRITEBACK;
-  std::vector<PlaneJob> jobs;
-  const uint64_t algo = build_jobs (fmt, W, H, frame_flags, &df, writeback ? &zf : &df, prep, true, jobs);
-  if (jobs.empty ())
-    return 0;
-  CU (c, cudaStreamWaitEvent (l.stream, prep->ready, 0));
-
-  /* rows each window touches: host -> device. Bands that are neighbours in y
-   * with the same byte range merge into one copy. */
-  struct Span { int pl, b0, nb, y0, rows; };
-  std::vector<Span> spans;
-  for (const PlaneJob &j : jobs) {
-    Span s;
-    s.pl = j.plane;
-    s.b0 = j.win_v0 * 16;
-    s.nb = std::min (j.win_nv * 16, j.row_bytes - s.b0);
-    s.y0 = j.win_y0;
-    s.rows = j.win_rows;
-    bool merged = false;
-    for (Span &o : spans)
-      if (o.pl == s.pl && o.b0 == s.b0 && o.nb == s.nb && o.y0 + o.rows == s.y0) {
-        o.rows += s.rows;
-        merged = true;
-        break;
-      }
-    if (!merged)
-      spans.push_back (s);
-  }
-  auto copy_span = [&](const Span &s, bool to_device) -> cudaError_t {
-    uint8_t *d = static_cast<uint8_t *> (df.plane[s.pl]) + (size_t) s.y0 * df.stride[s.pl] + s.b0;
-    uint8_t *h = static_cast<uint8_t *> (hf->plane[s.pl]) + (size_t) s.y0 * hf->stride[s.pl] + s.b0;
-    if (s.nb == df.stride[s.pl] && s.nb == hf->stride[s.pl]) {
-      /* full rows, equal strides: one linear copy */
-      return to_device ?
-          cudaMemcpyAsync (d, h, (size_t) s.nb * s.rows, cudaMemcpyHostToDevice, l.stream) :
-          cudaMemcpyAsync (h, d, (size_t) s.nb * s.rows, cudaMemcpyDeviceToHost, l.stream);
-    }
-    return to_device ?
-        cudaMemcpy2DAsync (d, df.stride[s.pl], h, hf->stride[s.pl], s.nb, s.rows,
-            cudaMemcpyHostToDevice, l.stream) :
-        cudaMemcpy2DAsync (h, hf->stride[s.pl], d, df.stride[s.pl], s.nb, s.rows,
-            cudaMemcpyDeviceToHost, l.stream);
-  };
-  for (const Span &s : spans) {
-    CU (c, copy_span (s, true));
-    c->stats.h2d_bytes += (uint64_t) s.nb * s.rows;
-  }
-  {
-    std::vector<PlaneJob> grp[2];
-    for (const PlaneJob &j : jobs)
-      grp[(j.flags & JF_FAST) ? 1 : 0].push_back (j);
-    for (int g = 0; g < 2; g++)
-      if (!grp[g].empty ()) {
-        if ((rc = launch_jobs (c, l.table[g], grp[g].data (), grp[g].size (), plane_kind (fmt),
-                    g == 1, 0, l.stream)))
-          return rc;
-      }
-  }
-  for (const Span &s : spans) {
-    if (!writeback)
-      CU (c, copy_span (s, false));
-    c->stats.d2h_bytes += (uint64_t) s.nb * s.rows;
-  }
-  CU (c, cudaEventRecord (l.done, l.stream));
-  l.busy = true;
-  l.ticket = tk;
-  l.host_lo = hull_lo;
-  l.host_hi = hull_hi;
-  l.keep = ov;
-  c->lane_tickets[tk] = lane_idx;
-  c->stats.frames_blended++;
-  c->stats.staged_frames++;
-  c->stats.algorithmic_bytes += algo;
-  return 0;
+  return stage_frame (c, lk, tk, stream, ov, prep, fmt, W, H, frame_flags, hf);
 }
 
 int
@@ -1597,72 +1410,6 @@ int
 fluc_ttmlblend_pcie_probe (FlucTtmlBlend *thiz, int mode, size_t bytes, double seconds, double *gbs)
 {
   ENTER (thiz);
-  if (mode >= 2 && mode <= 5) {
-    /* diagnostic: the DMA-batch pipeline shape (copy-in stream, blend stream, copy-out stream, three
-     * device sets, 2-D copies) with buffers of its own, on this context's streams (mode 2) or on
-     * fresh ones (mode 3) */
-    int rc0 = launch_pending (c);
-    if (rc0)
-      return rc0;
-    /* modes 4, 5: whole 4K NV12 frames 12.4 MB apart, the pieces where the cue rows are; 5: the
-     * copy-out lands in pool frames */
-    const bool wide = mode >= 4;
-    const size_t piece[4] = { 1382400, 552960, 691200, 276480 }, fb = wide ? 12441600 : 2903040;
-    const size_t yoff_w[4] = { (size_t) 1728 * 3840, (size_t) 72 * 3840, (size_t) 3840 * 2160 + (size_t) 864 * 3840,
-      (size_t) 3840 * 2160 + (size_t) 36 * 3840 };
-    const size_t yoff_n[4] = { 0, 1382400, 1382400 + 552960, 1382400 + 552960 + 691200 };
-    const size_t *yoff = wide ? yoff_w : yoff_n;
-    const size_t total = fb * 32;
-    uint8_t *h[2] = { nullptr, nullptr }, *d[3] = { nullptr, nullptr, nullptr };
-    for (auto &p : h) { cudaHostAlloc ((void **) &p, total, cudaHostAllocDefault); memset (p, 1, total); }
-    for (auto &p : d) cudaMalloc ((void **) &p, total);
-    cudaStream_t s1 = c->dma_in, s2 = c->dma_out, s3 = c->blend_stream;
-    if (mode == 3) {
-      cudaStreamCreateWithFlags (&s1, cudaStreamNonBlocking);
-      cudaStreamCreateWithFlags (&s2, cudaStreamNonBlocking);
-      cudaStreamCreateWithFlags (&s3, cudaStreamNonBlocking);
-    }
-    cudaEvent_t ein[4], ek[4], done[4], setdone[3];
-    for (auto &e : ein) cudaEventCreateWithFlags (&e, cudaEventDisableTiming);
-    for (auto &e : ek) cudaEventCreateWithFlags (&e, cudaEventDisableTiming);
-    for (auto &e : done) cudaEventCreateWithFlags (&e, cudaEventDisableTiming);
-    for (auto &e : setdone) cudaEventCreateWithFlags (&e, cudaEventDisableTiming);
-    lk.unlock ();
-    auto batch = [&](int i) {
-      uint8_t *hh = h[i & 1], *dd = d[i % 3];
-      if (i >= 3) cudaStreamWaitEvent (s1, setdone[i % 3], 0);
-      for (int k = 0; k < 4; k++)
-        cudaMemcpy2DAsync (dd + yoff[k], fb, hh + yoff[k], fb, piece[k], 32, cudaMemcpyHostToDevice, s1);
-      cudaEventRecord (ein[i & 3], s1);
-      cudaStreamWaitEvent (s3, ein[i & 3], 0);
-      launch_pcie_probe (dd, wide ? total / 4 : total, s3);
-      cudaEventRecord (ek[i & 3], s3);
-      cudaStreamWaitEvent (s2, ek[i & 3], 0);
-      for (int k = 0; k < 4; k++)
-        cudaMemcpy2DAsync (hh + yoff[k], fb, dd + yoff[k], fb, piece[k], 32, cudaMemcpyDeviceToHost, s2);
-      cudaEventRecord (setdone[i % 3], s2);
-      cudaEventRecord (done[i & 3], s2);
-    };
-    for (int i = 0; i < 4; i++) { batch (i); if (i) cudaEventSynchronize (done[(i - 1) & 3]); }
-    cudaStreamSynchronize (s2);
-    const auto t0 = std::chrono::steady_clock::now ();
-    int i = 4, n = 0;
-    double t = 0;
-    do {
-      batch (i);
-      cudaEventSynchronize (done[(i - 1) & 3]);
-      i++; n++;
-      t = std::chrono::duration<double> (std::chrono::steady_clock::now () - t0).count ();
-    } while (t < seconds);
-    cudaStreamSynchronize (s2);
-    t = std::chrono::duration<double> (std::chrono::steady_clock::now () - t0).count ();
-    lk.lock ();
-    if (gbs)
-      *gbs = 92897280.0 * n / t / 1e9;
-    for (auto &p : h) cudaFreeHost (p);
-    for (auto &p : d) cudaFree (p);
-    return cudaGetLastError () == cudaSuccess ? 0 : FLUC_TTMLBLEND_ERROR_CUDA;
-  }
   if (mode < 0 || mode > 1 || bytes < 4096 || bytes > ((size_t) 1 << 31) || !(seconds > 0.0) || seconds > 10.0)
     return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
   bytes &= ~(size_t) 4095;
@@ -1670,7 +1417,8 @@ fluc_ttmlblend_pcie_probe (FlucTtmlBlend *thiz, int mode, size_t bytes, double s
   if (rc)
     return rc;
   /* buffers of its own, nothing shared with frames in flight; the context stays unlocked while
-   * the probe runs (it touches only these buffers and two lane streams that are drained first) */
+   * the probe runs (it touches only these buffers and the two copy streams of host DMA batches,
+   * drained first) */
   uint8_t *h_in = nullptr, *h_out = nullptr, *d_in = nullptr, *d_out = nullptr;
   auto cleanup = [&]() {
     if (h_in) cudaFreeHost (h_in);
@@ -1690,7 +1438,7 @@ fluc_ttmlblend_pcie_probe (FlucTtmlBlend *thiz, int mode, size_t bytes, double s
   }
   memset (h_in, 0x5a, bytes);
   memset (h_out, 0xa5, bytes);
-  cudaStream_t s1 = c->lanes[0].stream, s2 = c->lanes[1].stream;
+  cudaStream_t s1 = c->dma_in, s2 = c->dma_out;
   cudaStreamSynchronize (s1);
   cudaStreamSynchronize (s2);
   lk.unlock ();

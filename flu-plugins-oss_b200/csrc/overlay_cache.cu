@@ -16,13 +16,8 @@ free_deferred (Ctx *c, const std::vector<void *> &ptrs)
 {
   if (ptrs.empty ())
     return;
-  cudaStream_t all[kLanes + 2];
-  int n = 0;
-  all[n++] = c->blend_stream;
-  all[n++] = c->up_stream;
-  for (int i = 0; i < kLanes; i++)
-    all[n++] = c->lanes[i].stream;
-  for (int i = 0; i < n; i++) {
+  const cudaStream_t all[2] = { c->blend_stream, c->up_stream };
+  for (int i = 0; i < 2; i++) {
     if (!all[i])
       continue;
     cudaEventRecord (c->ev_fence[i], all[i]);

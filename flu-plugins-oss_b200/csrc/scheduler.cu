@@ -50,8 +50,7 @@ slot_reserve (Ctx *c, TableSlot &s, size_t n, size_t words)
  * array holds the first chunk of every job, then the coarse index (job of every
  * 2^kCoarseShift-th chunk) the kernel starts its search from. */
 int
-launch_jobs (Ctx *c, TableSlot &s, const PlaneJob *jobs, size_t n, int kind, bool fast, int sync,
-    cudaStream_t stream)
+launch_jobs (Ctx *c, TableSlot &s, const PlaneJob *jobs, size_t n, int kind, bool fast, int sync)
 {
   if (n == 0)
     return 0;
@@ -77,14 +76,14 @@ launch_jobs (Ctx *c, TableSlot &s, const PlaneJob *jobs, size_t n, int kind, boo
       coarse[next] = (uint32_t) i;
   }
   /* the table goes up on the copy stream, so that it overlaps the kernel still
-   * running on `stream`; the slot is free (its last kernel waited on above) */
+   * running on the blend stream; the slot is free (its last kernel waited on above) */
   CU (c, cudaMemcpyAsync (s.d_jobs, s.h_jobs, n * sizeof (PlaneJob), cudaMemcpyHostToDevice, c->table_stream));
   CU (c, cudaMemcpyAsync (s.d_begin, s.h_begin, (n + n_coarse) * sizeof (uint32_t), cudaMemcpyHostToDevice,
           c->table_stream));
   CU (c, cudaEventRecord (s.uploaded, c->table_stream));
-  CU (c, cudaStreamWaitEvent (stream, s.uploaded, 0));
-  CU (c, launch_blend (s.d_jobs, s.d_begin, s.d_begin + n, (int) n, total, kind, fast, sync, stream));
-  CU (c, cudaEventRecord (s.copied, stream));    /* slot busy until this kernel is done */
+  CU (c, cudaStreamWaitEvent (c->blend_stream, s.uploaded, 0));
+  CU (c, launch_blend (s.d_jobs, s.d_begin, s.d_begin + n, (int) n, total, kind, fast, sync, c->blend_stream));
+  CU (c, cudaEventRecord (s.copied, c->blend_stream));    /* slot busy until this kernel is done */
   c->stats.launches++;
   return 0;
 }
@@ -511,7 +510,7 @@ launch_pending (Ctx *c)
     if (!dep)
       dep = sets_overlap (c->pending_dst, c->inflight_dst) || sets_overlap (c->pending_dst, c->inflight_src) ||
           sets_overlap (c->pending_src, c->inflight_dst);
-    /* Behind a stream wait (a new cue's prepare, a staging lane, the copies of a DMA batch) the
+    /* Behind a stream wait (a new cue's prepare, the copies of a DMA batch) the
      * launch goes out as an ordinary one: a programmatic launch behind a stream wait holds back
      * the completion of what was recorded before the wait (measured: the copy-out gated by an
      * event after kernel i did not start until the copy-in kernel i+1 waits for had finished).
@@ -629,8 +628,7 @@ launch_pending (Ctx *c)
         continue;
       TableSlot &s = c->slots[c->next_slot];
       c->next_slot = (c->next_slot + 1) % kTableSlots;
-      int rc = launch_jobs (c, s, by_kind[k].data (), by_kind[k].size (), k / 2, (k & 1) != 0, sync,
-          c->blend_stream);
+      int rc = launch_jobs (c, s, by_kind[k].data (), by_kind[k].size (), k / 2, (k & 1) != 0, sync);
       if (rc)
         return rc;
       sync &= ~JF_DEP;
@@ -706,20 +704,6 @@ scheduler_main (Ctx *c)
       c->cv.wait_until (lk, deadline);
     }
   }
-}
-
-int
-lane_reserve (Ctx *c, Lane &l, size_t bytes)
-{
-  if (l.dev_bytes >= bytes)
-    return 0;
-  if (l.dev)
-    CU (c, cudaFree (l.dev));
-  l.dev = nullptr;
-  l.dev_bytes = 0;
-  CU (c, cudaMalloc ((void **) &l.dev, bytes));
-  l.dev_bytes = bytes;
-  return 0;
 }
 
 }  // namespace tbh

@@ -478,18 +478,6 @@ struct PoolEntry {
   FlucTtmlBlendFrame frame;
 };
 
-struct Lane {
-  cudaStream_t stream = nullptr;
-  cudaEvent_t done = nullptr;
-  uint64_t ticket = 0;
-  bool busy = false;
-  uintptr_t host_lo = 0, host_hi = 0;  /* the host frame in flight (hull of its planes) */
-  uint8_t *dev = nullptr;
-  size_t dev_bytes = 0;
-  TableSlot table[2];
-  std::shared_ptr<Overlay> keep;
-};
-
 /* ---- staged host frames (staging.cu) ---- */
 struct StageJob {
   enum State { COPY_IN, ON_GPU, COPY_OUT, DONE };
@@ -508,10 +496,6 @@ struct StageJob {
   int rc = 0;
 };
 
-/* How blend_host moves a device-accessible (pinned) host frame. */
-enum HostMode { HM_STAGED = 0, HM_ZEROCOPY = 1, HM_WRITEBACK = 2 };
-
-constexpr int kLanes = 4;
 constexpr int kTableSlots = 8;
 
 struct Ctx {
@@ -528,7 +512,7 @@ struct Ctx {
 
   cudaStream_t blend_stream = nullptr, up_stream = nullptr, reaper = nullptr, table_stream = nullptr;
   cudaMemPool_t mem_pool = nullptr;    /* stream-ordered allocations of the overlay cache */
-  cudaEvent_t ev_fence[kLanes + 2] = {};
+  cudaEvent_t ev_fence[2] = {};        /* free_deferred: blend_stream, up_stream */
   cudaEvent_t timer0 = nullptr, timer1 = nullptr;
 
   std::unordered_map<uint32_t, std::shared_ptr<Overlay>> overlays;
@@ -576,7 +560,6 @@ struct Ctx {
   int next_slot = 0;
 
   uint32_t max_batch = 32, linger_us = 200;
-  int host_mode = HM_ZEROCOPY;
   bool auto_register = false;          /* pin pageable host frames on first sight (opt-in) */
   /* automatic registrations by first byte: [lo, hi) and when it was last used. At most
    * auto_reg_limit () of them, least recently used dropped first. */
@@ -598,12 +581,8 @@ struct Ctx {
   std::thread sched;
   bool quit = false;
 
-  Lane lanes[kLanes];
-  int next_lane = 0;
-  std::map<uint64_t, int> lane_tickets;
-
-  /* staged host frames (staging.cu): FLUC_TTMLBLEND_STAGE_THREADS copy workers (0: the DMA lanes
-   * above instead), at most FLUC_TTMLBLEND_STAGE_SLOTS pinned staging frames in use */
+  /* staged host frames (staging.cu): FLUC_TTMLBLEND_STAGE_THREADS copy workers, at most
+   * FLUC_TTMLBLEND_STAGE_SLOTS pinned staging frames in use */
   int stage_threads = 0, stage_slots_max = 64, stage_slots_total = 0;
   int stage_active = 0, stage_copying = 0;
   std::vector<PoolEntry> stage_slots_free;
@@ -758,12 +737,11 @@ void stage_free_slots (Ctx *c);
 
 /* scheduler.cu */
 cudaEvent_t event_get (Ctx *c);
-int launch_jobs (Ctx *c, TableSlot &s, const PlaneJob *jobs, size_t n, int kind, bool fast, int sync, cudaStream_t stream);
+int launch_jobs (Ctx *c, TableSlot &s, const PlaneJob *jobs, size_t n, int kind, bool fast, int sync);
 void reap_batches (Ctx *c);
 int launch_pending (Ctx *c);
 bool layout_takes_dma (const Layout *L);
 void scheduler_main (Ctx *c);
-int lane_reserve (Ctx *c, Lane &l, size_t bytes);
 
 }  // namespace tbh
 #endif

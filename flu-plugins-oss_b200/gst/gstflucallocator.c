@@ -9,7 +9,7 @@
  * Why: fluc_ttmlblend_blend_host () blends device-accessible host memory
  * zero-copy -- the kernel reads the rows under the cue over PCIe and writes
  * them back, batched across streams -- while pageable memory has to be staged
- * through copy lanes. ttmlblend proposes this allocator upstream in its
+ * by worker threads. ttmlblend proposes this allocator upstream in its
  * propose_allocation so that decoders / videotestsrc write their frames
  * straight into pinned pool frames. This is SURVEY.md section 8f rank 2, the
  * "device frame-buffer pool bridged to GstBuffer (pinned staging)" of

@@ -295,7 +295,8 @@ FLUC_EXPORT int fluc_ttmlblend_set_batch (FlucTtmlBlend *thiz, uint32_t max_fram
  * or memory passed to host_register, 16-byte aligned -- are blended zero copy:
  * they join the batch like submit() frames and the kernel reads and writes
  * them over PCIe itself. Anything else (pageable or unaligned memory) is
- * staged through copy lanes: host -> device, blend, device -> host.
+ * staged by worker threads: the rows under the cue are copied into a pinned
+ * staging frame, blended zero copy, and copied back.
  * Asynchronous either way: the frame is complete once wait(ticket) returns. */
 FLUC_EXPORT int fluc_ttmlblend_blend_host (FlucTtmlBlend *thiz, uint32_t stream,
     FlucTtmlBlendFormat fmt, int32_t width, int32_t height, uint32_t frame_flags,

@@ -147,7 +147,7 @@ def test_overlapping_views_of_one_buffer_are_ordered(ctx):
 @pytest.mark.parametrize("pinned", [True, False])
 def test_two_overlays_on_one_host_frame(ctx, pinned):
     """Two streams' cues blended onto the same host frame back to back (zero copy when the frame
-    is pinned, otherwise two staging lanes that must run one after the other)."""
+    is pinned, otherwise two staging jobs that must run one after the other)."""
     fmt = "NV12"
     ov1, ov2 = _overlays(2, 940)
     ctx.overlay_set_rectangles(740, _rects(ov1))
@@ -199,9 +199,7 @@ def test_host_forget_drops_automatic_registrations():
                 p[...] = s
             c.wait(c.blend_host(1, fmt, W, H, planes))
             assert_planes_equal(planes, want, f"auto-registered, repetition {rep}")
-            forgotten = c.host_forget(backing)
-            if os.environ.get("FLUC_TTMLBLEND_HOST_MODE", "1") != "0":     # mode 0 stages everything: nothing is pinned
-                assert forgotten >= 1
+            assert c.host_forget(backing) >= 1
         assert c.host_forget(backing) == 0                   # nothing left
     finally:
         c.close()
@@ -361,7 +359,6 @@ def test_host_dma_batches(ctx):
             ctx.wait(t3)
             after = ctx.stats()
             if (rep >= 1 or os.environ.get("FLUC_TTMLBLEND_HOST_DMA") == "1") \
-                    and os.environ.get("FLUC_TTMLBLEND_HOST_MODE", "1") == "1" \
                     and "FLUC_TTMLBLEND_GROUPS" not in os.environ and "FLUC_TTMLBLEND_LAZY" not in os.environ:
                 assert after["host_dma_batches"] - before["host_dma_batches"] >= 2, after     # in pieces of 8 frames
             for i, (hf, fr) in enumerate(zip(hosts, frames)):

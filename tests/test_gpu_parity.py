@@ -682,8 +682,7 @@ def test_sparse_cues_take_the_overlay_first_path_in_place(ctx, fmt):
             st = ctx.stats()
             # which variant ran is a property of the default configuration; under a knob that
             # forces another code path (tools/knob_matrix.sh) only the bytes are checked
-            if not any(k in os.environ for k in ("FLUC_TTMLBLEND_LAZY", "FLUC_TTMLBLEND_GROUPS", "FLUC_TTMLBLEND_AUTOCROP",
-                                                 "FLUC_TTMLBLEND_HOST_MODE")):
+            if not any(k in os.environ for k in ("FLUC_TTMLBLEND_LAZY", "FLUC_TTMLBLEND_GROUPS", "FLUC_TTMLBLEND_AUTOCROP")):
                 assert (st["lazy_launches"] > 0) == lazy, (name, on_host, st)
                 assert st["lazy_launches"] <= st["group_launches"]
             assert_planes_equal(got, want, f"{fmt} {name} host={on_host}")
@@ -750,7 +749,7 @@ def test_streams_with_different_cue_layouts_share_one_launch(ctx, fmt, mode):
 
 def test_blend_host_many_equals_blend_host(ctx):
     """One C call for a run of host frames: pinned pool frames (zero copy) and, through the
-    same call, pageable numpy frames (staging lanes) -- each must equal the oracle."""
+    same call, pageable numpy frames (staging threads) -- each must equal the oracle."""
     fmt, w, h, n = "NV12", 320, 180, 6
     rects = [dict(pixels=random_overlay(200, 40, 61), x=60, y=120)]
     ctx.overlay_set_rectangles(9, rects)

@@ -5,7 +5,7 @@
 // tools/pcie_ceiling.cu: the same box, the same moment, ceiling and product path side by side.
 //
 //   build/e2e_multi --gpus 0,1,2,3 [--threads] [--secs 2] [--pin] [--opaque]
-//   (FLUC_TTMLBLEND_SYNC=block, FLUC_TTMLBLEND_HOST_MODE=0/1/2 select library variants)
+//   (FLUC_TTMLBLEND_SYNC=block selects blocking waits in the library)
 #include "../include/fluc_ttmlblend.h"
 
 #include <atomic>
@@ -239,9 +239,9 @@ main (int argc, char **argv)
     fps += sh->fps[w];
     gbs += sh->gbs[w];
   }
-  const char *sy = getenv ("FLUC_TTMLBLEND_SYNC"), *hm = getenv ("FLUC_TTMLBLEND_HOST_MODE");
-  printf ("e2e %d GPU(s) as %s, pin=%d sync=%s host_mode=%s %s: %9.0f frames/s aggregate, %6.1f GB/s each way; per GPU:",
-      G, o.threads ? "threads" : "processes", o.pin ? 1 : 0, sy ? sy : "spin", hm ? hm : "1",
+  const char *sy = getenv ("FLUC_TTMLBLEND_SYNC");
+  printf ("e2e %d GPU(s) as %s, pin=%d sync=%s %s: %9.0f frames/s aggregate, %6.1f GB/s each way; per GPU:",
+      G, o.threads ? "threads" : "processes", o.pin ? 1 : 0, sy ? sy : "spin",
       o.pageable ? (o.opaque ? "opaque, pageable frames" : "translucent, pageable frames") : o.opaque ? "opaque" : "translucent", fps, gbs);
   for (int w = 0; w < G; w++)
     printf (" %.0f", sh->fps[w]);

@@ -13,6 +13,6 @@ done
 bash tools/knob_matrix.sh > $O/r02_knob_matrix.txt 2>&1
 grep -c passed $O/r02_knob_matrix.txt; grep -c failed $O/r02_knob_matrix.txt
 build/latency_probe > $O/r02_latency_probe.txt 2>&1
-{ for t in 4 8 12; do FLUC_TTMLBLEND_STAGE_THREADS=$t build/e2e_multi --gpus 0 --pageable --secs 1.5; done; FLUC_TTMLBLEND_STAGE_THREADS=0 build/e2e_multi --gpus 0 --pageable --secs 1.5; build/e2e_multi --gpus 0 --secs 1.5; } > $O/r02_pageable_probe.txt 2>&1
+{ for t in 4 8 12; do FLUC_TTMLBLEND_STAGE_THREADS=$t build/e2e_multi --gpus 0 --pageable --secs 1.5; done; build/e2e_multi --gpus 0 --secs 1.5; } > $O/r02_pageable_probe.txt 2>&1
 build/launch_floor > $O/r02_launch_floor.txt 2>&1
 bash tools/ab_opaque.sh > $O/r02_opaque_skip.txt 2>&1

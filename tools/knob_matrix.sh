@@ -1,15 +1,14 @@
 #!/bin/bash
 # Runs the parity tests with every alternative code path forced through its environment knob:
 # table kernel only, no multi-layout launches, in-place launches always / never lazy, no
-# auto-crop, register-staged instead of TMA-staged overlay, interleaved chunk order, and the two
-# other host-frame modes. Every line must end in "passed".
+# auto-crop, register-staged instead of TMA-staged overlay, interleaved chunk order, and the
+# host-frame knobs. Every line must end in "passed".
 #   gpurun -- bash tools/knob_matrix.sh
 K="rectangles_match_oracle or golden or fuzz or alpha_sweep or scaled_rectangles or regions or unaligned or chain or ping_pong or dependency or two_overlays or update or sparse_cues or host_path or host_dma"
 for v in FLUC_TTMLBLEND_GROUPS=0 FLUC_TTMLBLEND_MULTI=0 FLUC_TTMLBLEND_LAZY=1 FLUC_TTMLBLEND_LAZY=0 \
          FLUC_TTMLBLEND_AUTOCROP=0 FLUC_TTMLBLEND_BULK=0 FLUC_TTMLBLEND_LANES=7 \
-         FLUC_TTMLBLEND_HOST_MODE=0 FLUC_TTMLBLEND_HOST_MODE=2 \
          FLUC_TTMLBLEND_PDL=0 FLUC_TTMLBLEND_OPAQUE_SKIP=1 FLUC_TTMLBLEND_OPAQUE_SKIP=0 \
-         FLUC_TTMLBLEND_STAGE_THREADS=0 FLUC_TTMLBLEND_STAGE_THREADS=1 FLUC_TTMLBLEND_COMPACT_PARAMS=0 \
+         FLUC_TTMLBLEND_STAGE_THREADS=1 FLUC_TTMLBLEND_COMPACT_PARAMS=0 \
          FLUC_TTMLBLEND_SYNC=block FLUC_TTMLBLEND_STAGE_NT=0 FLUC_TTMLBLEND_HOST_DMA=1 FLUC_TTMLBLEND_HOST_DMA=0 \
          FLUC_TTMLBLEND_DMA_PIECE=0; do
   echo "== $v"

@@ -18,8 +18,6 @@ E="timeout 90 build/e2e_multi --secs 1.5"
   $E --gpus 0,1,2,3,4,5,6,7 --threads
   $E --gpus 0,1,2,3,4,5,6,7 --pin
   FLUC_TTMLBLEND_SYNC=block $E --gpus 0,1,2,3,4,5,6,7
-  FLUC_TTMLBLEND_HOST_MODE=0 $E --gpus 0,1,2,3,4,5,6,7
-  FLUC_TTMLBLEND_HOST_MODE=2 $E --gpus 0,1,2,3,4,5,6,7
   $E --gpus 0,1,2,3,4,5,6,7 --opaque
   $E --gpus 0 --opaque; } > $O/r02_e2e_multi.txt 2>&1
 timeout 200 python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29511 \

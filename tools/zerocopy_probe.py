@@ -1,5 +1,5 @@
-"""Scratch probe: blend pinned HOST frames in place by letting the kernel read/write them over
-PCIe directly (zero-copy), versus the staged blend_host path. Config 3."""
+"""Scratch probe: blend pinned HOST frames in place through blend_host, the kernel reading and
+writing them over PCIe directly (zero-copy). Config 3."""
 import sys, time, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -19,10 +19,10 @@ ctx.set_batch(n, 0)
 def step_zc():
     t = [ctx.submit(1, cfg.fmt, cfg.width, cfg.height, hf.c, hf.c) for hf in hosts]
     ctx.wait(t[-1])
-def step_staged():
+def step_host():
     t = [ctx.blend_host_frame(1, cfg.fmt, cfg.width, cfg.height, hf.c) for hf in hosts]
     for x in t: ctx.wait(x)
-for name, fn in ((f"blend_host mode {os.environ.get('FLUC_TTMLBLEND_HOST_MODE', 'default')}", step_staged),):
+for name, fn in (("blend_host", step_host),):
     for _ in range(3): fn()
     ctx.sync(); t0 = time.perf_counter(); k = 30
     for _ in range(k): fn()
