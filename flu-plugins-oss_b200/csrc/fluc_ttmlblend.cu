@@ -471,7 +471,8 @@ order_against_pending (Ctx *c, const FrameExtent &src, const FrameExtent &dst, b
 
 static int
 submit_locked (Ctx *c, uint32_t stream, int fmt, int32_t W, int32_t H, uint32_t frame_flags,
-    const FlucTtmlBlendFrame *src, const FlucTtmlBlendFrame *dst, uint64_t *ticket)
+    const FlucTtmlBlendFrame *src, const FlucTtmlBlendFrame *dst, uint64_t *ticket,
+    const std::shared_ptr<StreamAfter> &after)
 {
   int rc;
   fmt = format_canon (fmt);
@@ -479,6 +480,7 @@ submit_locked (Ctx *c, uint32_t stream, int fmt, int32_t W, int32_t H, uint32_t 
     return rc;
   PendingFrame f;
   f.prep = nullptr;
+  f.after = after;
   auto it = c->overlays.find (stream);
   if (it != c->overlays.end ()) {
     f.overlay = it->second;
@@ -518,10 +520,26 @@ fluc_ttmlblend_submit (FlucTtmlBlend *thiz, uint32_t stream, FlucTtmlBlendFormat
     const FlucTtmlBlendFrame *dst, uint64_t *ticket)
 {
   ENTER (thiz);
-  int rc = submit_locked (c, stream, fmt, W, H, frame_flags, src, dst, ticket);
+  int rc = submit_locked (c, stream, fmt, W, H, frame_flags, src, dst, ticket, nullptr);
   if (rc == 0 && c->linger_us && !c->pending.empty ())
     c->cv.notify_all ();
   return rc;
+}
+
+static int
+submit_many_locked (Ctx *c, uint32_t n, const uint32_t *streams, FlucTtmlBlendFormat fmt, int32_t W, int32_t H,
+    uint32_t frame_flags, const FlucTtmlBlendFrame *srcs, const FlucTtmlBlendFrame *dsts, uint64_t *tickets,
+    const std::shared_ptr<StreamAfter> &after)
+{
+  for (uint32_t i = 0; i < n; i++) {
+    int rc = submit_locked (c, streams[i], fmt, W, H, frame_flags, &srcs[i], &dsts[i],
+        tickets ? &tickets[i] : nullptr, after);
+    if (rc)
+      return rc;
+  }
+  if (c->linger_us && !c->pending.empty ())
+    c->cv.notify_all ();
+  return 0;
 }
 
 int
@@ -532,15 +550,42 @@ fluc_ttmlblend_submit_many (FlucTtmlBlend *thiz, uint32_t n, const uint32_t *str
   ENTER (thiz);
   if (n && (!streams || !srcs || !dsts))
     return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
-  for (uint32_t i = 0; i < n; i++) {
-    int rc = submit_locked (c, streams[i], fmt, W, H, frame_flags, &srcs[i], &dsts[i],
-        tickets ? &tickets[i] : nullptr);
-    if (rc)
-      return rc;
+  return submit_many_locked (c, n, streams, fmt, W, H, frame_flags, srcs, dsts, tickets, nullptr);
+}
+
+/* A caller's CUDA stream (NULL: the legacy default stream of the context's device), which must
+ * belong to the context's device: an event of one device cannot be recorded on, or waited for by,
+ * a stream of another. */
+static int
+caller_stream (Ctx *c, void *cuda_stream, cudaStream_t *out)
+{
+  *out = cuda_stream ? static_cast<cudaStream_t> (cuda_stream) : cudaStreamLegacy;
+  int dev = -1;
+  if (cudaStreamGetDevice (*out, &dev) != cudaSuccess) {
+    cudaGetLastError ();
+    return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
   }
-  if (c->linger_us && !c->pending.empty ())
-    c->cv.notify_all ();
-  return 0;
+  return dev == c->device ? 0 : FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
+}
+
+int
+fluc_ttmlblend_submit_many_after (FlucTtmlBlend *thiz, void *cuda_stream, uint32_t n,
+    const uint32_t *streams, FlucTtmlBlendFormat fmt, int32_t W, int32_t H, uint32_t frame_flags,
+    const FlucTtmlBlendFrame *srcs, const FlucTtmlBlendFrame *dsts, uint64_t *tickets)
+{
+  ENTER (thiz);
+  if (n && (!streams || !srcs || !dsts))
+    return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
+  cudaStream_t st;
+  int rc = caller_stream (c, cuda_stream, &st);
+  if (rc || n == 0)
+    return rc;
+  /* declared after lk: goes back to the pool (when no frame holds it any more) under the lock */
+  std::shared_ptr<StreamAfter> after (new StreamAfter ());
+  after->ctx = c;
+  after->ev = event_get (c);
+  CU (c, cudaEventRecord (after->ev, st));
+  return submit_many_locked (c, n, streams, fmt, W, H, frame_flags, srcs, dsts, tickets, after);
 }
 
 int
@@ -569,15 +614,14 @@ fluc_ttmlblend_flush (FlucTtmlBlend *thiz)
   return launch_pending (c);
 }
 
-int
-fluc_ttmlblend_wait (FlucTtmlBlend *thiz, uint64_t ticket)
+/* wait () and wait_on_stream () of a ticket that is not a staged host frame's: launches it if it is
+ * still queued, then finds the `done` event of its batch (*ev = nullptr: finished). *failed: the
+ * error of a batch whose launch failed half way. */
+static int
+launch_and_find (Ctx *c, std::unique_lock<std::mutex> &lk, uint64_t ticket, cudaEvent_t *ev, int *failed)
 {
-  ENTER (thiz);
-  if (ticket == 0 || ticket > c->next_ticket)
-    return FLUC_TTMLBLEND_ERROR_NOT_FOUND;
-  int staged_rc = 0;
-  if (stage_wait (c, lk, ticket, &staged_rc))
-    return staged_rc;
+  *ev = nullptr;
+  *failed = 0;
   if (!c->pending.empty () && ticket >= c->pending.front ().ticket) {
     /* The frame has not been launched yet. A lone stream launches now (lowest latency). When
      * several streams are active -- many elements calling blend + wait from their own
@@ -599,19 +643,34 @@ fluc_ttmlblend_wait (FlucTtmlBlend *thiz, uint64_t ticket)
     }
   }
   /* a batch whose launch failed half way: still synchronise with what went out, then say so */
-  int failed = 0;
   for (const Ctx::FailedRange &fr : c->failed_ranges)
     if (ticket >= fr.first && ticket <= fr.last)
-      failed = fr.rc;
+      *failed = fr.rc;
   /* a ticket whose batch has been retired is finished; it must not fall through to the next batch
    * in flight (a caller that waits one batch behind would then wait for the newest one) */
-  cudaEvent_t ev = nullptr;
   if (ticket > c->retired_through)
     for (auto &b : c->batches)
       if (b.last_ticket >= ticket) {
-        ev = b.done;
+        *ev = b.done;
         break;
       }
+  return 0;
+}
+
+int
+fluc_ttmlblend_wait (FlucTtmlBlend *thiz, uint64_t ticket)
+{
+  ENTER (thiz);
+  if (ticket == 0 || ticket > c->next_ticket)
+    return FLUC_TTMLBLEND_ERROR_NOT_FOUND;
+  int staged_rc = 0;
+  if (stage_wait (c, lk, ticket, &staged_rc))
+    return staged_rc;
+  cudaEvent_t ev;
+  int failed;
+  int rc = launch_and_find (c, lk, ticket, &ev, &failed);
+  if (rc)
+    return rc;
   if (!ev) {
     return failed;              /* already reaped: finished */
   }
@@ -626,6 +685,28 @@ fluc_ttmlblend_wait (FlucTtmlBlend *thiz, uint64_t ticket)
     return c->sticky;
   }
   reap_batches (c);
+  return failed;
+}
+
+int
+fluc_ttmlblend_wait_on_stream (FlucTtmlBlend *thiz, uint64_t ticket, void *cuda_stream)
+{
+  ENTER (thiz);
+  if (ticket == 0 || ticket > c->next_ticket)
+    return FLUC_TTMLBLEND_ERROR_NOT_FOUND;
+  cudaStream_t st;
+  int rc = caller_stream (c, cuda_stream, &st);
+  if (rc)
+    return rc;
+  /* a staged host frame is finished by a CPU copy, which no stream can wait for */
+  if (c->stage_jobs.count (ticket))
+    return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
+  cudaEvent_t ev;
+  int failed;
+  if ((rc = launch_and_find (c, lk, ticket, &ev, &failed)))
+    return rc;
+  if (ev)
+    CU (c, cudaStreamWaitEvent (st, ev, 0));
   return failed;
 }
 

@@ -21,6 +21,13 @@ event_get (Ctx *c)
   return e;
 }
 
+/* a stream wait captures the event's state when it is enqueued: the event may be recorded again */
+StreamAfter::~StreamAfter ()
+{
+  if (ctx && ev)
+    ctx->event_pool.push_back (ev);
+}
+
 int
 slot_reserve (Ctx *c, TableSlot &s, size_t n, size_t words)
 {
@@ -453,6 +460,19 @@ launch_pending (Ctx *c)
       f.prep->blend_waited = true;
       CU (c, cudaStreamWaitEvent (c->blend_stream, f.prep->ready, 0));
       c->blend_stream_waits = true;
+    }
+    if (f.after && !f.after->resolved) {
+      /* the caller's work before submit_many_after: once per call; when it has already finished,
+       * no wait, and the launch keeps programmatic dependent launch */
+      f.after->resolved = true;
+      const cudaError_t q = cudaEventQuery (f.after->ev);
+      if (q != cudaSuccess) {
+        if (q != cudaErrorNotReady)
+          CU (c, q);
+        cudaGetLastError ();
+        CU (c, cudaStreamWaitEvent (c->blend_stream, f.after->ev, 0));
+        c->blend_stream_waits = true;
+      }
     }
     c->stats.frames_blended++;
     c->stats.algorithmic_bytes += f.layout->algo_bytes;

@@ -346,11 +346,23 @@ struct Overlay {
   ~Overlay ();
 };
 
+/* The event submit_many_after records on the caller's stream, shared by every frame of the call.
+ * The first launch that carries one of them orders the blend stream after it (or finds it already
+ * complete); later launches follow in stream order. Back to the event pool with its last frame.
+ * Destroyed under the context lock. */
+struct StreamAfter {
+  Ctx *ctx = nullptr;
+  cudaEvent_t ev = nullptr;
+  bool resolved = false;               /* the blend stream is ordered after it */
+  ~StreamAfter ();
+};
+
 struct PendingFrame {
   uint64_t ticket;
   uint32_t stream;
   bool host = false;                   /* a device-accessible HOST frame, blended in place (zero copy or DMA batch) */
   uintptr_t host_lo = 0, host_hi = 0;  /* its bytes (hull of the planes) */
+  std::shared_ptr<StreamAfter> after;  /* submit_many_after: the caller's work to wait for */
   std::shared_ptr<Overlay> overlay;    /* keeps prep and layout alive */
   Prepared *prep;
   const Layout *layout;

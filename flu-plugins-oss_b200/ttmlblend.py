@@ -108,6 +108,10 @@ PROTOTYPES = {
     "fluc_ttmlblend_submit_many_repeat": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32), C.c_int,
                                                     C.c_int32, C.c_int32, C.c_uint32, C.POINTER(Frame),
                                                     C.POINTER(Frame), C.c_uint32, C.c_uint32]),
+    "fluc_ttmlblend_submit_many_after": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32),
+                                                   C.c_int, C.c_int32, C.c_int32, C.c_uint32, C.POINTER(Frame),
+                                                   C.POINTER(Frame), C.POINTER(C.c_uint64)]),
+    "fluc_ttmlblend_wait_on_stream": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p]),
     "fluc_ttmlblend_pcie_probe": (C.c_int, [C.c_void_p, C.c_int, C.c_size_t, C.c_double, C.POINTER(C.c_double)]),
     "fluc_ttmlblend_flush": (C.c_int, [C.c_void_p]),
     "fluc_ttmlblend_wait": (C.c_int, [C.c_void_p, C.c_uint64]),
@@ -385,6 +389,21 @@ class TtmlBlend:
             self.h, batch.n, batch.streams, batch.fmt, batch.width, batch.height, batch.flags,
             batch.srcs, batch.dsts, batch.tickets), "submit_many")
         return batch.tickets
+
+    def submit_many_after(self, batch: "TtmlBlend.Batch", cuda_stream: int):
+        """submit_many ordered after the work already enqueued on a CUDA stream of the context's
+        device (the raw cudaStream_t handle, e.g. torch.cuda.current_stream().cuda_stream; 0: the
+        legacy default stream). The host does not wait for that work. Returns the ticket array."""
+        self._check(self.lib.fluc_ttmlblend_submit_many_after(
+            self.h, cuda_stream or None, batch.n, batch.streams, batch.fmt, batch.width, batch.height,
+            batch.flags, batch.srcs, batch.dsts, batch.tickets), "submit_many_after")
+        return batch.tickets
+
+    def wait_on_stream(self, ticket: int, cuda_stream: int):
+        """Work enqueued on the CUDA stream after this call runs after the ticket's frame is
+        complete; the host does not wait."""
+        self._check(self.lib.fluc_ttmlblend_wait_on_stream(self.h, ticket, cuda_stream or None),
+                    "wait_on_stream")
 
     def submit_many_repeat(self, batch: "TtmlBlend.Batch", repeats: int):
         """`repeats` x submit_many (+ flush) inside one C call (bench helper)."""

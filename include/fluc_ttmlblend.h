@@ -288,6 +288,41 @@ FLUC_EXPORT int fluc_ttmlblend_sync (FlucTtmlBlend *thiz);
 FLUC_EXPORT int fluc_ttmlblend_set_batch (FlucTtmlBlend *thiz, uint32_t max_frames,
     uint32_t linger_us);
 
+/* ---- per frame, device-resident, ordered by the caller's CUDA stream --
+ * For frames another CUDA stream produces and consumes (decoder -> blend -> encoder), without a
+ * host thread blocking in between. `cuda_stream` is a cudaStream_t of the context's device passed
+ * as a pointer; NULL is the legacy default stream of that device. A stream of another device is
+ * INVALID_ARGUMENT.
+ *
+ * submit_many_after: submit_many, ordered after everything enqueued on cuda_stream before this
+ * call: the frames' launch does not start reading or writing them until that work is complete.
+ * The host never waits for it, with one exception: table-kernel launches rotate through 8 job-table
+ * slots, and a ninth such launch while 8 are held back waits for the first. The call records one
+ * event on cuda_stream; the launch that carries the call's frames waits for it on the blend stream
+ * (not at all when it has already completed). Such a launch goes out as an ordinary launch, not a
+ * programmatic dependent one. Frames of different calls, and submit* frames, still share launches:
+ * such a launch waits for all of its producers.
+ *
+ * wait_on_stream: work enqueued on cuda_stream after this call runs after the ticket's frame is
+ * complete. The ticket resolves as in wait(): NOT_FOUND for 0 or a ticket not handed out yet,
+ * nothing enqueued for a frame already complete, the error of a launch that failed. A frame that
+ * is still queued is launched under the same policy as wait() (it may linger for up to the linger
+ * time while several streams are active). The host never waits for the GPU. A host frame that
+ * went through the staging threads (blend_host of memory the GPU cannot reach) ends with a CPU
+ * copy no stream can wait for: INVALID_ARGUMENT, use wait(). Zero-copy host frames are fine.
+ *
+ * Batches complete in launch order, so waiting for the last ticket of a call covers every frame
+ * of it, even when the batch limit or a dependency between its frames split it into several
+ * launches.
+ *
+ * A frame may be reused -- rewritten by its producer, or freed -- only after its ticket has been
+ * waited for: with wait(), or with wait_on_stream() on the stream that reuses it. */
+FLUC_EXPORT int fluc_ttmlblend_submit_many_after (FlucTtmlBlend *thiz, void *cuda_stream,
+    uint32_t n, const uint32_t *streams, FlucTtmlBlendFormat fmt, int32_t width, int32_t height,
+    uint32_t frame_flags, const FlucTtmlBlendFrame *srcs, const FlucTtmlBlendFrame *dsts,
+    uint64_t *tickets);
+FLUC_EXPORT int fluc_ttmlblend_wait_on_stream (FlucTtmlBlend *thiz, uint64_t ticket, void *cuda_stream);
+
 /* ---- per frame, host-resident: the drop-in for -----------------------
  * gst_video_overlay_composition_blend (comp, frame). The frame is in HOST
  * memory and is modified in place; only the rows (and columns) the cue covers
