@@ -443,6 +443,21 @@ fluc_ttmlblend_overlay_clear (FlucTtmlBlend *thiz, uint32_t stream)
 }
 
 int
+fluc_ttmlblend_overlay_set_global_alpha (FlucTtmlBlend *thiz, uint32_t stream, const float *global_alpha, uint32_t n)
+{
+  ENTER (thiz);
+  if (!global_alpha || n == 0 || n > FLUC_TTMLBLEND_MAX_RECTANGLES)
+    return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
+  int ga[FLUC_TTMLBLEND_MAX_RECTANGLES];
+  for (uint32_t i = 0; i < n; i++) {
+    if (!(global_alpha[i] >= 0.0f && global_alpha[i] <= 1.0f))     /* NaN fails both */
+      return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
+    ga[i] = (int) (255.0 * global_alpha[i]);        /* gst_video_blend, as overlay_set_rectangles */
+  }
+  return overlay_set_alpha (c, stream, ga, n);
+}
+
+int
 fluc_ttmlblend_set_chroma_mode (FlucTtmlBlend *thiz, int mode)
 {
   ENTER (thiz);

@@ -379,15 +379,25 @@ frame_ptrs (const PendingFrame &f)
   return p;
 }
 
+/* JF_GA for the frames whose prepared overlay leaves a global alpha to the blend: a launch that
+ * holds one of them takes the kernel variant that scales the alpha bytes */
+static int
+frame_ga_flag (const PendingFrame &f)
+{
+  return f.prep && f.prep->fade ? JF_GA : 0;
+}
+
 /* The layout's table jobs with this frame's pointers, appended per (kind, fast). */
 void
 emit_table_jobs (const std::vector<PlaneJob> &tmpl, const PendingFrame &f, std::vector<PlaneJob> *by_kind)
 {
+  const int ga = frame_ga_flag (f);
   for (const PlaneJob &t : tmpl) {
     std::vector<PlaneJob> &v = by_kind[f.layout->kind * 2 + ((t.flags & JF_FAST) ? 1 : 0)];
     v.push_back (t);
     v.back ().src = f.src[t.plane];
     v.back ().dst = f.dst[t.plane];
+    v.back ().flags |= ga;
   }
 }
 
@@ -419,6 +429,7 @@ void
 group_add (Group &g, const PendingFrame &f)
 {
   g.P.frames[g.P.h.n_frames++] = frame_ptrs (f);
+  g.P.h.flags |= frame_ga_flag (f);
 }
 
 void
@@ -443,7 +454,7 @@ multi_add (MultiGroup &m, const PendingFrame &f)
 {
   const Layout &L = *f.layout;
   MultiParams &P = m.P;
-  if (m.kind != L.kind || P.flags != L.gflags || P.n_frames >= (uint32_t) kMaxGroupFrames ||
+  if (m.kind != L.kind || (P.flags & ~JF_GA) != L.gflags || P.n_frames >= (uint32_t) kMaxGroupFrames ||
       memcmp (P.src_pitch, L.src_pitch, sizeof P.src_pitch) || memcmp (P.dst_pitch, L.dst_pitch, sizeof P.dst_pitch))
     return false;
   if ((uint64_t) P.frame_begin[P.n_frames] + L.chunks_per_frame >= (1ull << 26))
@@ -472,6 +483,7 @@ multi_add (MultiGroup &m, const PendingFrame &f)
   P.frames[k] = frame_ptrs (f);
   P.frames[k].pad_ = (uint64_t) L.rect_off[0] | ((uint64_t) L.rect_off[1] << 16) | ((uint64_t) L.rect_off[2] << 32);
   P.frame_begin[k + 1] = P.frame_begin[k] + L.chunks_per_frame;
+  P.flags |= frame_ga_flag (f);
   return true;
 }
 

@@ -325,14 +325,36 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
   return 0;
 }
 
+/* The rectangle tables of P with every box's current global alpha: a box at 0 drops out (no
+ * band, no window in place), the others give it to the blend where the prepare did not fold it
+ * in -- RectRef::ga for the Cs*ga terms, RectRef::a_ga for the alpha bytes of the PLANE8 kinds. */
 static int
-prepare_assemble (Ctx *c, Prepared *P)
+prepare_assemble (Ctx *c, Prepared *P, const Overlay *ov)
 {
   for (int pl = 0; pl < 3; pl++)
     P->h_rects[pl].clear ();
-  for (const PreparedRect &pr : P->per_rect)
-    for (int k = 0; k < pr.n_refs; k++)
-      P->h_rects[pr.refs[k].plane].push_back (pr.refs[k].ref);
+  const int kind = plane_kind (P->format);
+  const bool planes = kind == PK_PLANE8 || kind == PK_PLANE8_RGB;
+  P->fade = false;
+  for (const OverlayBox &b : ov->boxes)
+    for (uint32_t i = b.first_rect; i < b.first_rect + b.n_rects; i++) {
+      const PreparedRect &pr = P->per_rect[i];
+      if (b.ga == 0)
+        continue;
+      const bool folded = planes && ov->rects[i].ga != 255;
+      for (int k = 0; k < pr.n_refs; k++) {
+        RectRef ref = pr.refs[k].ref;
+        ref.a_ga = 255;
+        if (!folded) {
+          if (kind != PK_PLANE8)
+            ref.ga = b.ga;
+          if (planes)
+            ref.a_ga = b.ga;
+        }
+        P->fade = P->fade || ref.a_ga != 255;
+        P->h_rects[pr.refs[k].plane].push_back (ref);
+      }
+    }
   /* rectangle tables: one contiguous device array, plane after plane */
   {
     size_t total = 0;
@@ -382,7 +404,7 @@ prepare_build (Ctx *c, Overlay *ov, int format, int W, int H, std::unique_ptr<Pr
     if (rc)
       return rc;
   }
-  return prepare_assemble (c, P.get ());
+  return prepare_assemble (c, P.get (), ov);
 }
 
 
@@ -484,6 +506,7 @@ struct Up {
   std::vector<int2> spans;
   std::vector<int> groups;      /* per row: 16-pixel groups with any alpha */
   std::vector<int> raw;         /* both as they come back from the GPU in one copy: h x int2, then h x int */
+  uint32_t slot = 0;            /* OverlayBox::slot */
 };
 
 /* Is this pointer device memory (a cue produced on the GPU, or left there by a previous stage)? */
@@ -562,6 +585,8 @@ append_box (Ctx *c, Overlay *ov, Up &u, size_t n_boxes)
   OverlayBox box;
   box.declared = { u.rr.x, u.rr.y, u.rr.w, u.rr.h };
   box.first_rect = (uint32_t) ov->rects.size ();
+  box.ga = u.rr.ga;
+  box.slot = u.slot;
   if (!c->autocrop) {
     ov->rects.push_back (u.rr);
   } else {
@@ -574,8 +599,7 @@ append_box (Ctx *c, Overlay *ov, Up &u, size_t n_boxes)
       box.groups_all += (uint64_t) ceil_div (s.w, 16) * (uint64_t) s.h;
       for (int y = s.y; y < s.y + s.h; y++) {
         box.groups_on += (uint64_t) (u.groups[y] & 0xffff);
-        if (u.rr.ga == 255)
-          box.groups_opaque += (uint64_t) (u.groups[y] >> 16);
+        box.groups_opaque += (uint64_t) (u.groups[y] >> 16);
       }
       RawRect q = u.rr;
       q.dev = u.rr.dev + (size_t) s.y * u.rr.pitch + (size_t) s.x * 4;
@@ -602,9 +626,10 @@ decide_lazy (Overlay *ov)
   static const char *lazy_env = getenv ("FLUC_TTMLBLEND_LAZY");
   uint64_t groups_all = 0, groups_on = 0, groups_opaque = 0;
   for (const OverlayBox &b : ov->boxes) {
+    /* what the blend sees: a box at global alpha 0 is transparent, only one at 1 has opaque vectors */
     groups_all += b.groups_all;
-    groups_on += b.groups_on;
-    groups_opaque += b.groups_opaque;
+    groups_on += b.ga ? b.groups_on : 0;
+    groups_opaque += b.ga == 255 ? b.groups_opaque : 0;
   }
   ov->transparent_fraction = groups_all ? 1.0 - (double) groups_on / (double) groups_all : 0.0;
   ov->opaque_fraction = groups_all ? (double) groups_opaque / (double) groups_all : 0.0;
@@ -708,6 +733,7 @@ overlay_install (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, cons
   ov->image_w = image_w;
   ov->image_h = image_h;
   ov->updatable = image_w > 0 && image_h > 0;
+  ov->n_alphas = std::max<uint32_t> (1, n);
   std::vector<Up> ups;
   std::vector<std::vector<int4>> plans;     /* host side of async uploads: alive until finish_install */
   InstallStats st;
@@ -726,6 +752,7 @@ overlay_install (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, cons
     if (xoff >= rw || yoff >= rh)
       continue;
     Up u;
+    u.slot = i;
     RawRect &rr = u.rr;
     rr.w = rw - xoff;
     rr.h = rh - yoff;
@@ -863,11 +890,17 @@ overlay_update_image (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream,
   nv->image_w = w;
   nv->image_h = h;
   nv->updatable = true;
+  nv->n_alphas = old->n_alphas;
   nv->declared = old->declared;
   std::vector<int> from_old;    /* new rectangle -> the old overlay's rectangle it is, or -1 */
   for (size_t b = 0; b < old->boxes.size (); b++) {
     if (touched[b]) {
+      /* new pixels, prepared without a global alpha; the box keeps its current one */
+      ups[b].slot = old->boxes[b].slot;
+      ups[b].rr.ga = old->boxes[b].ga;
       append_box (c, nv.get (), ups[b], old->boxes.size ());
+      for (uint32_t k = nv->boxes.back ().first_rect; k < nv->rects.size (); k++)
+        nv->rects[k].ga = 255;
       from_old.resize (nv->rects.size (), -1);
     } else {
       OverlayBox box = old->boxes[b];
@@ -903,7 +936,7 @@ overlay_update_image (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream,
         rc = prepare_rect (c, nv->rects[i], P->format, P->W, P->H, P->chroma_average, P->per_rect[i]);
     }
     if (!rc)
-      rc = prepare_assemble (c, P.get ());
+      rc = prepare_assemble (c, P.get (), nv.get ());
     if (rc) {
       if (P->ready)
         cudaEventDestroy (P->ready);
@@ -914,6 +947,81 @@ overlay_update_image (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream,
   c->overlays[stream] = nv;       /* frames already queued keep the old one */
   c->stats.overlays_set++;
   c->stats.overlays_updated++;
+  return 0;
+}
+
+/* overlay_set_global_alpha: a new generation of the stream's overlay that differs from the
+ * current one in its boxes' global alphas only. It shares every device block -- raw pixels and
+ * prepared planes -- and brings new rectangle tables (a few hundred bytes, uploaded on the upload
+ * stream and waited for through Prepared::ready like a cue change). Its layouts are built again
+ * at the first frame and get the ids of equal band lists, so a fading stream's frames still share
+ * launches. The PLANE8 kinds need the alpha bytes without a global alpha folded in: a box
+ * installed below 1 is prepared once more from its raw pixels the first time it changes. */
+int
+overlay_set_alpha (Ctx *c, uint32_t stream, const int *ga, uint32_t n)
+{
+  NvtxRange nvtx ("ttmlblend.overlay_set_global_alpha");
+  auto it = c->overlays.find (stream);
+  if (it == c->overlays.end ())
+    return FLUC_TTMLBLEND_ERROR_NOT_FOUND;
+  const std::shared_ptr<Overlay> old = it->second;
+  if (n != 1 && n != old->n_alphas)
+    return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
+  std::shared_ptr<Overlay> nv (new Overlay ());
+  nv->ctx = c;
+  nv->rects = old->rects;
+  nv->boxes = old->boxes;
+  nv->declared = old->declared;
+  nv->image_w = old->image_w;
+  nv->image_h = old->image_h;
+  nv->updatable = old->updatable;
+  nv->n_alphas = old->n_alphas;
+  std::vector<bool> again (nv->rects.size (), false);   /* prepared once more, without a global alpha */
+  bool changed = false;
+  for (OverlayBox &b : nv->boxes) {
+    const int v = ga[n == 1 ? 0 : b.slot];
+    if (v == b.ga)
+      continue;
+    changed = true;
+    b.ga = v;
+    for (uint32_t i = b.first_rect; i < b.first_rect + b.n_rects; i++)
+      if (nv->rects[i].ga != 255) {
+        again[i] = true;
+        nv->rects[i].ga = 255;
+      }
+  }
+  if (!changed)
+    return 0;
+  decide_lazy (nv.get ());
+  for (auto &p : old->prepared) {
+    const int kind = plane_kind (p->format);
+    const bool planes = kind == PK_PLANE8 || kind == PK_PLANE8_RGB;
+    std::unique_ptr<Prepared> P (new Prepared ());
+    P->format = p->format;
+    P->W = p->W;
+    P->H = p->H;
+    P->chroma_average = p->chroma_average;
+    P->overlay_px = p->overlay_px;
+    P->used = p->used;
+    P->per_rect.resize (nv->rects.size ());
+    int rc = 0;
+    for (size_t i = 0; i < nv->rects.size () && !rc; i++) {
+      /* the packed kinds never fold the global alpha in; a rectangle installed at 0 was not prepared */
+      if (again[i] && (planes || old->rects[i].ga == 0))
+        rc = prepare_rect (c, nv->rects[i], P->format, P->W, P->H, P->chroma_average, P->per_rect[i]);
+      else
+        P->per_rect[i] = p->per_rect[i];
+    }
+    if (!rc)
+      rc = prepare_assemble (c, P.get (), nv.get ());
+    if (rc) {
+      if (P->ready)
+        cudaEventDestroy (P->ready);
+      return rc;
+    }
+    nv->prepared.push_back (std::move (P));
+  }
+  c->overlays[stream] = nv;       /* frames already queued keep the old one */
   return 0;
 }
 

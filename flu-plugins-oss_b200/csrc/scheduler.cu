@@ -75,7 +75,9 @@ launch_jobs (Ctx *c, TableSlot &s, const PlaneJob *jobs, size_t n, int kind, boo
   uint32_t total = 0;
   uint32_t *coarse = s.h_begin + n;
   size_t next = 0;
+  bool ga = false;
   for (size_t i = 0; i < n; i++) {
+    ga = ga || (jobs[i].flags & JF_GA);
     s.h_jobs[i] = jobs[i];
     s.h_begin[i] = total;
     total += jobs[i].n_chunks;
@@ -89,7 +91,7 @@ launch_jobs (Ctx *c, TableSlot &s, const PlaneJob *jobs, size_t n, int kind, boo
           c->table_stream));
   CU (c, cudaEventRecord (s.uploaded, c->table_stream));
   CU (c, cudaStreamWaitEvent (c->blend_stream, s.uploaded, 0));
-  CU (c, launch_blend (s.d_jobs, s.d_begin, s.d_begin + n, (int) n, total, kind, fast, sync, c->blend_stream));
+  CU (c, launch_blend (s.d_jobs, s.d_begin, s.d_begin + n, (int) n, total, kind, fast, ga, sync, c->blend_stream));
   CU (c, cudaEventRecord (s.copied, c->blend_stream));    /* slot busy until this kernel is done */
   c->stats.launches++;
   return 0;

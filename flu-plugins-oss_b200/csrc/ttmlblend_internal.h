@@ -260,7 +260,7 @@ struct RawRect {
   uint8_t *dev = nullptr;
   int pitch = 0, w = 0, h = 0;
   int x = 0, y = 0;
-  int ga = 255;
+  int ga = 255;                        /* global alpha the prepare folds into PLANE8 alpha bytes (255 after a fade) */
   bool premul = true;
 };
 
@@ -315,6 +315,7 @@ struct Prepared {
   RectRef *d_rects_all = nullptr;      /* the three tables, contiguous */
   int32_t rect_off[3] = { 0, 0, 0 };   /* first entry of plane p in d_rects_all */
   uint64_t overlay_px = 0;             /* sum of clipped w*h */
+  bool fade = false;                   /* a RectRef has a_ga != 255: launches holding it take the JF_GA variant */
   cudaEvent_t ready = nullptr;
   bool blend_waited = false;           /* blend stream already ordered after `ready` */
   bool used = false;                   /* a frame has been blended with it (worth preparing the next cue for) */
@@ -326,7 +327,9 @@ struct Prepared {
 struct OverlayBox {
   FlucTtmlBlendRect declared = { 0, 0, 0, 0 };       /* frame coordinates, clipped at the left / top */
   uint32_t first_rect = 0, n_rects = 0;              /* its cropped sub-rectangles in Overlay::rects */
-  uint64_t groups_all = 0, groups_on = 0, groups_opaque = 0;   /* 16-pixel groups under them: all / some alpha / opaque */
+  uint64_t groups_all = 0, groups_on = 0, groups_opaque = 0;   /* 16-pixel groups under them: all / some alpha / alpha 255 */
+  int ga = 255;                        /* its current global alpha (overlay_set_global_alpha) */
+  uint32_t slot = 0;                   /* which value of overlay_set_global_alpha's list is its own */
 };
 
 struct Overlay {
@@ -338,9 +341,10 @@ struct Overlay {
    * alpha 1 -- what overlay_update can patch */
   int image_w = 0, image_h = 0;
   bool updatable = false;
+  uint32_t n_alphas = 1;               /* global alphas overlay_set_global_alpha takes besides one for all */
   std::vector<std::unique_ptr<Prepared>> prepared;
   double transparent_fraction = 0.0;   /* of the 16-pixel groups under the kept rectangles */
-  double opaque_fraction = 0.0;        /* alpha 255 all over (and global alpha 1) */
+  double opaque_fraction = 0.0;        /* alpha 255 all over (and the box's global alpha 1) */
   bool lazy_inplace = false;           /* in-place group launches look at the overlay first */
   bool opaque_skip = false;            /* out-of-place group launches do: no frame read under opaque vectors */
   ~Overlay ();
@@ -701,6 +705,8 @@ int overlay_update_image (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t str
     int stride, const FlucTtmlBlendRect *changed, uint32_t n_changed);
 int overlay_install_regions (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, int W, int H,
     const FlucTtmlBlendRegion *regions, uint32_t n);
+/* ga: n values 0..255, one for every box or (n == 1) for all; mu held throughout */
+int overlay_set_alpha (Ctx *c, uint32_t stream, const int *ga, uint32_t n);
 
 /* jobs.cu */
 void layout_spans (const Layout *L, std::vector<StageSpan> &out);

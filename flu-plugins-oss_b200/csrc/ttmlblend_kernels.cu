@@ -237,6 +237,24 @@ blend16_rgb24 (uint4 f, const uint4 &a, const uint4 &c, uint32_t ga, bool sp)
   return f;
 }
 
+/* The JF_GA variant of the PLANE8 kinds: the prepared alpha bytes hold the overlay's own alpha
+ * and the rectangle's current global alpha is applied per frame, asrc = a * ga / 255 on every
+ * byte (BLENDSPEC section 2), two 16-bit lanes per register as above (a * ga <= 65025). */
+__device__ __forceinline__ uint32_t
+scale4_alpha (uint32_t a, uint32_t ga)
+{
+  uint32_t e = (a & 0x00ff00ffu) * ga, o = ((a >> 8) & 0x00ff00ffu) * ga;
+  e = e + ((e >> 8) & 0x00ff00ffu) + 0x00010001u;
+  o = o + ((o >> 8) & 0x00ff00ffu) + 0x00010001u;
+  return ((e >> 8) & 0x00ff00ffu) | (o & 0xff00ff00u);
+}
+
+__device__ __forceinline__ uint4
+scale16_alpha (const uint4 &a, uint32_t ga)
+{
+  return make_uint4 (scale4_alpha (a.x, ga), scale4_alpha (a.y, ga), scale4_alpha (a.z, ga), scale4_alpha (a.w, ga));
+}
+
 /* kinds whose prepared overlay is an alpha byte plane + a colour byte plane */
 __host__ __device__ constexpr bool
 kind_is_planes (int kind)
@@ -365,14 +383,16 @@ rect_geom (const RectRef *r)
   return o;
 }
 
-template <int KIND>
+template <int KIND, bool GA = false>
 __device__ __forceinline__ uint4
 blend_with_rect (uint4 f, const RectRef *r, const RectGeom &g, int v, int y,
     bool dst_premul)
 {
   const int32_t pitch = __ldg (&r->pitch);
   const size_t off = (size_t) (y - g.y0) * pitch + (size_t) (v - g.v0) * 16;
-  const uint4 oa = ld_overlay16 (ldg_ptr (&r->a) + off);
+  uint4 oa = ld_overlay16 (ldg_ptr (&r->a) + off);
+  if (GA)
+    oa = scale16_alpha (oa, (uint32_t) __ldg (&r->a_ga));
   if (KIND == PK_PLANE8) {
     const uint4 oc = ld_overlay16 (ldg_ptr (&r->c) + off);
     return blend16_plane8 (f, oa, oc);
@@ -464,7 +484,7 @@ all_opaque (const uint4 &oa)
  * overlay first and touches only the vectors it will change: a vector whose
  * alpha is zero everywhere is neither loaded nor stored -- for cues without a
  * background box most of the region never crosses the bus. */
-template <int KIND, bool FAST, bool BULK, int LAZY = 0>
+template <int KIND, bool FAST, bool BULK, int LAZY = 0, bool GA = false>
 __device__ __forceinline__ void
 process_chunk (const JobRegs &J, uint32_t local_chunk)
 {
@@ -540,6 +560,7 @@ process_chunk (const JobRegs &J, uint32_t local_chunk)
           "bra OV_WAIT;\n"
           "OV_DONE:\n"
           "}" :: "r" (bar) : "memory");
+      const uint32_t a_ga = GA ? (uint32_t) __ldg (&r->a_ga) : 255u;
       if (LAZY) {
         /* overlay first. LAZY 1 (in place): only vectors with some alpha are written back, and
          * of those only the ones that are not opaque all over are fetched (all fetches in flight
@@ -552,7 +573,9 @@ process_chunk (const JobRegs &J, uint32_t local_chunk)
         const uint32_t fill = KIND == PK_PACKED_A0 ? 0x000000ffu : KIND == PK_PACKED_A3 ? 0xff000000u : 0u;
 #pragma unroll
         for (int k = 0; k < kUnroll; k++) {
-          const uint4 oa = *reinterpret_cast<const uint4 *> (ov_smem + (threadIdx.x + k * kThreads) * 16u);
+          uint4 oa = *reinterpret_cast<const uint4 *> (ov_smem + (threadIdx.x + k * kThreads) * 16u);
+          if (GA)
+            oa = scale16_alpha (oa, a_ga);      /* effective alpha: opaque only where a_ga is 255 too */
           if (LAZY == 1)
             act[k] = act[k] && any_alpha<KIND> (oa);
           f[k] = make_uint4 (fill, fill, fill, fill);
@@ -567,7 +590,9 @@ process_chunk (const JobRegs &J, uint32_t local_chunk)
       for (int k = 0; k < kUnroll; k++)
         if (act[k]) {
           const uint32_t so = (threadIdx.x + k * kThreads) * 16u;
-          const uint4 oa = *reinterpret_cast<const uint4 *> (ov_smem + so);
+          uint4 oa = *reinterpret_cast<const uint4 *> (ov_smem + so);
+          if (GA)
+            oa = scale16_alpha (oa, a_ga);
           uint4 out;
           if (KIND == PK_PLANE8) {
             const uint4 oc = *reinterpret_cast<const uint4 *> (ov_smem + kItemsPerChunk * 16 + so);
@@ -598,12 +623,15 @@ process_chunk (const JobRegs &J, uint32_t local_chunk)
         const uint8_t *pc = ldg_ptr (&r->c);
         const uint32_t ga1 = KIND == PK_PLANE8 ? 255u : (uint32_t) __ldg (&r->ga);
         const bool sp1 = KIND == PK_PLANE8 ? false : __ldg (&r->src_premul) != 0;
+        const uint32_t a_ga = GA ? (uint32_t) __ldg (&r->a_ga) : 255u;
 #pragma unroll
         for (int k = 0; k < kUnroll; k++)
           if (act[k]) {
             const size_t off = (size_t) (yy[k] - g.y0) * pitch + (size_t) (vv[k] - g.v0) * 16;
             oa[k] = ld_overlay16 (pa + off);
             oc[k] = ld_overlay16 (pc + off);
+            if (GA)
+              oa[k] = scale16_alpha (oa[k], a_ga);
           }
 #pragma unroll
         for (int k = 0; k < kUnroll; k++)
@@ -650,11 +678,15 @@ process_chunk (const JobRegs &J, uint32_t local_chunk)
       if (LAZY == 1) {
         const int32_t pitch = __ldg (&r->pitch);
         const uint8_t *pa = ldg_ptr (&r->a);
+        const uint32_t a_ga = GA ? (uint32_t) __ldg (&r->a_ga) : 255u;
 #pragma unroll
         for (int k = 0; k < kUnroll; k++)
-          if (act[k] && !hit[k] && vv[k] >= g.v0 && vv[k] < g.v1)
-            hit[k] = any_alpha<KIND> (ld_overlay16 (pa + (size_t) (yy[k] - g.y0) * pitch +
-                    (size_t) (vv[k] - g.v0) * 16));
+          if (act[k] && !hit[k] && vv[k] >= g.v0 && vv[k] < g.v1) {
+            uint4 oa = ld_overlay16 (pa + (size_t) (yy[k] - g.y0) * pitch + (size_t) (vv[k] - g.v0) * 16);
+            if (GA)
+              oa = scale16_alpha (oa, a_ga);
+            hit[k] = any_alpha<KIND> (oa);
+          }
       } else {
 #pragma unroll
         for (int k = 0; k < kUnroll; k++)
@@ -686,7 +718,7 @@ process_chunk (const JobRegs &J, uint32_t local_chunk)
 #pragma unroll
     for (int k = 0; k < kUnroll; k++)
       if (act[k] && vv[k] >= g.v0 && vv[k] < g.v1)
-        f[k] = blend_with_rect<KIND> (f[k], r, g, vv[k], yy[k], dst_premul);
+        f[k] = blend_with_rect<KIND, GA> (f[k], r, g, vv[k], yy[k], dst_premul);
   }
 
 #pragma unroll
@@ -714,7 +746,7 @@ process_chunk (const JobRegs &J, uint32_t local_chunk)
 #define TTMLBLEND_MIN_CTAS 5
 #endif
 
-template <int KIND, bool FAST>
+template <int KIND, bool FAST, bool GA = false>
 __global__ void __launch_bounds__ (kThreads, FAST ? 4 : 2)
 ttmlblend_blend_kernel (const PlaneJob *__restrict__ jobs,
     const uint32_t *__restrict__ chunk_begin, const uint32_t *__restrict__ coarse, int n_jobs,
@@ -738,7 +770,7 @@ ttmlblend_blend_kernel (const PlaneJob *__restrict__ jobs,
   while (j + 1u < (uint32_t) n_jobs && __ldg (chunk_begin + j + 1u) <= chunk)
     j++;
   const JobRegs J = load_job (jobs + j);
-  process_chunk<KIND, FAST, false> (J, chunk - __ldg (chunk_begin + j));
+  process_chunk<KIND, FAST, false, 0, GA> (J, chunk - __ldg (chunk_begin + j));
   pdl_end (sync);
 }
 
@@ -751,7 +783,7 @@ ttmlblend_blend_kernel (const PlaneJob *__restrict__ jobs,
  * first frame load without a single dependent global load or barrier in
  * front of it (the table search of the generic kernel above costs ~8 % of a
  * streaming copy: tools/copybench.cu "+prologue"). */
-template <int KIND, int LAZY, int NF, int NB>
+template <int KIND, int LAZY, int NF, int NB, bool GA = false>
 __global__ void __launch_bounds__ (kThreads, LAZY == 1 ? 4 : TTMLBLEND_MIN_CTAS)
 ttmlblend_group_kernel (const __grid_constant__ GroupParamsT<NF, NB> P)
 {
@@ -790,7 +822,7 @@ ttmlblend_group_kernel (const __grid_constant__ GroupParamsT<NF, NB> P)
   J.one_rect = B.one_rect;
   J.flags = Hd.flags;
   J.row_bytes = 0;              /* FAST: never read */
-  process_chunk<KIND, true, true, LAZY> (J, cif - B.chunk_begin);
+  process_chunk<KIND, true, true, LAZY, GA> (J, cif - B.chunk_begin);
   pdl_end (Hd.flags);
 }
 
@@ -799,7 +831,7 @@ ttmlblend_group_kernel (const __grid_constant__ GroupParamsT<NF, NB> P)
  * uses. A CTA finds its frame by bisecting the frames' first chunks (six uniform
  * constant-bank reads), then its band as above -- still no global load and no barrier before
  * the first frame load. */
-template <int KIND, int LAZY>
+template <int KIND, int LAZY, bool GA = false>
 __global__ void __launch_bounds__ (kThreads, LAZY == 1 ? 4 : TTMLBLEND_MIN_CTAS)
 ttmlblend_multi_kernel (const __grid_constant__ MultiParams P)
 {
@@ -843,7 +875,7 @@ ttmlblend_multi_kernel (const __grid_constant__ MultiParams P)
   J.one_rect = B.one_rect;
   J.flags = P.flags;
   J.row_bytes = 0;              /* FAST: never read */
-  process_chunk<KIND, true, true, LAZY> (J, cif - B.chunk_begin);
+  process_chunk<KIND, true, true, LAZY, GA> (J, cif - B.chunk_begin);
   pdl_end (P.flags);
 }
 
@@ -867,7 +899,7 @@ interleave_lanes (int kind)
   return kind_is_planes (kind) ? 1u : 61u;
 }
 
-template <int KIND>
+template <int KIND, bool GA = false>
 static cudaError_t
 launch_blend_kind (const PlaneJob *d_jobs, const uint32_t *d_chunk_begin, const uint32_t *d_coarse, int n_jobs,
     uint32_t total_chunks, bool fast, int sync, cudaStream_t stream)
@@ -883,39 +915,50 @@ launch_blend_kind (const PlaneJob *d_jobs, const uint32_t *d_chunk_begin, const 
   const uint32_t magic = lanes == 1 ? 0u : (uint32_t) (((1ull << 32) + lanes - 1) / lanes);
   const bool pdl = (sync & JF_PDL) != 0;
   if (fast)
-    return launch_ex (ttmlblend_blend_kernel<KIND, true>, grid, 0, stream, pdl, d_jobs, d_chunk_begin, d_coarse,
+    return launch_ex (ttmlblend_blend_kernel<KIND, true, GA>, grid, 0, stream, pdl, d_jobs, d_chunk_begin, d_coarse,
         n_jobs, total_chunks, lanes, per_lane, magic, sync);
-  return launch_ex (ttmlblend_blend_kernel<KIND, false>, grid, 0, stream, pdl, d_jobs, d_chunk_begin, d_coarse,
+  return launch_ex (ttmlblend_blend_kernel<KIND, false, GA>, grid, 0, stream, pdl, d_jobs, d_chunk_begin, d_coarse,
       n_jobs, total_chunks, lanes, per_lane, magic, sync);
 }
 
 /* One variant of the group kernel: copies what the launch needs into a parameter block of the
  * variant's size (the full-size block itself when NF / NB are the maxima). */
-template <int KIND, int LAZY, int NF, int NB>
+template <int KIND, int LAZY, int NF, int NB, bool GA>
 static cudaError_t
 launch_group_variant (const GroupParams &P, uint32_t grid, size_t smem, cudaStream_t stream)
 {
   const bool pdl = (P.h.flags & JF_PDL) != 0;
   if (NF == kMaxPlainGroupFrames && NB == kMaxGroupBands)
-    return launch_ex (ttmlblend_group_kernel<KIND, LAZY, kMaxPlainGroupFrames, kMaxGroupBands>, grid, smem, stream,
+    return launch_ex (ttmlblend_group_kernel<KIND, LAZY, kMaxPlainGroupFrames, kMaxGroupBands, GA>, grid, smem, stream,
         pdl, P);
   GroupParamsT<NF, NB> S;
   S.h = P.h;
   memcpy (S.bands, P.bands, P.h.n_bands * sizeof (BandDesc));
   memcpy (S.frames, P.frames, P.h.n_frames * sizeof (FramePtrs));
-  return launch_ex (ttmlblend_group_kernel<KIND, LAZY, NF, NB>, grid, smem, stream, pdl, S);
+  return launch_ex (ttmlblend_group_kernel<KIND, LAZY, NF, NB, GA>, grid, smem, stream, pdl, S);
 }
 
-template <int KIND, int LAZY>
+template <int KIND, int LAZY, bool GA = false>
 static cudaError_t
 launch_group_sized (const GroupParams &P, uint32_t grid, size_t smem, cudaStream_t stream)
 {
   static const bool compact = !getenv ("FLUC_TTMLBLEND_COMPACT_PARAMS") || atoi (getenv ("FLUC_TTMLBLEND_COMPACT_PARAMS")) != 0;
   if (compact && P.h.n_frames <= 4u && P.h.n_bands <= 16u)
-    return launch_group_variant<KIND, LAZY, 4, 16> (P, grid, smem, stream);
+    return launch_group_variant<KIND, LAZY, 4, 16, GA> (P, grid, smem, stream);
   if (compact && P.h.n_frames <= 32u)
-    return launch_group_variant<KIND, LAZY, 32, kMaxGroupBands> (P, grid, smem, stream);
-  return launch_group_variant<KIND, LAZY, kMaxPlainGroupFrames, kMaxGroupBands> (P, grid, smem, stream);
+    return launch_group_variant<KIND, LAZY, 32, kMaxGroupBands, GA> (P, grid, smem, stream);
+  return launch_group_variant<KIND, LAZY, kMaxPlainGroupFrames, kMaxGroupBands, GA> (P, grid, smem, stream);
+}
+
+/* The JF_GA variants exist for the PLANE8 kinds only (the packed kinds apply RectRef::ga in every
+ * variant). */
+template <int KIND, int LAZY>
+static cudaError_t
+launch_group_ga (const GroupParams &P, uint32_t grid, size_t smem, cudaStream_t stream)
+{
+  if (kind_is_planes (KIND) && (P.h.flags & JF_GA))
+    return launch_group_sized<KIND, LAZY, kind_is_planes (KIND)> (P, grid, smem, stream);
+  return launch_group_sized<KIND, LAZY> (P, grid, smem, stream);
 }
 
 cudaError_t
@@ -942,8 +985,8 @@ launch_group (GroupParams &P, int kind, int sync, cudaStream_t stream)
   const int look = (Hd.flags & JF_LAZY) ? 1 : (Hd.flags & JF_OPAQUE) ? 2 : 0;
 #define GROUP_CASE(K, SM) \
     case K: \
-      return look == 1 ? launch_group_sized<K, 1> (P, grid, SM, stream) : \
-          look == 2 ? launch_group_sized<K, 2> (P, grid, SM, stream) : launch_group_sized<K, 0> (P, grid, SM, stream);
+      return look == 1 ? launch_group_ga<K, 1> (P, grid, SM, stream) : \
+          look == 2 ? launch_group_ga<K, 2> (P, grid, SM, stream) : launch_group_ga<K, 0> (P, grid, SM, stream);
   switch (kind) {
     GROUP_CASE (PK_PLANE8, smem_plane8)
     GROUP_CASE (PK_PLANE8_RGB, smem_plane8)
@@ -974,8 +1017,13 @@ launch_multi (MultiParams &P, int kind, int sync, cudaStream_t stream)
   const size_t smem_plane8 = 2 * kItemsPerChunk * 16, smem_packed = kItemsPerChunk * 16;
   const int look = (P.flags & JF_LAZY) ? 1 : (P.flags & JF_OPAQUE) ? 2 : 0;
   const bool pdl = (P.flags & JF_PDL) != 0;
+  const bool ga = (P.flags & JF_GA) != 0;
 #define MULTI_CASE(K, SM) \
     case K: \
+      if (kind_is_planes (K) && ga) \
+        return look == 1 ? launch_ex (ttmlblend_multi_kernel<K, 1, kind_is_planes (K)>, grid, SM, stream, pdl, P) : \
+            look == 2 ? launch_ex (ttmlblend_multi_kernel<K, 2, kind_is_planes (K)>, grid, SM, stream, pdl, P) : \
+            launch_ex (ttmlblend_multi_kernel<K, 0, kind_is_planes (K)>, grid, SM, stream, pdl, P); \
       return look == 1 ? launch_ex (ttmlblend_multi_kernel<K, 1>, grid, SM, stream, pdl, P) : \
           look == 2 ? launch_ex (ttmlblend_multi_kernel<K, 2>, grid, SM, stream, pdl, P) : \
           launch_ex (ttmlblend_multi_kernel<K, 0>, grid, SM, stream, pdl, P);
@@ -992,14 +1040,19 @@ launch_multi (MultiParams &P, int kind, int sync, cudaStream_t stream)
 
 cudaError_t
 launch_blend (const PlaneJob *d_jobs, const uint32_t *d_chunk_begin, const uint32_t *d_coarse, int n_jobs,
-    uint32_t total_chunks, int kind, bool fast, int sync, cudaStream_t stream)
+    uint32_t total_chunks, int kind, bool fast, bool ga, int sync, cudaStream_t stream)
 {
   if (n_jobs <= 0 || total_chunks == 0)
     return cudaSuccess;
   switch (kind) {
     case PK_PLANE8:
+      if (ga)
+        return launch_blend_kind<PK_PLANE8, true> (d_jobs, d_chunk_begin, d_coarse, n_jobs, total_chunks, fast, sync, stream);
       return launch_blend_kind<PK_PLANE8> (d_jobs, d_chunk_begin, d_coarse, n_jobs, total_chunks, fast, sync, stream);
     case PK_PLANE8_RGB:
+      if (ga)
+        return launch_blend_kind<PK_PLANE8_RGB, true> (d_jobs, d_chunk_begin, d_coarse, n_jobs, total_chunks, fast, sync,
+            stream);
       return launch_blend_kind<PK_PLANE8_RGB> (d_jobs, d_chunk_begin, d_coarse, n_jobs, total_chunks, fast, sync, stream);
     case PK_PACKED_A0:
       return launch_blend_kind<PK_PACKED_A0> (d_jobs, d_chunk_begin, d_coarse, n_jobs, total_chunks, fast, sync, stream);

@@ -54,7 +54,9 @@ enum JobFlags : int32_t {
    *           that) before they touch anything. */
   JF_DEP = 32,
   JF_PDL = 64,
-  JF_OPAQUE = 128       /* host-side, group launches out of place: overlay first, no frame read under opaque vectors */
+  JF_OPAQUE = 128,      /* host-side, group launches out of place: overlay first, no frame read under opaque vectors */
+  JF_GA = 256           /* host-side, PLANE8 kinds: the launch holds a rectangle with RectRef::a_ga != 255 -> the
+                         * variant that scales the prepared alpha bytes (overlay_set_global_alpha) */
 };
 
 /* One prepared rectangle as seen from one destination plane. */
@@ -64,9 +66,10 @@ struct alignas (16) RectRef {
   int32_t v0, v1;       /* 16-byte vector columns [v0, v1) of the plane row */
   int32_t y0, y1;       /* plane rows [y0, y1); v0..y1 are read as one int4 */
   int32_t pitch;        /* bytes per prepared row, multiple of 16 */
-  int32_t ga;           /* PACKED: global alpha 0..255 (PLANE8 folds it in) */
+  int32_t ga;           /* global alpha 0..255 of the Cs*ga terms (PACKED, PLANE8_RGB premultiplied) */
   int32_t src_premul;   /* PACKED: source colours are premultiplied */
-  int32_t pad_;
+  int32_t a_ga;         /* PLANE8 kinds: global alpha the blend still applies to the alpha bytes, asrc =
+                         * a*a_ga/255 (JF_GA launches). 255 when it is 1 or the prepare folded it in */
 };
 
 enum JobClass : int32_t {
@@ -218,9 +221,11 @@ enum PrepareMode : int32_t {
 /* d_coarse[i] = index of the job that holds chunk i << kCoarseShift. */
 constexpr int kCoarseShift = 4;
 /* sync = JF_PDL / JF_DEP bits of this launch (0: an ordinary, fully serialised launch) */
+/* ga: some job carries JF_GA (PLANE8 kinds): the variant that scales the prepared alpha bytes */
 cudaError_t launch_blend (const PlaneJob *d_jobs, const uint32_t *d_chunk_begin, const uint32_t *d_coarse,
-    int n_jobs, uint32_t total_chunks, int kind, bool fast, int sync, cudaStream_t stream);
-/* Fills in total_chunks and the interleave fields of P, then launches. */
+    int n_jobs, uint32_t total_chunks, int kind, bool fast, bool ga, int sync, cudaStream_t stream);
+/* Fills in total_chunks and the interleave fields of P, then launches (the JF_GA variant when
+ * P's flags carry it). */
 cudaError_t launch_group (GroupParams &P, int kind, int sync, cudaStream_t stream);
 /* Fills in total_chunks (from frame_begin[n_frames]) and the interleave fields, then launches. */
 cudaError_t launch_multi (MultiParams &P, int kind, int sync, cudaStream_t stream);

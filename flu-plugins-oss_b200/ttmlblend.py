@@ -98,6 +98,8 @@ PROTOTYPES = {
     "fluc_ttmlblend_overlay_set_regions": (C.c_int, [C.c_void_p, C.c_uint32, C.c_int32, C.c_int32,
                                                      C.POINTER(Region), C.c_uint32]),
     "fluc_ttmlblend_overlay_clear": (C.c_int, [C.c_void_p, C.c_uint32]),
+    "fluc_ttmlblend_overlay_set_global_alpha": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_float),
+                                                          C.c_uint32]),
     "fluc_ttmlblend_set_chroma_mode": (C.c_int, [C.c_void_p, C.c_int]),
     "fluc_ttmlblend_submit": (C.c_int, [C.c_void_p, C.c_uint32, C.c_int, C.c_int32, C.c_int32,
                                         C.c_uint32, C.POINTER(Frame), C.POINTER(Frame),
@@ -355,6 +357,16 @@ class TtmlBlend:
 
     def overlay_clear(self, stream: int):
         self._check(self.lib.fluc_ttmlblend_overlay_clear(self.h, stream), "overlay_clear")
+
+    def overlay_set_global_alpha(self, stream: int, alphas):
+        """gst_video_overlay_rectangle_set_global_alpha for the stream's current overlay, without a
+        new upload or prepare. `alphas`: one float for every rectangle, or a sequence with one value
+        per rectangle the overlay was installed with (overlay_set_rectangles: list order;
+        overlay_set: its region boxes). Frames submitted afterwards blend with the new values."""
+        vals = [float(alphas)] if np.ndim(alphas) == 0 else [float(a) for a in alphas]
+        arr = (C.c_float * max(1, len(vals)))(*vals)
+        self._check(self.lib.fluc_ttmlblend_overlay_set_global_alpha(self.h, stream, arr, len(vals)),
+                    "overlay_set_global_alpha")
 
     def set_chroma_mode(self, average: bool):
         """False (default): GStreamer's sited chroma, bit-exact. True: 2x2 mean, NOT bit-exact."""

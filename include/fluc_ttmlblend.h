@@ -247,6 +247,25 @@ FLUC_EXPORT int fluc_ttmlblend_overlay_set_regions (FlucTtmlBlend *thiz, uint32_
  * (/root/reference/plugins/ttml/gstttmlevent.c:221-224): frames pass through. */
 FLUC_EXPORT int fluc_ttmlblend_overlay_clear (FlucTtmlBlend *thiz, uint32_t stream);
 
+/* gst_video_overlay_rectangle_set_global_alpha for the stream's current overlay, without a new
+ * upload or prepare: a fade costs a few hundred bytes of rectangle tables instead of a cue change.
+ * n == 1: every rectangle gets global_alpha[0]. Otherwise n == the number of rectangles the
+ * overlay was installed with, one value each: overlay_set_rectangles: the list, in order (also
+ * rectangles that lie outside the frame); overlay_set: its region boxes as installed, i.e.
+ * clipped to the image, overlapping boxes split into disjoint ones (1 without boxes);
+ * overlay_set_regions: 1, its regions are composed into one image first. Values in [0, 1].
+ * Replaces the values, as set_global_alpha does. Frames submitted after the call (submit*,
+ * submit_many_after, blend_host*) are blended exactly as gst_video_blend does with those global
+ * alphas (ga = (int) (255.0 * global_alpha)); frames already submitted keep theirs.
+ * overlay_update keeps the current values when it patches the overlay (when it falls back to
+ * installing the whole image, that starts at 1); overlay_set* / overlay_clear start again from
+ * the new cue's own values. A rectangle installed with a global alpha below 1 is prepared once
+ * more the first time its value changes.
+ * Returns NOT_FOUND when the stream has no overlay, INVALID_ARGUMENT for a wrong n, NULL, NaN or
+ * a value outside [0, 1]. */
+FLUC_EXPORT int fluc_ttmlblend_overlay_set_global_alpha (FlucTtmlBlend *thiz, uint32_t stream,
+    const float *global_alpha, uint32_t n);
+
 /* How the overlay reaches the chroma planes of 4:2:0 frames. SITED (default) is what
  * GStreamer does and the only bit-exact mode: a chroma sample takes the overlay pixel at
  * (even x, even y). AVERAGE is an explicit NON-PARITY option: the alpha-weighted mean of
