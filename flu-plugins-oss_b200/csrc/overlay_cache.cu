@@ -47,9 +47,12 @@ Overlay::~Overlay ()
   for (RawRect &r : rects)
     take (r.block);
   for (auto &p : prepared) {
-    for (PreparedRect &pr : p->per_rect)
+    for (PreparedRect &pr : p->per_rect) {
       for (auto &b : pr.blocks)
         take (b);
+      for (auto &b : pr.avg_blocks)
+        take (b);
+    }
     take (p->table_block);
     if (p->ready)
       cudaEventDestroy (p->ready);
@@ -75,14 +78,14 @@ dev_block (Ctx *c, size_t bytes, std::shared_ptr<DevBlock> *out)
 }
 
 static int
-dev_alloc (Ctx *c, PreparedRect *pr, size_t bytes, uint8_t **out)
+dev_alloc (Ctx *c, std::vector<std::shared_ptr<DevBlock>> *blocks, size_t bytes, uint8_t **out)
 {
   std::shared_ptr<DevBlock> b;
   int rc = dev_block (c, bytes, &b);
   if (rc)
     return rc;
   *out = static_cast<uint8_t *> (b->ptr);
-  pr->blocks.push_back (std::move (b));
+  blocks->push_back (std::move (b));
   return 0;
 }
 
@@ -112,22 +115,17 @@ prepare_overlay (Ctx *c, Overlay *ov, int format, int W, int H, Prepared **out)
   return 0;
 }
 
-/* Prepares one rectangle for one destination format: allocates its planes, runs the prepare
- * kernel(s) on the upload stream, and notes how each destination plane sees it. */
-static int
-prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_average, PreparedRect &out)
+/* The prepare parameters every plane of a rectangle shares; false when nothing of it is inside
+ * the frame. */
+static bool
+rect_params (const RawRect &rr, int format, int W, int H, PrepareParams &pp)
 {
-  const int kind = plane_kind (format);
-  const int n_planes = format_planes (format);
   /* gst_video_blend clipping: rr is already clipped at the left/top */
   const int cx0 = rr.x, cy0 = rr.y;
   const int cx1 = std::min (rr.x + rr.w, W), cy1 = std::min (rr.y + rr.h, H);
   if (cx1 <= cx0 || cy1 <= cy0)
-    return 0;
-  if (rr.ga == 0)
-    return 0;                 /* asrc == 0 everywhere: blends nothing */
-
-  PrepareParams pp = {};
+    return false;
+  pp = {};
   pp.raw = rr.dev;
   pp.raw_pitch = rr.pitch;
   pp.raw_w = rr.w;
@@ -137,9 +135,112 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
   pp.cx0 = cx0; pp.cy0 = cy0; pp.cx1 = cx1; pp.cy1 = cy1;
   pp.ga = rr.ga;
   pp.premul = rr.premul ? 1 : 0;
-
   pp.sub_x = format_sub_x (format);
   pp.sub_y = format_sub_y (format);
+  return true;
+}
+
+/* The chroma planes of a planar / semi-planar YUV format: the samples sited on the even pixel
+ * of each pair / the even line of each line pair, as far as the format subsamples (parity);
+ * with the non-parity 2x2 average of 4:2:0 (avg) every sample with at least one covered pixel.
+ * Their planes go to `blocks`. */
+static int
+prepare_chroma (Ctx *c, PrepareParams pp, int format, bool avg, std::vector<std::shared_ptr<DevBlock>> *blocks,
+    PreparedRect &out)
+{
+  const int n_planes = format_planes (format);
+  const int sx = pp.sub_x, sy = pp.sub_y;
+  pp.chroma_average = avg ? 1 : 0;
+  const int bx0 = avg ? pp.cx0 / 2 : ceil_div (pp.cx0, sx), bx1 = ceil_div (pp.cx1, sx);
+  const int by0 = avg ? pp.cy0 / 2 : ceil_div (pp.cy0, sy), by1 = ceil_div (pp.cy1, sy);
+  if (n_planes < 2 || bx1 <= bx0 || by1 <= by0)
+    return 0;
+  if (n_planes == 3) {
+    RectRef ref = {};
+    ref.v0 = bx0 / 16;
+    ref.v1 = ceil_div (bx1, 16);
+    ref.y0 = by0;
+    ref.y1 = by1;
+    ref.pitch = (ref.v1 - ref.v0) * 16;
+    ref.ga = 255;
+    const size_t bytes = (size_t) ref.pitch * (by1 - by0);
+    uint8_t *a, *u, *v;
+    int rc;
+    if ((rc = dev_alloc (c, blocks, bytes, &a)) || (rc = dev_alloc (c, blocks, bytes, &u))
+        || (rc = dev_alloc (c, blocks, bytes, &v)))
+      return rc;
+    pp.mode = PM_CHROMA_PLANAR;
+    pp.out_a = a; pp.out_c = u; pp.out_c2 = v;
+    pp.out_pitch = ref.pitch;
+    pp.v0 = ref.v0;
+    pp.row0 = by0;
+    pp.rows = by1 - by0;
+    CU (c, launch_prepare (pp, ref.pitch, c->up_stream));
+    c->stats.prepare_launches++;
+    const int pu = format == FLUC_TTMLBLEND_FORMAT_YV12 ? 2 : 1;
+    const int pv = 3 - pu;
+    ref.a = a;
+    ref.c = u;
+    out.refs[out.n_refs++] = { pu, ref };
+    ref.c = v;
+    out.refs[out.n_refs++] = { pv, ref };
+  } else {
+    RectRef ref = {};
+    ref.v0 = (2 * bx0) / 16;
+    ref.v1 = ceil_div (2 * bx1, 16);
+    ref.y0 = by0;
+    ref.y1 = by1;
+    ref.pitch = (ref.v1 - ref.v0) * 16;
+    ref.ga = 255;
+    const size_t bytes = (size_t) ref.pitch * (by1 - by0);
+    uint8_t *a, *uv;
+    int rc;
+    if ((rc = dev_alloc (c, blocks, bytes, &a)) || (rc = dev_alloc (c, blocks, bytes, &uv)))
+      return rc;
+    pp.mode = (format == FLUC_TTMLBLEND_FORMAT_NV21 || format == FLUC_TTMLBLEND_FORMAT_NV61) ?
+        PM_CHROMA_VU : PM_CHROMA_UV;
+    pp.out_a = a; pp.out_c = uv; pp.out_c2 = nullptr;
+    pp.out_pitch = ref.pitch;
+    pp.v0 = ref.v0;
+    pp.row0 = by0;
+    pp.rows = by1 - by0;
+    CU (c, launch_prepare (pp, ref.pitch / 2, c->up_stream));
+    c->stats.prepare_launches++;
+    ref.a = a;
+    ref.c = uv;
+    out.refs[out.n_refs++] = { 1, ref };
+  }
+  return 0;
+}
+
+/* Averaged 4:2:0 chroma at the box's global alpha `ga`: asrc = a*ga/255 per pixel before the
+ * 2x2 sums (BLENDSPEC section 7), so unlike every other PLANE8 plane the value is folded in
+ * here and the blend leaves these refs alone. Nothing at 0: the box is not blended. */
+static int
+prepare_avg_chroma (Ctx *c, PrepareParams pp, int format, int ga, PreparedRect &out)
+{
+  out.avg_ga = ga;
+  if (ga == 0)
+    return 0;
+  pp.ga = ga;
+  return prepare_chroma (c, pp, format, true, &out.avg_blocks, out);
+}
+
+/* Prepares one rectangle for one destination format: allocates its planes, runs the prepare
+ * kernel(s) on the upload stream, and notes how each destination plane sees it. ga_now is the
+ * current global alpha of its box, which only averaged chroma folds in. */
+static int
+prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_average, int ga_now,
+    PreparedRect &out)
+{
+  const int kind = plane_kind (format);
+  PrepareParams pp;
+  if (!rect_params (rr, format, W, H, pp))
+    return 0;
+  if (rr.ga == 0)
+    return 0;                 /* asrc == 0 everywhere: blends nothing */
+  const int cx0 = pp.cx0, cy0 = pp.cy0, cx1 = pp.cx1, cy1 = pp.cy1;
+
   if (kind == PK_PLANE8 && format_packed_422 (format)) {
     /* YUY2 / UYVY: one plane of macropixels, every byte gets its own alpha + colour */
     RectRef ref = {};
@@ -152,7 +253,7 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
     const size_t bytes = (size_t) ref.pitch * (cy1 - cy0);
     uint8_t *a, *col;
     int rc;
-    if ((rc = dev_alloc (c, &out, bytes, &a)) || (rc = dev_alloc (c, &out, bytes, &col)))
+    if ((rc = dev_alloc (c, &out.blocks, bytes, &a)) || (rc = dev_alloc (c, &out.blocks, bytes, &col)))
       return rc;
     ref.a = a;
     ref.c = col;
@@ -179,7 +280,7 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
     const size_t bytes = (size_t) ref.pitch * (cy1 - cy0);
     uint8_t *a, *col;
     int rc;
-    if ((rc = dev_alloc (c, &out, bytes, &a)) || (rc = dev_alloc (c, &out, bytes, &col)))
+    if ((rc = dev_alloc (c, &out.blocks, bytes, &a)) || (rc = dev_alloc (c, &out.blocks, bytes, &col)))
       return rc;
     ref.a = a;
     ref.c = col;
@@ -210,7 +311,7 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
       const size_t bytes = (size_t) ref.pitch * (cy1 - cy0);
       uint8_t *a, *y;
       int rc;
-      if ((rc = dev_alloc (c, &out, bytes, &a)) || (rc = dev_alloc (c, &out, bytes, &y)))
+      if ((rc = dev_alloc (c, &out.blocks, bytes, &a)) || (rc = dev_alloc (c, &out.blocks, bytes, &y)))
         return rc;
       ref.a = a;
       ref.c = y;
@@ -224,71 +325,9 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
       c->stats.prepare_launches++;
       out.refs[out.n_refs++] = { 0, ref };
     }
-    /* chroma: the samples sited on the even pixel of each pair / the even line of each
-     * line pair, as far as the format subsamples (parity); with the non-parity 2x2 average
-     * of 4:2:0 every sample with at least one covered pixel */
-    const int sx = pp.sub_x, sy = pp.sub_y;
-    const bool avg = chroma_average && sx == 2 && sy == 2;
-    pp.chroma_average = avg ? 1 : 0;
-    const int bx0 = avg ? cx0 / 2 : ceil_div (cx0, sx), bx1 = ceil_div (cx1, sx);
-    const int by0 = avg ? cy0 / 2 : ceil_div (cy0, sy), by1 = ceil_div (cy1, sy);
-    if (n_planes >= 2 && bx1 > bx0 && by1 > by0) {
-      if (n_planes == 3) {
-        RectRef ref = {};
-        ref.v0 = bx0 / 16;
-        ref.v1 = ceil_div (bx1, 16);
-        ref.y0 = by0;
-        ref.y1 = by1;
-        ref.pitch = (ref.v1 - ref.v0) * 16;
-        ref.ga = 255;
-        const size_t bytes = (size_t) ref.pitch * (by1 - by0);
-        uint8_t *a, *u, *v;
-        int rc;
-        if ((rc = dev_alloc (c, &out, bytes, &a)) || (rc = dev_alloc (c, &out, bytes, &u))
-            || (rc = dev_alloc (c, &out, bytes, &v)))
-          return rc;
-        pp.mode = PM_CHROMA_PLANAR;
-        pp.out_a = a; pp.out_c = u; pp.out_c2 = v;
-        pp.out_pitch = ref.pitch;
-        pp.v0 = ref.v0;
-        pp.row0 = by0;
-        pp.rows = by1 - by0;
-        CU (c, launch_prepare (pp, ref.pitch, c->up_stream));
-        c->stats.prepare_launches++;
-        const int pu = format == FLUC_TTMLBLEND_FORMAT_YV12 ? 2 : 1;
-        const int pv = 3 - pu;
-        ref.a = a;
-        ref.c = u;
-        out.refs[out.n_refs++] = { pu, ref };
-        ref.c = v;
-        out.refs[out.n_refs++] = { pv, ref };
-      } else {
-        RectRef ref = {};
-        ref.v0 = (2 * bx0) / 16;
-        ref.v1 = ceil_div (2 * bx1, 16);
-        ref.y0 = by0;
-        ref.y1 = by1;
-        ref.pitch = (ref.v1 - ref.v0) * 16;
-        ref.ga = 255;
-        const size_t bytes = (size_t) ref.pitch * (by1 - by0);
-        uint8_t *a, *uv;
-        int rc;
-        if ((rc = dev_alloc (c, &out, bytes, &a)) || (rc = dev_alloc (c, &out, bytes, &uv)))
-          return rc;
-        pp.mode = (format == FLUC_TTMLBLEND_FORMAT_NV21 || format == FLUC_TTMLBLEND_FORMAT_NV61) ?
-            PM_CHROMA_VU : PM_CHROMA_UV;
-        pp.out_a = a; pp.out_c = uv; pp.out_c2 = nullptr;
-        pp.out_pitch = ref.pitch;
-        pp.v0 = ref.v0;
-        pp.row0 = by0;
-        pp.rows = by1 - by0;
-        CU (c, launch_prepare (pp, ref.pitch / 2, c->up_stream));
-        c->stats.prepare_launches++;
-        ref.a = a;
-        ref.c = uv;
-        out.refs[out.n_refs++] = { 1, ref };
-      }
-    }
+    if (chroma_average && pp.sub_x == 2 && pp.sub_y == 2)
+      return prepare_avg_chroma (c, pp, format, ga_now, out);
+    return prepare_chroma (c, pp, format, false, &out.blocks, out);
   } else {
     RectRef ref = {};
     ref.v0 = cx0 / 4;
@@ -302,7 +341,7 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
     const size_t bytes = (size_t) ref.pitch * (cy1 - cy0);
     uint8_t *w;
     int rc;
-    if ((rc = dev_alloc (c, &out, bytes, &w)))
+    if ((rc = dev_alloc (c, &out.blocks, bytes, &w)))
       return rc;
     switch (format) {
       case FLUC_TTMLBLEND_FORMAT_AYUV: pp.mode = PM_PACKED_AYUV; break;
@@ -327,7 +366,8 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
 
 /* The rectangle tables of P with every box's current global alpha: a box at 0 drops out (no
  * band, no window in place), the others give it to the blend where the prepare did not fold it
- * in -- RectRef::ga for the Cs*ga terms, RectRef::a_ga for the alpha bytes of the PLANE8 kinds. */
+ * in -- RectRef::ga for the Cs*ga terms, RectRef::a_ga for the alpha bytes of the PLANE8 kinds.
+ * Averaged 4:2:0 chroma has it folded in (prepare_avg_chroma). */
 static int
 prepare_assemble (Ctx *c, Prepared *P, const Overlay *ov)
 {
@@ -345,7 +385,7 @@ prepare_assemble (Ctx *c, Prepared *P, const Overlay *ov)
       for (int k = 0; k < pr.n_refs; k++) {
         RectRef ref = pr.refs[k].ref;
         ref.a_ga = 255;
-        if (!folded) {
+        if (!folded && !(pr.avg_ga >= 0 && pr.refs[k].plane != 0)) {
           if (kind != PK_PLANE8)
             ref.ga = b.ga;
           if (planes)
@@ -386,6 +426,16 @@ prepare_assemble (Ctx *c, Prepared *P, const Overlay *ov)
   return 0;
 }
 
+/* the current global alpha of the box that rectangle i of ov belongs to */
+static int
+box_ga (const Overlay *ov, size_t i)
+{
+  for (const OverlayBox &b : ov->boxes)
+    if (i >= b.first_rect && i < b.first_rect + b.n_rects)
+      return b.ga;
+  return ov->rects[i].ga;
+}
+
 static int
 prepare_build (Ctx *c, Overlay *ov, int format, int W, int H, std::unique_ptr<Prepared> &P)
 {
@@ -400,7 +450,7 @@ prepare_build (Ctx *c, Overlay *ov, int format, int W, int H, std::unique_ptr<Pr
   }
   P->per_rect.resize (ov->rects.size ());
   for (size_t i = 0; i < ov->rects.size (); i++) {
-    const int rc = prepare_rect (c, ov->rects[i], format, W, H, P->chroma_average, P->per_rect[i]);
+    const int rc = prepare_rect (c, ov->rects[i], format, W, H, P->chroma_average, box_ga (ov, i), P->per_rect[i]);
     if (rc)
       return rc;
   }
@@ -895,7 +945,8 @@ overlay_update_image (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream,
   std::vector<int> from_old;    /* new rectangle -> the old overlay's rectangle it is, or -1 */
   for (size_t b = 0; b < old->boxes.size (); b++) {
     if (touched[b]) {
-      /* new pixels, prepared without a global alpha; the box keeps its current one */
+      /* new pixels, prepared without a global alpha (but averaged chroma); the box keeps its
+       * current one */
       ups[b].slot = old->boxes[b].slot;
       ups[b].rr.ga = old->boxes[b].ga;
       append_box (c, nv.get (), ups[b], old->boxes.size ());
@@ -933,7 +984,8 @@ overlay_update_image (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream,
       if (from_old[i] >= 0)
         P->per_rect[i] = p->per_rect[(size_t) from_old[i]];
       else
-        rc = prepare_rect (c, nv->rects[i], P->format, P->W, P->H, P->chroma_average, P->per_rect[i]);
+        rc = prepare_rect (c, nv->rects[i], P->format, P->W, P->H, P->chroma_average, box_ga (nv.get (), i),
+            P->per_rect[i]);
     }
     if (!rc)
       rc = prepare_assemble (c, P.get (), nv.get ());
@@ -956,7 +1008,9 @@ overlay_update_image (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream,
  * stream and waited for through Prepared::ready like a cue change). Its layouts are built again
  * at the first frame and get the ids of equal band lists, so a fading stream's frames still share
  * launches. The PLANE8 kinds need the alpha bytes without a global alpha folded in: a box
- * installed below 1 is prepared once more from its raw pixels the first time it changes. */
+ * installed below 1 is prepared once more from its raw pixels the first time it changes.
+ * Averaged 4:2:0 chroma (chroma_average) holds the value itself: it is prepared again, alone,
+ * for every box whose value changed. */
 int
 overlay_set_alpha (Ctx *c, uint32_t stream, const int *ga, uint32_t n)
 {
@@ -1006,11 +1060,23 @@ overlay_set_alpha (Ctx *c, uint32_t stream, const int *ga, uint32_t n)
     P->per_rect.resize (nv->rects.size ());
     int rc = 0;
     for (size_t i = 0; i < nv->rects.size () && !rc; i++) {
+      const PreparedRect &was = p->per_rect[i];
+      const int v = box_ga (nv.get (), i);
+      PrepareParams pp;
       /* the packed kinds never fold the global alpha in; a rectangle installed at 0 was not prepared */
-      if (again[i] && (planes || old->rects[i].ga == 0))
-        rc = prepare_rect (c, nv->rects[i], P->format, P->W, P->H, P->chroma_average, P->per_rect[i]);
-      else
-        P->per_rect[i] = p->per_rect[i];
+      if (again[i] && (planes || old->rects[i].ga == 0)) {
+        rc = prepare_rect (c, nv->rects[i], P->format, P->W, P->H, P->chroma_average, v, P->per_rect[i]);
+      } else if (was.avg_ga >= 0 && was.avg_ga != v && rect_params (nv->rects[i], P->format, P->W, P->H, pp)) {
+        /* the luma planes as they were, the averaged chroma at the new value */
+        PreparedRect &pr = P->per_rect[i];
+        pr.blocks = was.blocks;
+        for (int k = 0; k < was.n_refs; k++)
+          if (was.refs[k].plane == 0)
+            pr.refs[pr.n_refs++] = was.refs[k];
+        rc = prepare_avg_chroma (c, pp, P->format, v, pr);
+      } else {
+        P->per_rect[i] = was;
+      }
     }
     if (!rc)
       rc = prepare_assemble (c, P.get (), nv.get ());

@@ -301,6 +301,11 @@ struct PreparedRect {
   std::vector<std::shared_ptr<DevBlock>> blocks;      /* alpha / colour planes or pixel words */
   struct { int plane; RectRef ref; } refs[3];
   int n_refs = 0;
+  /* chroma_average: the averaged 4:2:0 chroma refs (planes 1, 2) have the box's global alpha
+   * folded in, since the 2x2 mean weights colours by asrc (BLENDSPEC section 7). A fade prepares
+   * them again on their own, so their planes are kept apart from the luma's. */
+  std::vector<std::shared_ptr<DevBlock>> avg_blocks;
+  int avg_ga = -1;                     /* the global alpha folded into them; -1: no averaged chroma */
 };
 
 /* everything frame-independent, for one (format, W, H) */

@@ -15,7 +15,11 @@ at tolerance 0.
 7. host frames: pinned zero copy, host DMA batches, pageable frames through the staging
    threads, and submit_many_after;
 8. global alpha 0: out of place the copy, in place nothing is touched and nothing launched;
-9. the error codes."""
+9. the error codes;
+10. the same fades under FLUC_TTMLBLEND_CHROMA_AVERAGE on the four 4:2:0 formats, at odd
+   origins, against model_blend(chroma_average=True) at the faded values: per-rectangle values,
+   a fade inside one batch, queued frames, overlay_update of a faded box, and the cache's memory
+   back at its baseline once the cues are cleared."""
 import os
 import subprocess
 import sys
@@ -23,8 +27,8 @@ import sys
 import numpy as np
 import pytest
 
-from helpers import (assert_planes_equal, copy_planes, gpu_blend, oracle_blend, pkg, random_frame,
-                     random_overlay, wl)
+from helpers import (PLANAR_420, assert_planes_equal, copy_planes, gpu_blend, model_blend, oracle_blend, pkg,
+                     random_frame, random_overlay, wl)
 from oracle import oracle
 
 pytestmark = pytest.mark.gpu
@@ -53,22 +57,59 @@ def blend(ctx, stream, fmt, frame, mode="out", dp=False, w=W, h=H):
     return gpu_blend(ctx, fmt, w, h, frame, mode=mode, stream=stream, dest_premul=dp, set_overlay=False)
 
 
-@pytest.mark.parametrize("alpha", ALPHAS)
-@pytest.mark.parametrize("fmt", FORMATS)
-def test_faded_cue_matches_oracle(ctx, fmt, alpha):
+def expected(fmt, frame, rl, dp=False, avg=False, w=W, h=H):
+    """The oracle's blend; under chroma averaging the numpy model of that option (its luma is the
+    oracle's, which is checked too)."""
+    want = oracle_blend(fmt, w, h, copy_planes(frame), rl, dp)
+    if not avg:
+        return want
+    got = model_blend(fmt, w, h, copy_planes(frame), rl, dp, chroma_average=True)
+    assert np.array_equal(got[0], want[0])
+    return got
+
+
+@pytest.fixture
+def averaging(ctx):
+    """The session context with FLUC_TTMLBLEND_CHROMA_AVERAGE for one test."""
+    ctx.set_chroma_mode(True)
+    try:
+        yield ctx
+    finally:
+        ctx.set_chroma_mode(False)
+
+
+def odd_rects(seed, sp=True, ga=1.0, w=W):
+    """rects() at odd origins: 2x2 chroma blocks half inside, half outside every rectangle."""
+    return [dict(r, x=r["x"] + 1, y=r["y"] + 1) for r in rects(seed, sp, ga, w)]
+
+
+def check_faded_cue(ctx, fmt, alpha, avg=False):
     frame = random_frame(fmt, W, H, 7)
     for sp in (True, False):
-        rl = rects(11, sp)
+        rl = (odd_rects if avg else rects)(11, sp)
         ctx.overlay_set_rectangles(900, rl)
         # one frame at 1.0 first, so that the fade re-uses prepared planes instead of preparing them
-        assert_planes_equal(blend(ctx, 900, fmt, frame), oracle_blend(fmt, W, H, copy_planes(frame), rl),
-                            f"{fmt} before the fade")
+        assert_planes_equal(blend(ctx, 900, fmt, frame), expected(fmt, frame, rl, avg=avg), f"{fmt} before the fade")
         ctx.overlay_set_global_alpha(900, alpha)
         for dp in (False, True):
-            want = oracle_blend(fmt, W, H, copy_planes(frame), faded(rl, alpha), dp)
+            want = expected(fmt, frame, faded(rl, alpha), dp, avg)
             for mode in ("out", "inplace"):
                 assert_planes_equal(blend(ctx, 900, fmt, frame, mode, dp), want,
                                     f"{fmt} ga={alpha} sp={sp} dp={dp} {mode}")
+
+
+@pytest.mark.parametrize("alpha", ALPHAS)
+@pytest.mark.parametrize("fmt", FORMATS)
+def test_faded_cue_matches_oracle(ctx, fmt, alpha):
+    check_faded_cue(ctx, fmt, alpha)
+
+
+@pytest.mark.parametrize("alpha", ALPHAS)
+@pytest.mark.parametrize("fmt", PLANAR_420)
+def test_faded_cue_under_chroma_averaging(averaging, fmt, alpha):
+    """The averaged chroma sample weighs its four pixels by asrc = a*ga/255 (BLENDSPEC section 7),
+    so a fade gives what installing the rectangles at the new value gives."""
+    check_faded_cue(averaging, fmt, alpha, avg=True)
 
 
 @pytest.mark.parametrize("fmt", ["NV12", "Y444", "RGB", "BGRA"])
@@ -81,38 +122,48 @@ def test_fade_before_the_first_frame(ctx, fmt):
     assert_planes_equal(blend(ctx, 906, fmt, frame), oracle_blend(fmt, W, H, copy_planes(frame), faded(rl, 0.3)))
 
 
-@pytest.mark.parametrize("fmt", ["NV12", "RGB", "BGRA"])
-def test_per_rectangle_values(ctx, fmt):
+def check_per_rectangle_values(ctx, fmt, avg=False):
     frame = random_frame(fmt, W, H, 9)
-    rl = [dict(pixels=random_overlay(90, 60, 21), x=10, y=10),
-          dict(pixels=random_overlay(90, 60, 22, premultiplied=False), x=50, y=30, premultiplied=False),
-          dict(pixels=random_overlay(90, 60, 23), x=80, y=50)]
+    o = 1 if avg else 0
+    rl = [dict(pixels=random_overlay(90, 60, 21), x=10 + o, y=10 + o),
+          dict(pixels=random_overlay(90, 60, 22, premultiplied=False), x=50 + o, y=30 + o, premultiplied=False),
+          dict(pixels=random_overlay(90, 60, 23), x=80 + o, y=50 + o)]
     ctx.overlay_set_rectangles(910, rl)
     blend(ctx, 910, fmt, frame)
-    for alphas in ([0.3, 0.0, 0.9], [1.0, 0.6, 0.25], [0.75]):
+    for alphas in ([0.3, 0.0, 0.9], [1.0, 0.6, 0.25], [0.75], [0.75, 0.5, 0.75]):
         ctx.overlay_set_global_alpha(910, alphas)
-        want = oracle_blend(fmt, W, H, copy_planes(frame), faded(rl, alphas if len(alphas) > 1 else alphas[0]))
+        want = expected(fmt, frame, faded(rl, alphas if len(alphas) > 1 else alphas[0]), avg=avg)
         for mode in ("out", "inplace"):
             assert_planes_equal(blend(ctx, 910, fmt, frame, mode), want, f"{alphas} {mode}")
 
 
-def test_fade_inside_one_batch(ctx):
-    fmt, w, h, n = "NV12", 1280, 720, 32
-    rl = rects(31, w=w)
-    ctx.overlay_set_rectangles(920, rl)
+@pytest.mark.parametrize("fmt", ["NV12", "RGB", "BGRA"])
+def test_per_rectangle_values(ctx, fmt):
+    check_per_rectangle_values(ctx, fmt)
+
+
+@pytest.mark.parametrize("fmt", PLANAR_420)
+def test_per_rectangle_values_under_chroma_averaging(averaging, fmt):
+    check_per_rectangle_values(averaging, fmt, avg=True)
+
+
+def check_fade_inside_one_batch(ctx, fmt, avg=False, stream=920):
+    w, h, n = 1280, 720, 32
+    rl = (odd_rects if avg else rects)(31, w=w)
+    ctx.overlay_set_rectangles(stream, rl)
     frame = random_frame(fmt, w, h, 10)
     src = ctx.acquire(fmt, w, h)
     dsts = [ctx.acquire(fmt, w, h) for _ in range(n)]
     src.upload(frame)
-    ctx.wait(ctx.submit(920, fmt, w, h, src.c, dsts[0].c))       # prepared at 1.0
+    ctx.wait(ctx.submit(stream, fmt, w, h, src.c, dsts[0].c))    # prepared at 1.0
     alphas = [(n - k) / n for k in range(n)]                      # 1.0 down to 1/32 (0 would drop the bands)
     ctx.set_batch(64, 1_000_000)
     try:
         st0 = ctx.stats()
         tickets = []
         for a, d in zip(alphas, dsts):
-            ctx.overlay_set_global_alpha(920, a)
-            tickets.append(ctx.submit(920, fmt, w, h, src.c, d.c))
+            ctx.overlay_set_global_alpha(stream, a)
+            tickets.append(ctx.submit(stream, fmt, w, h, src.c, d.c))
         ctx.flush()
         for t in tickets:
             ctx.wait(t)
@@ -120,17 +171,30 @@ def test_fade_inside_one_batch(ctx):
     finally:
         ctx.set_batch(32, 200)
     assert st1["launches"] - st0["launches"] == 1
-    assert st1["prepare_launches"] == st0["prepare_launches"]
+    if avg:
+        # the averaged chroma of both rectangles again at each new value (BLENDSPEC section 7)
+        assert st1["prepare_launches"] - st0["prepare_launches"] == 2 * (n - 1)
+    else:
+        assert st1["prepare_launches"] == st0["prepare_launches"]
     for k in (0, 1, 7, 16, 30, 31):
-        want = oracle_blend(fmt, w, h, copy_planes(frame), faded(rl, alphas[k]))
+        want = expected(fmt, frame, faded(rl, alphas[k]), avg=avg, w=w, h=h)
         assert_planes_equal(dsts[k].download(), want, f"frame {k} ga={alphas[k]}")
     for f in [src] + dsts:
         f.release()
 
 
-def test_queued_frames_keep_their_alpha(ctx):
-    fmt = "I420"
-    rl = rects(41)
+def test_fade_inside_one_batch(ctx):
+    check_fade_inside_one_batch(ctx, "NV12")
+
+
+@pytest.mark.parametrize("fmt", ["NV12", "I420"])
+def test_fade_inside_one_batch_under_chroma_averaging(averaging, fmt):
+    # a stream of its own per format: a fade prepares again for every format the stream has used
+    check_fade_inside_one_batch(averaging, fmt, avg=True, stream=921 if fmt == "NV12" else 922)
+
+
+def check_queued_frames(ctx, fmt, avg=False):
+    rl = (odd_rects if avg else rects)(41)
     ctx.overlay_set_rectangles(930, rl)
     frame = random_frame(fmt, W, H, 11)
     src, d1, d2 = ctx.acquire(fmt, W, H), ctx.acquire(fmt, W, H), ctx.acquire(fmt, W, H)
@@ -146,10 +210,19 @@ def test_queued_frames_keep_their_alpha(ctx):
         ctx.wait(t2)
     finally:
         ctx.set_batch(32, 200)
-    assert_planes_equal(d1.download(), oracle_blend(fmt, W, H, copy_planes(frame), faded(rl, 0.3)), "first")
-    assert_planes_equal(d2.download(), oracle_blend(fmt, W, H, copy_planes(frame), faded(rl, 0.8)), "second")
+    assert_planes_equal(d1.download(), expected(fmt, frame, faded(rl, 0.3), avg=avg), "first")
+    assert_planes_equal(d2.download(), expected(fmt, frame, faded(rl, 0.8), avg=avg), "second")
     for f in (src, d1, d2):
         f.release()
+
+
+def test_queued_frames_keep_their_alpha(ctx):
+    check_queued_frames(ctx, "I420")
+
+
+@pytest.mark.parametrize("fmt", ["YV12", "NV21"])
+def test_queued_frames_keep_their_alpha_under_chroma_averaging(averaging, fmt):
+    check_queued_frames(averaging, fmt, avg=True)
 
 
 REGIONS = [wl.Region(16, 8, 160, 30, (0, 0, 0, 255), 0.8),
@@ -165,43 +238,65 @@ def region_image(seeds):
     return img
 
 
-def ttml_want(fmt, frame, img, alpha):
-    return oracle_blend(fmt, W, H, copy_planes(frame), faded(oracle.ttmlrender_rectangles(img), alpha))
+def ttml_want(fmt, frame, img, alpha, avg=False):
+    return expected(fmt, frame, faded(oracle.ttmlrender_rectangles(img), alpha), avg=avg)
 
 
-@pytest.mark.parametrize("fmt", ["NV12", "BGRA"])
-def test_lifecycle(ctx, fmt):
+def check_lifecycle(ctx, fmt, avg=False):
     frame = random_frame(fmt, W, H, 12)
     a, b = region_image([1, 1]), region_image([1, 2])
     ctx.overlay_set(940, a, BOXES)
     blend(ctx, 940, fmt, frame)
     ctx.overlay_set_global_alpha(940, [0.5, 0.5])                 # one value per region box
-    assert_planes_equal(blend(ctx, 940, fmt, frame), ttml_want(fmt, frame, a, 0.5), "faded")
+    assert_planes_equal(blend(ctx, 940, fmt, frame), ttml_want(fmt, frame, a, 0.5, avg), "faded")
     ctx.overlay_update(940, b, [BOXES[1]])                         # a patch keeps the value
-    assert_planes_equal(blend(ctx, 940, fmt, frame), ttml_want(fmt, frame, b, 0.5), "after overlay_update")
+    assert_planes_equal(blend(ctx, 940, fmt, frame), ttml_want(fmt, frame, b, 0.5, avg), "after overlay_update")
+    ctx.overlay_set_global_alpha(940, [0.5, 0.25])                 # the patched box faded on its own
+    assert_planes_equal(blend(ctx, 940, fmt, frame), expected(fmt, frame, regions_faded(b, [0.5, 0.25]), avg=avg),
+                        "patched box faded")
     ctx.overlay_set(940, a, BOXES)                                 # a new cue starts at 1
-    assert_planes_equal(blend(ctx, 940, fmt, frame), ttml_want(fmt, frame, a, 1.0), "after overlay_set")
+    assert_planes_equal(blend(ctx, 940, fmt, frame), ttml_want(fmt, frame, a, 1.0, avg), "after overlay_set")
 
     # installed at 0.4: prepared with it folded in; the first fade prepares once more, later ones never
-    rl = rects(51, ga=0.4)
-    st = 941 if fmt == "NV12" else 942     # a stream of its own: eager prepare adds the formats a stream used
-    ctx.overlay_set_rectangles(st, rl)
-    assert_planes_equal(blend(ctx, st, fmt, frame), oracle_blend(fmt, W, H, copy_planes(frame), rl), "at 0.4")
+    rl = (odd_rects if avg else rects)(51, ga=0.4)
+    st = (941 if fmt == "NV12" else 942) + (10 if avg else 0)   # a stream of its own: eager prepare adds
+    ctx.overlay_set_rectangles(st, rl)                          # the formats a stream used
+    assert_planes_equal(blend(ctx, st, fmt, frame), expected(fmt, frame, rl, avg=avg), "at 0.4")
     p0 = ctx.stats()["prepare_launches"]
     ctx.overlay_set_global_alpha(st, 0.8)
     p1 = ctx.stats()["prepare_launches"]
-    assert_planes_equal(blend(ctx, st, fmt, frame), oracle_blend(fmt, W, H, copy_planes(frame), faded(rl, 0.8)),
-                        "0.4 -> 0.8")
+    assert_planes_equal(blend(ctx, st, fmt, frame), expected(fmt, frame, faded(rl, 0.8), avg=avg), "0.4 -> 0.8")
     ctx.overlay_set_global_alpha(st, 0.6)
     ctx.overlay_set_global_alpha(st, [0.0, 1.0])
-    assert_planes_equal(blend(ctx, st, fmt, frame),
-                        oracle_blend(fmt, W, H, copy_planes(frame), faded(rl, [0.0, 1.0])), "-> 0, 1")
+    assert_planes_equal(blend(ctx, st, fmt, frame), expected(fmt, frame, faded(rl, [0.0, 1.0]), avg=avg), "-> 0, 1")
     p2 = ctx.stats()["prepare_launches"]
-    if fmt == "NV12":
-        assert p1 > p0                  # PLANE8: the alpha bytes had 0.4 in them
-    else:
+    if fmt == "BGRA":
         assert p1 == p0                 # the packed kinds never fold it in
-    assert p2 == p1
+    else:
+        assert p1 > p0                  # PLANE8: the alpha bytes had 0.4 in them
+    if avg:
+        assert p2 > p1                  # averaged chroma holds the value: prepared again per change
+    else:
+        assert p2 == p1
+
+
+def regions_faded(img, alphas):
+    """The region image as one rectangle per region box, each at its own global alpha (the boxes
+    are disjoint and the image is transparent outside them)."""
+    out = []
+    for (x, y, w, h), a in zip(BOXES, alphas):
+        out.append(dict(pixels=np.ascontiguousarray(img[y:y + h, x:x + w]), x=x, y=y, global_alpha=a))
+    return out
+
+
+@pytest.mark.parametrize("fmt", ["NV12", "BGRA"])
+def test_lifecycle(ctx, fmt):
+    check_lifecycle(ctx, fmt)
+
+
+@pytest.mark.parametrize("fmt", ["NV12", "I420"])
+def test_lifecycle_under_chroma_averaging(averaging, fmt):
+    check_lifecycle(averaging, fmt, avg=True)
 
 
 def opaque_cue():
@@ -245,8 +340,11 @@ def test_opaque_box_faded(ctx):
     blend(ctx, 950, "NV12", random_frame("NV12", W, H, 1), "inplace")
     blend(ctx, 950, "NV12", random_frame("NV12", W, H, 1), "out")
     st1 = ctx.stats()
-    assert st1["lazy_launches"] > st0["lazy_launches"]               # the cue takes both shortcuts at 1.0
-    assert st1["opaque_skip_launches"] > st0["opaque_skip_launches"]
+    on = lambda knob: os.environ.get(knob, "1") != "0" and os.environ.get("FLUC_TTMLBLEND_GROUPS", "1") != "0"
+    if on("FLUC_TTMLBLEND_LAZY"):                                     # not forced off (tools/knob_matrix.sh)
+        assert st1["lazy_launches"] > st0["lazy_launches"]           # the cue takes both shortcuts at 1.0
+    if on("FLUC_TTMLBLEND_OPAQUE_SKIP"):
+        assert st1["opaque_skip_launches"] > st0["opaque_skip_launches"]
     check_opaque_cue(ctx, 951)
 
 
@@ -330,6 +428,41 @@ def test_zero_alpha(ctx, fmt):
     assert ctx.stats()["launches"] == before           # no band left: nothing to launch in place
     assert_planes_equal(src.download(), frame, "in place")
     src.release()
+
+
+def test_fades_under_chroma_averaging_do_not_leak():
+    """Every fade under chroma averaging prepares new chroma planes: the memory the overlay cache
+    holds is back at its baseline once the cue is cleared and the work has drained."""
+    import time
+    c = pkg.TtmlBlend(0)
+    try:
+        c.set_chroma_mode(True)
+        fmt = "NV12"
+        frame = random_frame(fmt, W, H, 15)
+        src, dst = c.acquire(fmt, W, H), c.acquire(fmt, W, H)
+        src.upload(frame)
+        c.sync()
+        base = c.stats()["cache_bytes"]
+        rl = odd_rects(101)
+        c.overlay_set_rectangles(990, rl)
+        for k in range(24):
+            alphas = [(k % 8 + 1) / 8, ((k + 3) % 8) / 8]
+            c.overlay_set_global_alpha(990, alphas)
+            c.submit(990, fmt, W, H, src.c, dst.c)
+        c.sync()
+        assert_planes_equal(dst.download(), expected(fmt, frame, faded(rl, alphas), avg=True), "last fade")
+        assert c.stats()["cache_bytes"] > base
+        c.overlay_clear(990)
+        c.sync()
+        c.sync()        # deferred frees run on the reaper stream after the fences
+        deadline = time.time() + 5
+        while c.stats()["cache_bytes"] > base and time.time() < deadline:
+            time.sleep(0.01)
+        assert c.stats()["cache_bytes"] == base
+        src.release()
+        dst.release()
+    finally:
+        c.close()
 
 
 def test_errors(ctx):

@@ -2,7 +2,8 @@
 # Runs the parity tests with every alternative code path forced through its environment knob:
 # table kernel only, no multi-layout launches, in-place launches always / never lazy, no
 # auto-crop, register-staged instead of TMA-staged overlay, interleaved chunk order, and the
-# host-frame knobs. Every line must end in "passed".
+# host-frame knobs; then the global-alpha and operator-domain files under each knob. Every line
+# must end in "passed".
 #   gpurun -- bash tools/knob_matrix.sh
 K="rectangles_match_oracle or golden or fuzz or alpha_sweep or scaled_rectangles or regions or unaligned or chain or ping_pong or dependency or two_overlays or update or sparse_cues or host_path or host_dma"
 for v in FLUC_TTMLBLEND_GROUPS=0 FLUC_TTMLBLEND_MULTI=0 FLUC_TTMLBLEND_LAZY=1 FLUC_TTMLBLEND_LAZY=0 \
@@ -15,4 +16,6 @@ for v in FLUC_TTMLBLEND_GROUPS=0 FLUC_TTMLBLEND_MULTI=0 FLUC_TTMLBLEND_LAZY=1 FL
   env $v timeout 300 python -m pytest tests/test_gpu_parity.py tests/test_gpu_scale.py tests/test_gpu_regions.py \
       tests/test_gpu_hazards.py tests/test_gpu_update.py tests/test_gpu_configs.py \
       -q -x -k "$K" 2>&1 | tail -1
+  # every global-alpha (JF_GA) instantiation and the operator domains under the same knob
+  env $v timeout 600 python -m pytest tests/test_gpu_global_alpha.py tests/test_gpu_domain.py -q -x 2>&1 | tail -1
 done
