@@ -775,6 +775,11 @@ overlay_install (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, cons
     const int rw = r.render_width ? r.render_width : r.width, rh = r.render_height ? r.render_height : r.height;
     if ((rw != r.width || rh != r.height) && (r.width < 2 || r.height < 2))
       return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;   /* upstream reads outside the image here */
+    /* the scaler's 16.16 positions ((side - 1) << 16, x * x_inc, the row plan's accumulator)
+     * are 32-bit: past 32768 on a side they overflow (upstream's gint arithmetic is undefined
+     * there too) and the kernel would read outside the source */
+    if ((rw != r.width || rh != r.height) && (r.width > 32768 || r.height > 32768 || rw > 32768 || rh > 32768))
+      return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
   }
   std::shared_ptr<Overlay> ov (new Overlay ());
   ov->ctx = c;

@@ -118,7 +118,10 @@ typedef struct {
  * image is rendered at its pixel size (render_width = render_height = 0); a
  * rectangle with another render size is first scaled on the GPU exactly as
  * gst_video_overlay_composition_blend does with gst_video_blend_scale_linear_RGBA
- * (once per cue, cached like everything else); its pixel size must then be >= 2x2. */
+ * (once per cue, cached like everything else); its pixel size must then be >= 2x2,
+ * and neither its pixel size nor its render size may exceed 32768 on either side
+ * (the scaler's 16.16 positions are 32-bit): FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT
+ * otherwise. render_width / render_height above 32768 are refused in any case. */
 typedef struct {
   const uint8_t *pixels;   /* host memory -- or device memory of the context's GPU: a cue that is
                             * already in HBM is copied there -- read before the call returns */

@@ -368,6 +368,23 @@ def test_scale_row_plan_is_the_simulated_line_cache(hooks, sh, dh):
         assert naive != got          # the quirk is really exercised
 
 
+@pytest.mark.parametrize("dh", [3, 1000, 32767])
+def test_scale_row_plan_at_the_largest_source_height(hooks, dh):
+    """32768 source rows is the most a scaled rectangle may have: (32768 - 1) << 16 and the
+    plan's accumulator still fit in 32 bits, and the runtime's plan equals the model's. One
+    row more overflows them, so overlay_install refuses such a rectangle (docs/BLENDSPEC.md
+    section 10; tests/test_gpu_cue_kernels.py checks the refusal)."""
+    from helpers import model_scale_rows
+    sh = 32768
+    assert ((sh - 1) << 16) < 2 ** 31 and (dh - 1) * (((sh - 1) << 16) // max(dh - 1, 1)) < 2 ** 31
+    out = (C.c_int32 * (3 * dh))()
+    assert hooks.tb_hook_scale_row_plan(sh, dh, out) == dh
+    got = np.frombuffer(out, dtype=np.int32).reshape(dh, 3)
+    want = np.array(model_scale_rows(sh, dh), dtype=np.int32)
+    assert np.array_equal(got, want)
+    assert got[-1, 0] >= sh - 2 and got[:, :2].max() < sh       # reaches the bottom, stays inside
+
+
 # ---------------------------------------------------------------------------------------------
 
 def pack(hooks, W, H, ov, rects, strides):
