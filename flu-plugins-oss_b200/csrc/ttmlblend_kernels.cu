@@ -22,6 +22,7 @@
 
 #include <cstdlib>
 #include <cstring>
+#include <type_traits>
 #include <utility>
 
 namespace tb {
@@ -369,6 +370,37 @@ blend16_packed (uint4 f, const uint4 &o, uint32_t ga, bool sp, bool dp)
   return f;
 }
 
+/* The scalars of a rectangle that its blend operator takes. PLANE8 has one operator, so its ga
+ * and src_premul are constants; a_ga is read by the JF_GA variants only. */
+struct RectOp { uint32_t ga, a_ga; bool sp; };
+
+template <int KIND, bool GA>
+__device__ __forceinline__ RectOp
+rect_op (const RectRef *r)
+{
+  RectOp op;
+  op.ga = KIND == PK_PLANE8 ? 255u : (uint32_t) __ldg (&r->ga);
+  op.sp = KIND == PK_PLANE8 ? false : __ldg (&r->src_premul) != 0;
+  op.a_ga = GA ? (uint32_t) __ldg (&r->a_ga) : 255u;
+  return op;
+}
+
+/* One 16-byte vector of frame f blended with one rectangle: oa = its alpha bytes (PLANE8 kinds)
+ * or pixel words (packed), oc = its colour bytes (PLANE8 kinds; not read by the packed kinds),
+ * dp = destination premultiplied. */
+template <int KIND, bool GA>
+__device__ __forceinline__ uint4
+blend16 (const uint4 &f, uint4 oa, const uint4 &oc, const RectOp &op, bool dp)
+{
+  if (GA)
+    oa = scale16_alpha (oa, op.a_ga);
+  if (KIND == PK_PLANE8)
+    return blend16_plane8 (f, oa, oc);
+  if (KIND == PK_PLANE8_RGB)
+    return blend16_rgb24 (f, oa, oc, op.ga, op.sp);
+  return blend16_packed<KIND == PK_PACKED_A0 ? 0 : 3> (f, oa, op.ga, op.sp, dp);
+}
+
 /* ---------------------------------------------------------------------- */
 /* the per-frame blend kernel                                             */
 
@@ -390,20 +422,9 @@ blend_with_rect (uint4 f, const RectRef *r, const RectGeom &g, int v, int y,
 {
   const int32_t pitch = __ldg (&r->pitch);
   const size_t off = (size_t) (y - g.y0) * pitch + (size_t) (v - g.v0) * 16;
-  uint4 oa = ld_overlay16 (ldg_ptr (&r->a) + off);
-  if (GA)
-    oa = scale16_alpha (oa, (uint32_t) __ldg (&r->a_ga));
-  if (KIND == PK_PLANE8) {
-    const uint4 oc = ld_overlay16 (ldg_ptr (&r->c) + off);
-    return blend16_plane8 (f, oa, oc);
-  } else if (KIND == PK_PLANE8_RGB) {
-    const uint4 oc = ld_overlay16 (ldg_ptr (&r->c) + off);
-    return blend16_rgb24 (f, oa, oc, (uint32_t) __ldg (&r->ga), __ldg (&r->src_premul) != 0);
-  } else {
-    const uint32_t ga = (uint32_t) __ldg (&r->ga);
-    const bool sp = __ldg (&r->src_premul) != 0;
-    return blend16_packed<KIND == PK_PACKED_A0 ? 0 : 3> (f, oa, ga, sp, dst_premul);
-  }
+  const uint4 oa = ld_overlay16 (ldg_ptr (&r->a) + off);
+  const uint4 oc = kind_is_planes (KIND) ? ld_overlay16 (ldg_ptr (&r->c) + off) : oa;
+  return blend16<KIND, GA> (f, oa, oc, rect_op<KIND, GA> (r), dst_premul);
 }
 
 /* Job fields a CTA keeps in registers while it works through the job. */
@@ -560,7 +581,7 @@ process_chunk (const JobRegs &J, uint32_t local_chunk)
           "bra OV_WAIT;\n"
           "OV_DONE:\n"
           "}" :: "r" (bar) : "memory");
-      const uint32_t a_ga = GA ? (uint32_t) __ldg (&r->a_ga) : 255u;
+      const RectOp op = rect_op<KIND, GA> (r);
       if (LAZY) {
         /* overlay first. LAZY 1 (in place): only vectors with some alpha are written back, and
          * of those only the ones that are not opaque all over are fetched (all fetches in flight
@@ -568,14 +589,13 @@ process_chunk (const JobRegs &J, uint32_t local_chunk)
          * but the ones under an opaque vector are not fetched. Under an opaque vector the
          * result is the overlay colour whatever the frame holds; a stand-in with an opaque
          * alpha byte keeps the packed kinds on their fast path. */
-        const bool ga_full = kind_is_planes (KIND) && KIND != PK_PLANE8_RGB ? true :
-            __ldg (&r->ga) == 255;
+        const bool ga_full = op.ga == 255u;
         const uint32_t fill = KIND == PK_PACKED_A0 ? 0x000000ffu : KIND == PK_PACKED_A3 ? 0xff000000u : 0u;
 #pragma unroll
         for (int k = 0; k < kUnroll; k++) {
           uint4 oa = *reinterpret_cast<const uint4 *> (ov_smem + (threadIdx.x + k * kThreads) * 16u);
           if (GA)
-            oa = scale16_alpha (oa, a_ga);      /* effective alpha: opaque only where a_ga is 255 too */
+            oa = scale16_alpha (oa, op.a_ga);   /* effective alpha: opaque only where a_ga is 255 too */
           if (LAZY == 1)
             act[k] = act[k] && any_alpha<KIND> (oa);
           f[k] = make_uint4 (fill, fill, fill, fill);
@@ -583,27 +603,16 @@ process_chunk (const JobRegs &J, uint32_t local_chunk)
             f[k] = ld_frame16 (src + (size_t) yy[k] * src_pitch + (size_t) vv[k] * 16);
         }
       }
-      const uint32_t ga = KIND == PK_PLANE8 ? 255u : (uint32_t) __ldg (&r->ga);
-      const bool sp = KIND == PK_PLANE8 ? false : __ldg (&r->src_premul) != 0;
       const bool dp = (J.flags & JF_DST_PREMUL) != 0;
 #pragma unroll
       for (int k = 0; k < kUnroll; k++)
         if (act[k]) {
           const uint32_t so = (threadIdx.x + k * kThreads) * 16u;
-          uint4 oa = *reinterpret_cast<const uint4 *> (ov_smem + so);
-          if (GA)
-            oa = scale16_alpha (oa, a_ga);
-          uint4 out;
-          if (KIND == PK_PLANE8) {
-            const uint4 oc = *reinterpret_cast<const uint4 *> (ov_smem + kItemsPerChunk * 16 + so);
-            out = blend16_plane8 (f[k], oa, oc);
-          } else if (KIND == PK_PLANE8_RGB) {
-            const uint4 oc = *reinterpret_cast<const uint4 *> (ov_smem + kItemsPerChunk * 16 + so);
-            out = blend16_rgb24 (f[k], oa, oc, ga, sp);
-          } else {
-            out = blend16_packed<KIND == PK_PACKED_A0 ? 0 : 3> (f[k], oa, ga, sp, dp);
-          }
-          st_frame16 (dst + (size_t) yy[k] * dst_pitch + (size_t) vv[k] * 16, out);
+          const uint4 oa = *reinterpret_cast<const uint4 *> (ov_smem + so);
+          const uint4 oc = kind_is_planes (KIND) ? *reinterpret_cast<const uint4 *> (ov_smem + kItemsPerChunk * 16 + so)
+              : oa;
+          st_frame16 (dst + (size_t) yy[k] * dst_pitch + (size_t) vv[k] * 16,
+              blend16<KIND, GA> (f[k], oa, oc, op, dp));
         }
       return;
     }
@@ -619,40 +628,28 @@ process_chunk (const JobRegs &J, uint32_t local_chunk)
       for (int k = 0; k < kUnroll; k++)
         if (act[k])
           f[k] = ld_frame16 (src + (size_t) yy[k] * src_pitch + (size_t) vv[k] * 16);
-      if (kind_is_planes (KIND)) {
-        const uint8_t *pc = ldg_ptr (&r->c);
-        const uint32_t ga1 = KIND == PK_PLANE8 ? 255u : (uint32_t) __ldg (&r->ga);
-        const bool sp1 = KIND == PK_PLANE8 ? false : __ldg (&r->src_premul) != 0;
-        const uint32_t a_ga = GA ? (uint32_t) __ldg (&r->a_ga) : 255u;
+      /* the rectangle's scalars after the frame loads, out of those loads' live range; the JF_GA
+       * alpha is scaled as it arrives, which spills nothing (scaled at the blend, it does) */
+      const uint8_t *pc = kind_is_planes (KIND) ? ldg_ptr (&r->c) : pa;
+      const RectOp op = rect_op<KIND, GA> (r);
+      const bool dp = (J.flags & JF_DST_PREMUL) != 0;
 #pragma unroll
-        for (int k = 0; k < kUnroll; k++)
-          if (act[k]) {
-            const size_t off = (size_t) (yy[k] - g.y0) * pitch + (size_t) (vv[k] - g.v0) * 16;
-            oa[k] = ld_overlay16 (pa + off);
-            oc[k] = ld_overlay16 (pc + off);
-            if (GA)
-              oa[k] = scale16_alpha (oa[k], a_ga);
-          }
+      for (int k = 0; k < kUnroll; k++)
+        if (act[k]) {
+          const size_t off = (size_t) (yy[k] - g.y0) * pitch + (size_t) (vv[k] - g.v0) * 16;
+          oa[k] = ld_overlay16 (pa + off);
+          oc[k] = kind_is_planes (KIND) ? ld_overlay16 (pc + off) : oa[k];
+          if (GA)
+            oa[k] = scale16_alpha (oa[k], op.a_ga);
+        }
 #pragma unroll
-        for (int k = 0; k < kUnroll; k++)
-          if (act[k])
-            st_frame16 (dst + (size_t) yy[k] * dst_pitch + (size_t) vv[k] * 16,
-                KIND == PK_PLANE8 ? blend16_plane8 (f[k], oa[k], oc[k]) :
-                blend16_rgb24 (f[k], oa[k], oc[k], ga1, sp1));
-      } else {
-        const uint32_t ga = (uint32_t) __ldg (&r->ga);
-        const bool sp = __ldg (&r->src_premul) != 0;
-        const bool dp = (J.flags & JF_DST_PREMUL) != 0;
-#pragma unroll
-        for (int k = 0; k < kUnroll; k++)
-          if (act[k])
-            oa[k] = ld_overlay16 (pa + (size_t) (yy[k] - g.y0) * pitch + (size_t) (vv[k] - g.v0) * 16);
-#pragma unroll
-        for (int k = 0; k < kUnroll; k++)
-          if (act[k])
-            st_frame16 (dst + (size_t) yy[k] * dst_pitch + (size_t) vv[k] * 16,
-                blend16_packed<KIND == PK_PACKED_A0 ? 0 : 3> (f[k], oa[k], ga, sp, dp));
-      }
+      for (int k = 0; k < kUnroll; k++)
+        if (act[k])
+          /* the packed kinds call their operator directly: through blend16, ptxas makes this
+           * table kernel 72 instructions longer and 0.15 % slower on a B200 (config 4) */
+          st_frame16 (dst + (size_t) yy[k] * dst_pitch + (size_t) vv[k] * 16,
+              kind_is_planes (KIND) ? blend16<KIND, false> (f[k], oa[k], oc[k], op, dp)
+              : blend16_packed<KIND == PK_PACKED_A0 ? 0 : 3> (f[k], oa[k], op.ga, op.sp, dp));
       return;
     }
   }
@@ -746,6 +743,14 @@ process_chunk (const JobRegs &J, uint32_t local_chunk)
 #define TTMLBLEND_MIN_CTAS 5
 #endif
 
+/* the chunk of this CTA; lanes_magic = ceil (2^32 / lanes) (chunk_order) */
+__device__ __forceinline__ uint32_t
+cta_chunk (uint32_t lanes, uint32_t lanes_magic, uint32_t per_lane)
+{
+  const uint32_t q = lanes == 1u ? blockIdx.x : __umulhi (blockIdx.x, lanes_magic);
+  return (blockIdx.x - q * lanes) * per_lane + q;
+}
+
 template <int KIND, bool FAST, bool GA = false>
 __global__ void __launch_bounds__ (kThreads, FAST ? 4 : 2)
 ttmlblend_blend_kernel (const PlaneJob *__restrict__ jobs,
@@ -753,9 +758,7 @@ ttmlblend_blend_kernel (const PlaneJob *__restrict__ jobs,
     uint32_t total_chunks, uint32_t lanes, uint32_t per_lane, uint32_t lanes_magic, int sync)
 {
   pdl_begin (sync);
-  const uint32_t q = lanes == 1u ? blockIdx.x : __umulhi (blockIdx.x, lanes_magic);
-  const uint32_t r = blockIdx.x - q * lanes;
-  const uint32_t chunk = r * per_lane + q;
+  const uint32_t chunk = cta_chunk (lanes, lanes_magic, per_lane);
   if (chunk >= total_chunks) {
     pdl_end (sync);
     return;
@@ -774,6 +777,32 @@ ttmlblend_blend_kernel (const PlaneJob *__restrict__ jobs,
   pdl_end (sync);
 }
 
+/* The job of a band of one frame of a parameter-block launch (group and multi-layout kernels);
+ * `rects` is the frame's rectangle table of the band's plane. */
+__device__ __forceinline__ JobRegs
+band_job (const BandDesc &B, const FramePtrs &F, const RectRef *rects, const int32_t *src_pitch,
+    const int32_t *dst_pitch, int flags)
+{
+  const int pl = B.plane;
+  JobRegs J;
+  J.src = F.src[pl];
+  J.dst = F.dst[pl];
+  J.rects = rects;
+  J.rect_mask = ((unsigned long long) B.rect_mask_hi << 32) | B.rect_mask_lo;
+  J.src_pitch = src_pitch[pl];
+  J.dst_pitch = dst_pitch[pl];
+  J.win_v0 = B.win_v0;
+  J.win_y0 = B.win_y0;
+  J.win_nv = (uint32_t) B.win_nv;
+  J.total_items = (uint32_t) B.win_nv * (uint32_t) B.win_rows;
+  J.magic = B.div_magic;
+  J.cls = B.cls;
+  J.one_rect = B.one_rect;
+  J.flags = flags;
+  J.row_bytes = 0;              /* FAST: never read */
+  return J;
+}
+
 /* The common case -- a batch of frames that share format, size, strides and
  * cue layout (consecutive frames of a stream, or many streams with the same
  * region boxes) -- needs no table in global memory at all: the band list is
@@ -789,9 +818,7 @@ ttmlblend_group_kernel (const __grid_constant__ GroupParamsT<NF, NB> P)
 {
   const GroupHeader &Hd = P.h;
   pdl_begin (Hd.flags);
-  const uint32_t q = Hd.lanes == 1u ? blockIdx.x : __umulhi (blockIdx.x, Hd.lanes_magic);
-  const uint32_t r = blockIdx.x - q * Hd.lanes;
-  const uint32_t chunk = r * Hd.per_lane + q;
+  const uint32_t chunk = cta_chunk (Hd.lanes, Hd.lanes_magic, Hd.per_lane);
   if (chunk >= Hd.total_chunks) {
     pdl_end (Hd.flags);
     return;
@@ -804,24 +831,7 @@ ttmlblend_group_kernel (const __grid_constant__ GroupParamsT<NF, NB> P)
     b += cif >= P.bands[i].chunk_begin ? 1u : 0u;
   const BandDesc &B = P.bands[b];
   const FramePtrs &F = P.frames[frame];
-  const int pl = B.plane;
-
-  JobRegs J;
-  J.src = F.src[pl];
-  J.dst = F.dst[pl];
-  J.rects = F.rects + Hd.rect_off[pl];
-  J.rect_mask = ((unsigned long long) B.rect_mask_hi << 32) | B.rect_mask_lo;
-  J.src_pitch = Hd.src_pitch[pl];
-  J.dst_pitch = Hd.dst_pitch[pl];
-  J.win_v0 = B.win_v0;
-  J.win_y0 = B.win_y0;
-  J.win_nv = (uint32_t) B.win_nv;
-  J.total_items = (uint32_t) B.win_nv * (uint32_t) B.win_rows;
-  J.magic = B.div_magic;
-  J.cls = B.cls;
-  J.one_rect = B.one_rect;
-  J.flags = Hd.flags;
-  J.row_bytes = 0;              /* FAST: never read */
+  const JobRegs J = band_job (B, F, F.rects + Hd.rect_off[B.plane], Hd.src_pitch, Hd.dst_pitch, Hd.flags);
   process_chunk<KIND, true, true, LAZY, GA> (J, cif - B.chunk_begin);
   pdl_end (Hd.flags);
 }
@@ -836,9 +846,7 @@ __global__ void __launch_bounds__ (kThreads, LAZY == 1 ? 4 : TTMLBLEND_MIN_CTAS)
 ttmlblend_multi_kernel (const __grid_constant__ MultiParams P)
 {
   pdl_begin (P.flags);
-  const uint32_t q = P.lanes == 1u ? blockIdx.x : __umulhi (blockIdx.x, P.lanes_magic);
-  const uint32_t r = blockIdx.x - q * P.lanes;
-  const uint32_t chunk = r * P.per_lane + q;
+  const uint32_t chunk = cta_chunk (P.lanes, P.lanes_magic, P.per_lane);
   if (chunk >= P.total_chunks) {
     pdl_end (P.flags);
     return;
@@ -857,35 +865,21 @@ ttmlblend_multi_kernel (const __grid_constant__ MultiParams P)
     b += cif >= P.bands[b0 + i].chunk_begin ? 1u : 0u;
   const BandDesc &B = P.bands[b];
   const FramePtrs &F = P.frames[frame];
-  const int pl = B.plane;
-
-  JobRegs J;
-  J.src = F.src[pl];
-  J.dst = F.dst[pl];
-  J.rects = F.rects + ((F.pad_ >> (16 * pl)) & 0xffffu);
-  J.rect_mask = ((unsigned long long) B.rect_mask_hi << 32) | B.rect_mask_lo;
-  J.src_pitch = P.src_pitch[pl];
-  J.dst_pitch = P.dst_pitch[pl];
-  J.win_v0 = B.win_v0;
-  J.win_y0 = B.win_y0;
-  J.win_nv = (uint32_t) B.win_nv;
-  J.total_items = (uint32_t) B.win_nv * (uint32_t) B.win_rows;
-  J.magic = B.div_magic;
-  J.cls = B.cls;
-  J.one_rect = B.one_rect;
-  J.flags = P.flags;
-  J.row_bytes = 0;              /* FAST: never read */
+  const JobRegs J = band_job (B, F, F.rects + ((F.pad_ >> (16 * B.plane)) & 0xffffu), P.src_pitch, P.dst_pitch,
+      P.flags);
   process_chunk<KIND, true, true, LAZY, GA> (J, cif - B.chunk_begin);
   pdl_end (P.flags);
 }
 
-/* Number of interleaved streams the chunk list is walked in. Measured on the
- * 4K configs: the packed kinds (more ALU work per blended vector) gain 3 %
- * with 61 lanes, PLANE8 loses 2 % against list order, so the default follows
- * the kind; FLUC_TTMLBLEND_LANES overrides both (1 = list order). A prime
- * keeps lane starts from lining up with the frame structure of a batch. */
-static uint32_t
-interleave_lanes (int kind)
+/* The interleaved chunk order of a launch (cta_chunk). Number of lanes: measured on the 4K
+ * configs, the packed kinds (more ALU work per blended vector) gain 3 % with 61 lanes, PLANE8
+ * loses 2 % against list order, so the default follows the kind; FLUC_TTMLBLEND_LANES overrides
+ * both (1 = list order). A prime keeps lane starts from lining up with the frame structure of a
+ * batch. */
+struct ChunkOrder { uint32_t lanes, per_lane, magic, grid; };
+
+static cudaError_t
+chunk_order (int kind, uint32_t total_chunks, ChunkOrder &o)
 {
   static int env = -1;
   if (env < 0) {
@@ -894,31 +888,54 @@ interleave_lanes (int kind)
     if (env < 0) env = 0;
     if (env > 4096) env = 4096;
   }
-  if (env)
-    return (uint32_t) env;
-  return kind_is_planes (kind) ? 1u : 61u;
+  o.lanes = env ? (uint32_t) env : kind_is_planes (kind) ? 1u : 61u;
+  if (total_chunks < o.lanes * 8u)
+    o.lanes = 1;
+  o.per_lane = (total_chunks + o.lanes - 1) / o.lanes;
+  o.grid = o.lanes * o.per_lane;
+  /* umulhi (i, ceil (2^32 / lanes)) == i / lanes while i * lanes < 2^32 */
+  if ((unsigned long long) o.grid * o.lanes >= (1ull << 32))
+    return cudaErrorInvalidValue;
+  o.magic = o.lanes == 1 ? 0u : (uint32_t) (((1ull << 32) + o.lanes - 1) / o.lanes);
+  return cudaSuccess;
 }
 
-template <int KIND, bool GA = false>
+template <int V>
+using IntC = std::integral_constant<int, V>;
+
+/* Picks the kernel variant of a launch: calls fn (KIND, LAZY, GA), each a std::integral_constant,
+ * for its PlaneKind and its JobFlags. LAZY 1: in place (dst == src, host frames over PCIe) under
+ * a sparse cue, the overlay is read first and the vectors it would not change are skipped;
+ * LAZY 2: out of place, no frame read under opaque vectors. The JF_GA variants exist for the
+ * PLANE8 kinds only (the packed kinds apply RectRef::ga in every variant). */
+template <typename Fn>
 static cudaError_t
-launch_blend_kind (const PlaneJob *d_jobs, const uint32_t *d_chunk_begin, const uint32_t *d_coarse, int n_jobs,
-    uint32_t total_chunks, bool fast, int sync, cudaStream_t stream)
+with_variant (int kind, int flags, Fn &&fn)
 {
-  uint32_t lanes = interleave_lanes (KIND);
-  if (total_chunks < lanes * 8u)
-    lanes = 1;
-  const uint32_t per_lane = (total_chunks + lanes - 1) / lanes;
-  const uint32_t grid = lanes * per_lane;
-  /* umulhi (i, ceil (2^32 / lanes)) == i / lanes while i * lanes < 2^32 */
-  if ((unsigned long long) grid * lanes >= (1ull << 32))
-    return cudaErrorInvalidValue;
-  const uint32_t magic = lanes == 1 ? 0u : (uint32_t) (((1ull << 32) + lanes - 1) / lanes);
-  const bool pdl = (sync & JF_PDL) != 0;
-  if (fast)
-    return launch_ex (ttmlblend_blend_kernel<KIND, true, GA>, grid, 0, stream, pdl, d_jobs, d_chunk_begin, d_coarse,
-        n_jobs, total_chunks, lanes, per_lane, magic, sync);
-  return launch_ex (ttmlblend_blend_kernel<KIND, false, GA>, grid, 0, stream, pdl, d_jobs, d_chunk_begin, d_coarse,
-      n_jobs, total_chunks, lanes, per_lane, magic, sync);
+  const auto by_look = [&] (auto K) {
+    const auto by_ga = [&] (auto L) {
+      if constexpr (kind_is_planes (K)) {
+        if (flags & JF_GA)
+          return fn (K, L, std::true_type ());
+      }
+      return fn (K, L, std::false_type ());
+    };
+    return (flags & JF_LAZY) ? by_ga (IntC<1> ()) : (flags & JF_OPAQUE) ? by_ga (IntC<2> ()) : by_ga (IntC<0> ());
+  };
+  switch (kind) {
+    case PK_PLANE8: return by_look (IntC<PK_PLANE8> ());
+    case PK_PLANE8_RGB: return by_look (IntC<PK_PLANE8_RGB> ());
+    case PK_PACKED_A0: return by_look (IntC<PK_PACKED_A0> ());
+    case PK_PACKED_A3: return by_look (IntC<PK_PACKED_A3> ());
+    default: return cudaErrorInvalidValue;
+  }
+}
+
+/* shared memory for the TMA-staged overlay slice of a JC_ONE_BULK chunk */
+static size_t
+bulk_smem (int kind)
+{
+  return (kind_is_planes (kind) ? 2 : 1) * kItemsPerChunk * 16;
 }
 
 /* One variant of the group kernel: copies what the launch needs into a parameter block of the
@@ -938,29 +955,6 @@ launch_group_variant (const GroupParams &P, uint32_t grid, size_t smem, cudaStre
   return launch_ex (ttmlblend_group_kernel<KIND, LAZY, NF, NB, GA>, grid, smem, stream, pdl, S);
 }
 
-template <int KIND, int LAZY, bool GA = false>
-static cudaError_t
-launch_group_sized (const GroupParams &P, uint32_t grid, size_t smem, cudaStream_t stream)
-{
-  static const bool compact = !getenv ("FLUC_TTMLBLEND_COMPACT_PARAMS") || atoi (getenv ("FLUC_TTMLBLEND_COMPACT_PARAMS")) != 0;
-  if (compact && P.h.n_frames <= 4u && P.h.n_bands <= 16u)
-    return launch_group_variant<KIND, LAZY, 4, 16, GA> (P, grid, smem, stream);
-  if (compact && P.h.n_frames <= 32u)
-    return launch_group_variant<KIND, LAZY, 32, kMaxGroupBands, GA> (P, grid, smem, stream);
-  return launch_group_variant<KIND, LAZY, kMaxPlainGroupFrames, kMaxGroupBands, GA> (P, grid, smem, stream);
-}
-
-/* The JF_GA variants exist for the PLANE8 kinds only (the packed kinds apply RectRef::ga in every
- * variant). */
-template <int KIND, int LAZY>
-static cudaError_t
-launch_group_ga (const GroupParams &P, uint32_t grid, size_t smem, cudaStream_t stream)
-{
-  if (kind_is_planes (KIND) && (P.h.flags & JF_GA))
-    return launch_group_sized<KIND, LAZY, kind_is_planes (KIND)> (P, grid, smem, stream);
-  return launch_group_sized<KIND, LAZY> (P, grid, smem, stream);
-}
-
 cudaError_t
 launch_group (GroupParams &P, int kind, int sync, cudaStream_t stream)
 {
@@ -969,33 +963,20 @@ launch_group (GroupParams &P, int kind, int sync, cudaStream_t stream)
   Hd.total_chunks = Hd.n_frames * Hd.chunks_per_frame;
   if (Hd.total_chunks == 0)
     return cudaSuccess;
-  uint32_t lanes = interleave_lanes (kind);
-  if (Hd.total_chunks < lanes * 8u)
-    lanes = 1;
-  Hd.lanes = lanes;
-  Hd.per_lane = (Hd.total_chunks + lanes - 1) / lanes;
-  const uint32_t grid = lanes * Hd.per_lane;
-  if ((unsigned long long) grid * lanes >= (1ull << 32))
+  ChunkOrder o;
+  if (chunk_order (kind, Hd.total_chunks, o) != cudaSuccess)
     return cudaErrorInvalidValue;
-  Hd.lanes_magic = lanes == 1 ? 0u : (uint32_t) (((1ull << 32) + lanes - 1) / lanes);
-  /* shared memory for the TMA-staged overlay slice of a JC_ONE_BULK chunk */
-  const size_t smem_plane8 = 2 * kItemsPerChunk * 16, smem_packed = kItemsPerChunk * 16;
-  /* in place (dst == src, host frames over PCIe) under a sparse cue: the variant that reads
-   * the overlay first and skips the vectors it would not change */
-  const int look = (Hd.flags & JF_LAZY) ? 1 : (Hd.flags & JF_OPAQUE) ? 2 : 0;
-#define GROUP_CASE(K, SM) \
-    case K: \
-      return look == 1 ? launch_group_ga<K, 1> (P, grid, SM, stream) : \
-          look == 2 ? launch_group_ga<K, 2> (P, grid, SM, stream) : launch_group_ga<K, 0> (P, grid, SM, stream);
-  switch (kind) {
-    GROUP_CASE (PK_PLANE8, smem_plane8)
-    GROUP_CASE (PK_PLANE8_RGB, smem_plane8)
-    GROUP_CASE (PK_PACKED_A0, smem_packed)
-    GROUP_CASE (PK_PACKED_A3, smem_packed)
-    default:
-      return cudaErrorInvalidValue;
-  }
-#undef GROUP_CASE
+  Hd.lanes = o.lanes;
+  Hd.per_lane = o.per_lane;
+  Hd.lanes_magic = o.magic;
+  static const bool compact = !getenv ("FLUC_TTMLBLEND_COMPACT_PARAMS") || atoi (getenv ("FLUC_TTMLBLEND_COMPACT_PARAMS")) != 0;
+  return with_variant (kind, Hd.flags, [&] (auto K, auto L, auto G) {
+    if (compact && Hd.n_frames <= 4u && Hd.n_bands <= 16u)
+      return launch_group_variant<K, L, 4, 16, G> (P, o.grid, bulk_smem (K), stream);
+    if (compact && Hd.n_frames <= 32u)
+      return launch_group_variant<K, L, 32, kMaxGroupBands, G> (P, o.grid, bulk_smem (K), stream);
+    return launch_group_variant<K, L, kMaxPlainGroupFrames, kMaxGroupBands, G> (P, o.grid, bulk_smem (K), stream);
+  });
 }
 
 cudaError_t
@@ -1005,37 +986,16 @@ launch_multi (MultiParams &P, int kind, int sync, cudaStream_t stream)
   P.total_chunks = P.frame_begin[P.n_frames];
   if (P.total_chunks == 0)
     return cudaSuccess;
-  uint32_t lanes = interleave_lanes (kind);
-  if (P.total_chunks < lanes * 8u)
-    lanes = 1;
-  P.lanes = lanes;
-  P.per_lane = (P.total_chunks + lanes - 1) / lanes;
-  const uint32_t grid = lanes * P.per_lane;
-  if ((unsigned long long) grid * lanes >= (1ull << 32))
+  ChunkOrder o;
+  if (chunk_order (kind, P.total_chunks, o) != cudaSuccess)
     return cudaErrorInvalidValue;
-  P.lanes_magic = lanes == 1 ? 0u : (uint32_t) (((1ull << 32) + lanes - 1) / lanes);
-  const size_t smem_plane8 = 2 * kItemsPerChunk * 16, smem_packed = kItemsPerChunk * 16;
-  const int look = (P.flags & JF_LAZY) ? 1 : (P.flags & JF_OPAQUE) ? 2 : 0;
+  P.lanes = o.lanes;
+  P.per_lane = o.per_lane;
+  P.lanes_magic = o.magic;
   const bool pdl = (P.flags & JF_PDL) != 0;
-  const bool ga = (P.flags & JF_GA) != 0;
-#define MULTI_CASE(K, SM) \
-    case K: \
-      if (kind_is_planes (K) && ga) \
-        return look == 1 ? launch_ex (ttmlblend_multi_kernel<K, 1, kind_is_planes (K)>, grid, SM, stream, pdl, P) : \
-            look == 2 ? launch_ex (ttmlblend_multi_kernel<K, 2, kind_is_planes (K)>, grid, SM, stream, pdl, P) : \
-            launch_ex (ttmlblend_multi_kernel<K, 0, kind_is_planes (K)>, grid, SM, stream, pdl, P); \
-      return look == 1 ? launch_ex (ttmlblend_multi_kernel<K, 1>, grid, SM, stream, pdl, P) : \
-          look == 2 ? launch_ex (ttmlblend_multi_kernel<K, 2>, grid, SM, stream, pdl, P) : \
-          launch_ex (ttmlblend_multi_kernel<K, 0>, grid, SM, stream, pdl, P);
-  switch (kind) {
-    MULTI_CASE (PK_PLANE8, smem_plane8)
-    MULTI_CASE (PK_PLANE8_RGB, smem_plane8)
-    MULTI_CASE (PK_PACKED_A0, smem_packed)
-    MULTI_CASE (PK_PACKED_A3, smem_packed)
-    default:
-      return cudaErrorInvalidValue;
-  }
-#undef MULTI_CASE
+  return with_variant (kind, P.flags, [&] (auto K, auto L, auto G) {
+    return launch_ex (ttmlblend_multi_kernel<K, L, G>, o.grid, bulk_smem (K), stream, pdl, P);
+  });
 }
 
 cudaError_t
@@ -1044,23 +1004,15 @@ launch_blend (const PlaneJob *d_jobs, const uint32_t *d_chunk_begin, const uint3
 {
   if (n_jobs <= 0 || total_chunks == 0)
     return cudaSuccess;
-  switch (kind) {
-    case PK_PLANE8:
-      if (ga)
-        return launch_blend_kind<PK_PLANE8, true> (d_jobs, d_chunk_begin, d_coarse, n_jobs, total_chunks, fast, sync, stream);
-      return launch_blend_kind<PK_PLANE8> (d_jobs, d_chunk_begin, d_coarse, n_jobs, total_chunks, fast, sync, stream);
-    case PK_PLANE8_RGB:
-      if (ga)
-        return launch_blend_kind<PK_PLANE8_RGB, true> (d_jobs, d_chunk_begin, d_coarse, n_jobs, total_chunks, fast, sync,
-            stream);
-      return launch_blend_kind<PK_PLANE8_RGB> (d_jobs, d_chunk_begin, d_coarse, n_jobs, total_chunks, fast, sync, stream);
-    case PK_PACKED_A0:
-      return launch_blend_kind<PK_PACKED_A0> (d_jobs, d_chunk_begin, d_coarse, n_jobs, total_chunks, fast, sync, stream);
-    case PK_PACKED_A3:
-      return launch_blend_kind<PK_PACKED_A3> (d_jobs, d_chunk_begin, d_coarse, n_jobs, total_chunks, fast, sync, stream);
-    default:
-      return cudaErrorInvalidValue;
-  }
+  ChunkOrder o;
+  if (chunk_order (kind, total_chunks, o) != cudaSuccess)
+    return cudaErrorInvalidValue;
+  const bool pdl = (sync & JF_PDL) != 0;
+  /* the table kernel has no LAZY variants */
+  return with_variant (kind, ga ? JF_GA : 0, [&] (auto K, auto, auto G) {
+    return launch_ex (fast ? ttmlblend_blend_kernel<K, true, G> : ttmlblend_blend_kernel<K, false, G>, o.grid, 0,
+        stream, pdl, d_jobs, d_chunk_begin, d_coarse, n_jobs, total_chunks, o.lanes, o.per_lane, o.magic, sync);
+  });
 }
 
 /* ---------------------------------------------------------------------- */
