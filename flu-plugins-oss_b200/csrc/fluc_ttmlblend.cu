@@ -458,6 +458,16 @@ fluc_ttmlblend_overlay_set_global_alpha (FlucTtmlBlend *thiz, uint32_t stream, c
 }
 
 int
+fluc_ttmlblend_overlay_set_positions (FlucTtmlBlend *thiz, uint32_t stream, const int32_t *x, const int32_t *y,
+    uint32_t n)
+{
+  ENTER (thiz);
+  if (!x || !y)
+    return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
+  return overlay_set_positions (c, stream, x, y, n);
+}
+
+int
 fluc_ttmlblend_set_chroma_mode (FlucTtmlBlend *thiz, int mode)
 {
   ENTER (thiz);

@@ -115,13 +115,29 @@ prepare_overlay (Ctx *c, Overlay *ov, int format, int W, int H, Prepared **out)
   return 0;
 }
 
+/* One prepare launch of n_elems elements per row, counted -- or, with a batch (a move,
+ * overlay_set_positions), one item of its single launch. Averaged chroma keeps its own kernel. */
+static int
+issue_prepare (Ctx *c, const PrepareParams &pp, int n_elems, std::vector<PrepareItem> *batch)
+{
+  if (batch && !pp.chroma_average) {
+    if (n_elems > 0 && pp.rows > 0)
+      batch->push_back ({ pp, n_elems, 0 });
+    return 0;
+  }
+  CU (c, launch_prepare (pp, n_elems, c->up_stream));
+  c->stats.prepare_launches++;
+  return 0;
+}
+
 /* The prepare parameters every plane of a rectangle shares; false when nothing of it is inside
  * the frame. */
 static bool
 rect_params (const RawRect &rr, int format, int W, int H, PrepareParams &pp)
 {
-  /* gst_video_blend clipping: rr is already clipped at the left/top */
-  const int cx0 = rr.x, cy0 = rr.y;
+  /* gst_video_blend clipping at all four edges (a rectangle of the composition form keeps the
+   * part above / left of the frame on the device, raw pixel (0,0) at frame (rr.x, rr.y)) */
+  const int cx0 = std::max (rr.x, 0), cy0 = std::max (rr.y, 0);
   const int cx1 = std::min (rr.x + rr.w, W), cy1 = std::min (rr.y + rr.h, H);
   if (cx1 <= cx0 || cy1 <= cy0)
     return false;
@@ -146,7 +162,7 @@ rect_params (const RawRect &rr, int format, int W, int H, PrepareParams &pp)
  * Their planes go to `blocks`. */
 static int
 prepare_chroma (Ctx *c, PrepareParams pp, int format, bool avg, std::vector<std::shared_ptr<DevBlock>> *blocks,
-    PreparedRect &out)
+    PreparedRect &out, std::vector<PrepareItem> *batch)
 {
   const int n_planes = format_planes (format);
   const int sx = pp.sub_x, sy = pp.sub_y;
@@ -175,8 +191,8 @@ prepare_chroma (Ctx *c, PrepareParams pp, int format, bool avg, std::vector<std:
     pp.v0 = ref.v0;
     pp.row0 = by0;
     pp.rows = by1 - by0;
-    CU (c, launch_prepare (pp, ref.pitch, c->up_stream));
-    c->stats.prepare_launches++;
+    if ((rc = issue_prepare (c, pp, ref.pitch, batch)))
+      return rc;
     const int pu = format == FLUC_TTMLBLEND_FORMAT_YV12 ? 2 : 1;
     const int pv = 3 - pu;
     ref.a = a;
@@ -204,8 +220,8 @@ prepare_chroma (Ctx *c, PrepareParams pp, int format, bool avg, std::vector<std:
     pp.v0 = ref.v0;
     pp.row0 = by0;
     pp.rows = by1 - by0;
-    CU (c, launch_prepare (pp, ref.pitch / 2, c->up_stream));
-    c->stats.prepare_launches++;
+    if ((rc = issue_prepare (c, pp, ref.pitch / 2, batch)))
+      return rc;
     ref.a = a;
     ref.c = uv;
     out.refs[out.n_refs++] = { 1, ref };
@@ -223,15 +239,16 @@ prepare_avg_chroma (Ctx *c, PrepareParams pp, int format, int ga, PreparedRect &
   if (ga == 0)
     return 0;
   pp.ga = ga;
-  return prepare_chroma (c, pp, format, true, &out.avg_blocks, out);
+  return prepare_chroma (c, pp, format, true, &out.avg_blocks, out, nullptr);
 }
 
 /* Prepares one rectangle for one destination format: allocates its planes, runs the prepare
- * kernel(s) on the upload stream, and notes how each destination plane sees it. ga_now is the
- * current global alpha of its box, which only averaged chroma folds in. */
+ * kernel(s) on the upload stream (or adds them to `batch`, issue_prepare), and notes how each
+ * destination plane sees it. ga_now is the current global alpha of its box, which only averaged
+ * chroma folds in. */
 static int
 prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_average, int ga_now,
-    PreparedRect &out)
+    PreparedRect &out, std::vector<PrepareItem> *batch = nullptr)
 {
   const int kind = plane_kind (format);
   PrepareParams pp;
@@ -264,8 +281,8 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
     pp.v0 = ref.v0;
     pp.row0 = cy0;
     pp.rows = cy1 - cy0;
-    CU (c, launch_prepare (pp, ref.pitch / 4, c->up_stream));
-    c->stats.prepare_launches++;
+    if ((rc = issue_prepare (c, pp, ref.pitch / 4, batch)))
+      return rc;
     out.refs[out.n_refs++] = { 0, ref };
   } else if (kind == PK_PLANE8_RGB || (kind == PK_PLANE8 && format_packed_444_3 (format))) {
     /* v308 / IYU2 / RGB / BGR: one plane, three bytes per pixel, every byte its own alpha +
@@ -295,8 +312,8 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
     pp.v0 = ref.v0;
     pp.row0 = cy0;
     pp.rows = cy1 - cy0;
-    CU (c, launch_prepare (pp, ref.pitch, c->up_stream));
-    c->stats.prepare_launches++;
+    if ((rc = issue_prepare (c, pp, ref.pitch, batch)))
+      return rc;
     out.refs[out.n_refs++] = { 0, ref };
   } else if (kind == PK_PLANE8) {
     /* luma plane: byte == pixel */
@@ -321,13 +338,13 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
       pp.v0 = ref.v0;
       pp.row0 = cy0;
       pp.rows = cy1 - cy0;
-      CU (c, launch_prepare (pp, ref.pitch, c->up_stream));
-      c->stats.prepare_launches++;
+      if ((rc = issue_prepare (c, pp, ref.pitch, batch)))
+        return rc;
       out.refs[out.n_refs++] = { 0, ref };
     }
     if (chroma_average && pp.sub_x == 2 && pp.sub_y == 2)
       return prepare_avg_chroma (c, pp, format, ga_now, out);
-    return prepare_chroma (c, pp, format, false, &out.blocks, out);
+    return prepare_chroma (c, pp, format, false, &out.blocks, out, batch);
   } else {
     RectRef ref = {};
     ref.v0 = cx0 / 4;
@@ -355,8 +372,8 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
     pp.v0 = ref.v0;
     pp.row0 = cy0;
     pp.rows = cy1 - cy0;
-    CU (c, launch_prepare (pp, ref.pitch / 4, c->up_stream));
-    c->stats.prepare_launches++;
+    if ((rc = issue_prepare (c, pp, ref.pitch / 4, batch)))
+      return rc;
     ref.a = w;
     ref.c = nullptr;
     out.refs[out.n_refs++] = { 0, ref };
@@ -367,9 +384,11 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
 /* The rectangle tables of P with every box's current global alpha: a box at 0 drops out (no
  * band, no window in place), the others give it to the blend where the prepare did not fold it
  * in -- RectRef::ga for the Cs*ga terms, RectRef::a_ga for the alpha bytes of the PLANE8 kinds.
- * Averaged 4:2:0 chroma has it folded in (prepare_avg_chroma). */
+ * Averaged 4:2:0 chroma has it folded in (prepare_avg_chroma). A move's batch of prepares
+ * (overlay_set_positions) goes out here as one launch; when its items do not fit in the kernel
+ * parameters they are uploaded in the tables' allocation, behind them. */
 static int
-prepare_assemble (Ctx *c, Prepared *P, const Overlay *ov)
+prepare_assemble (Ctx *c, Prepared *P, const Overlay *ov, std::vector<PrepareItem> *batch = nullptr)
 {
   for (int pl = 0; pl < 3; pl++)
     P->h_rects[pl].clear ();
@@ -404,13 +423,31 @@ prepare_assemble (Ctx *c, Prepared *P, const Overlay *ov)
       P->rect_off[pl] = (int32_t) total;
       total += P->h_rects[pl].size ();
     }
+    const uint32_t n_items = batch ? (uint32_t) batch->size () : 0;
+    const uint32_t ctas = n_items ? prepare_batch_plan (batch->data (), n_items) : 0;
+    const size_t item_bytes = n_items > kPrepareBatchInline ? n_items * sizeof (PrepareItem) : 0;
+    if (total || item_bytes) {
+      int rc;
+      if ((rc = dev_block (c, total * sizeof (RectRef) + item_bytes, &P->table_block)))
+        return rc;
+    }
+    if (n_items) {
+      const PrepareItem *d_items = nullptr;
+      if (item_bytes) {
+        P->h_items = std::move (*batch);      /* the async copy's source lives as long as P */
+        d_items = reinterpret_cast<const PrepareItem *> (static_cast<uint8_t *> (P->table_block->ptr) +
+            total * sizeof (RectRef));
+        CU (c, cudaMemcpyAsync ((void *) d_items, P->h_items.data (), item_bytes, cudaMemcpyHostToDevice,
+                c->up_stream));
+      }
+      CU (c, launch_prepare_batch (item_bytes ? P->h_items.data () : batch->data (), n_items, d_items, ctas,
+              c->up_stream));
+      c->stats.prepare_launches++;
+    }
     if (total) {
       P->h_rects_all.clear ();
       for (int pl = 0; pl < 3; pl++)
         P->h_rects_all.insert (P->h_rects_all.end (), P->h_rects[pl].begin (), P->h_rects[pl].end ());
-      int rc;
-      if ((rc = dev_block (c, total * sizeof (RectRef), &P->table_block)))
-        return rc;
       uint8_t *d = static_cast<uint8_t *> (P->table_block->ptr);
       /* h_rects_all lives as long as the Prepared: safe source for the async copy */
       CU (c, cudaMemcpyAsync (d, P->h_rects_all.data (), total * sizeof (RectRef),
@@ -436,6 +473,19 @@ box_ga (const Overlay *ov, size_t i)
   return ov->rects[i].ga;
 }
 
+/* the pixels of ov's rectangles as handed in, clipped to a W x H frame (algorithmic bytes) */
+static uint64_t
+declared_px (const Overlay *ov, int W, int H)
+{
+  uint64_t px = 0;
+  for (const FlucTtmlBlendRect &d : ov->declared) {
+    const int w = std::min (d.x + d.w, W) - std::max (d.x, 0), h = std::min (d.y + d.h, H) - std::max (d.y, 0);
+    if (w > 0 && h > 0)
+      px += (uint64_t) w * (uint64_t) h;
+  }
+  return px;
+}
+
 static int
 prepare_build (Ctx *c, Overlay *ov, int format, int W, int H, std::unique_ptr<Prepared> &P)
 {
@@ -443,11 +493,7 @@ prepare_build (Ctx *c, Overlay *ov, int format, int W, int H, std::unique_ptr<Pr
   P->W = W;
   P->H = H;
   P->chroma_average = c->chroma_average;
-  for (const FlucTtmlBlendRect &d : ov->declared) {
-    const int w = std::min (d.x + d.w, W) - d.x, h = std::min (d.y + d.h, H) - d.y;
-    if (w > 0 && h > 0)
-      P->overlay_px += (uint64_t) w * (uint64_t) h;
-  }
+  P->overlay_px = declared_px (ov, W, H);
   P->per_rect.resize (ov->rects.size ());
   for (size_t i = 0; i < ov->rects.size (); i++) {
     const int rc = prepare_rect (c, ov->rects[i], format, W, H, P->chroma_average, box_ga (ov, i), P->per_rect[i]);
@@ -788,6 +834,7 @@ overlay_install (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, cons
   ov->image_w = image_w;
   ov->image_h = image_h;
   ov->updatable = image_w > 0 && image_h > 0;
+  ov->movable = !ov->updatable;
   ov->n_alphas = std::max<uint32_t> (1, n);
   std::vector<Up> ups;
   std::vector<std::vector<int4>> plans;     /* host side of async uploads: alive until finish_install */
@@ -802,8 +849,10 @@ overlay_install (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, cons
     /* gst_video_overlay_rectangle_needs_scaling: render size != pixel size */
     const int rw = r.render_width ? r.render_width : r.width, rh = r.render_height ? r.render_height : r.height;
     const bool scaled = rw != r.width || rh != r.height;
-    /* gst_video_blend: negative offsets skip source columns / rows */
-    const int xoff = r.x < 0 ? -r.x : 0, yoff = r.y < 0 ? -r.y : 0;
+    /* gst_video_blend: negative offsets skip source columns / rows. The composition form keeps
+     * them on the device all the same, clipped at prepare time (rect_params), so that
+     * overlay_set_positions can bring them into the frame later. */
+    const int xoff = (!ov->movable && r.x < 0) ? -r.x : 0, yoff = (!ov->movable && r.y < 0) ? -r.y : 0;
     if (xoff >= rw || yoff >= rh)
       continue;
     Up u;
@@ -1034,6 +1083,7 @@ overlay_set_alpha (Ctx *c, uint32_t stream, const int *ga, uint32_t n)
   nv->image_w = old->image_w;
   nv->image_h = old->image_h;
   nv->updatable = old->updatable;
+  nv->movable = old->movable;
   nv->n_alphas = old->n_alphas;
   std::vector<bool> again (nv->rects.size (), false);   /* prepared once more, without a global alpha */
   bool changed = false;
@@ -1085,6 +1135,88 @@ overlay_set_alpha (Ctx *c, uint32_t stream, const int *ga, uint32_t n)
     }
     if (!rc)
       rc = prepare_assemble (c, P.get (), nv.get ());
+    if (rc) {
+      if (P->ready)
+        cudaEventDestroy (P->ready);
+      return rc;
+    }
+    nv->prepared.push_back (std::move (P));
+  }
+  c->overlays[stream] = nv;       /* frames already queued keep the old one */
+  return 0;
+}
+
+/* overlay_set_positions: a new generation of the stream's overlay whose boxes sit at (x[i], y[i])
+ * (box i = rectangle i of overlay_set_rectangles). It shares every raw block; the crop runs are in
+ * the rectangle's own coordinates and move with it. What depends on the position -- the shift
+ * onto each destination plane's 16-byte grid, the chroma siting, the clipping at the frame
+ * edges -- is prepared again from the resident pixels for every moved rectangle: one batch launch
+ * per (format, size) the old generation was prepared for, on the upload stream, waited for through
+ * Prepared::ready like a cue change. Global alphas carry over; averaged 4:2:0 chroma is prepared
+ * again at the box's current value by its own kernel. Rectangles that stay keep their planes. */
+int
+overlay_set_positions (Ctx *c, uint32_t stream, const int32_t *x, const int32_t *y, uint32_t n)
+{
+  NvtxRange nvtx ("ttmlblend.overlay_set_positions");
+  auto it = c->overlays.find (stream);
+  if (it == c->overlays.end ())
+    return FLUC_TTMLBLEND_ERROR_NOT_FOUND;
+  const std::shared_ptr<Overlay> old = it->second;
+  if (!old->movable || n != old->boxes.size ())
+    return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
+  for (const OverlayBox &b : old->boxes)
+    if ((int64_t) x[b.slot] + b.declared.w > INT32_MAX || (int64_t) y[b.slot] + b.declared.h > INT32_MAX)
+      return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
+  std::shared_ptr<Overlay> nv (new Overlay ());
+  nv->ctx = c;
+  nv->rects = old->rects;
+  nv->boxes = old->boxes;
+  nv->declared = old->declared;
+  nv->image_w = old->image_w;
+  nv->image_h = old->image_h;
+  nv->updatable = old->updatable;
+  nv->movable = old->movable;
+  nv->n_alphas = old->n_alphas;
+  std::vector<bool> moved (nv->rects.size (), false);
+  bool changed = false;
+  for (OverlayBox &b : nv->boxes) {
+    const int bx = x[b.slot], by = y[b.slot];
+    if (bx == b.declared.x && by == b.declared.y)
+      continue;
+    changed = true;
+    for (uint32_t i = b.first_rect; i < b.first_rect + b.n_rects; i++) {
+      RawRect &rr = nv->rects[i];
+      rr.x = bx + (rr.x - b.declared.x);      /* the crop run's offset inside the rectangle */
+      rr.y = by + (rr.y - b.declared.y);
+      moved[i] = true;
+    }
+    b.declared.x = bx;
+    b.declared.y = by;
+    nv->declared[b.slot] = b.declared;
+  }
+  if (!changed)
+    return 0;
+  decide_lazy (nv.get ());
+  for (auto &p : old->prepared) {
+    std::unique_ptr<Prepared> P (new Prepared ());
+    P->format = p->format;
+    P->W = p->W;
+    P->H = p->H;
+    P->chroma_average = p->chroma_average;
+    P->overlay_px = declared_px (nv.get (), P->W, P->H);
+    P->used = p->used;
+    P->per_rect.resize (nv->rects.size ());
+    std::vector<PrepareItem> batch;
+    int rc = 0;
+    for (size_t i = 0; i < nv->rects.size () && !rc; i++) {
+      if (moved[i])
+        rc = prepare_rect (c, nv->rects[i], P->format, P->W, P->H, P->chroma_average, box_ga (nv.get (), i),
+            P->per_rect[i], &batch);
+      else
+        P->per_rect[i] = p->per_rect[i];
+    }
+    if (!rc)
+      rc = prepare_assemble (c, P.get (), nv.get (), &batch);
     if (rc) {
       if (P->ready)
         cudaEventDestroy (P->ready);

@@ -254,7 +254,9 @@ struct DevBlock {
   ~DevBlock ();
 };
 
-/* device copy of one rectangle's BGRA pixels (left/top clipped at 0) */
+/* device copy of one rectangle's BGRA pixels: (x, y) is the frame position of its pixel (0,0).
+ * Clipped at the left / top for the ttmlrender and region forms; the composition form keeps the
+ * whole rectangle, so x and y may be negative (overlay_set_positions) */
 struct RawRect {
   std::shared_ptr<DevBlock> block;     /* the allocation `dev` points into */
   uint8_t *dev = nullptr;
@@ -321,6 +323,7 @@ struct Prepared {
   int32_t rect_off[3] = { 0, 0, 0 };   /* first entry of plane p in d_rects_all */
   uint64_t overlay_px = 0;             /* sum of clipped w*h */
   bool fade = false;                   /* a RectRef has a_ga != 255: launches holding it take the JF_GA variant */
+  std::vector<PrepareItem> h_items;    /* a move's batch prepare items, when uploaded (source of the async copy) */
   cudaEvent_t ready = nullptr;
   bool blend_waited = false;           /* blend stream already ordered after `ready` */
   bool used = false;                   /* a frame has been blended with it (worth preparing the next cue for) */
@@ -330,7 +333,7 @@ struct Prepared {
 /* One rectangle as it was handed in (a region box of ttmlrender's image): the unit a cue update
  * keeps or replaces. */
 struct OverlayBox {
-  FlucTtmlBlendRect declared = { 0, 0, 0, 0 };       /* frame coordinates, clipped at the left / top */
+  FlucTtmlBlendRect declared = { 0, 0, 0, 0 };       /* frame coordinates (clipped at the left / top but for the composition form) */
   uint32_t first_rect = 0, n_rects = 0;              /* its cropped sub-rectangles in Overlay::rects */
   uint64_t groups_all = 0, groups_on = 0, groups_opaque = 0;   /* 16-pixel groups under them: all / some alpha / alpha 255 */
   int ga = 255;                        /* its current global alpha (overlay_set_global_alpha) */
@@ -346,6 +349,7 @@ struct Overlay {
    * alpha 1 -- what overlay_update can patch */
   int image_w = 0, image_h = 0;
   bool updatable = false;
+  bool movable = false;                /* composition form (overlay_set_rectangles): overlay_set_positions takes it */
   uint32_t n_alphas = 1;               /* global alphas overlay_set_global_alpha takes besides one for all */
   std::vector<std::unique_ptr<Prepared>> prepared;
   double transparent_fraction = 0.0;   /* of the 16-pixel groups under the kept rectangles */
@@ -712,6 +716,8 @@ int overlay_install_regions (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t 
     const FlucTtmlBlendRegion *regions, uint32_t n);
 /* ga: n values 0..255, one for every box or (n == 1) for all; mu held throughout */
 int overlay_set_alpha (Ctx *c, uint32_t stream, const int *ga, uint32_t n);
+/* x, y: one position per box (n == the number of rectangles installed); mu held throughout */
+int overlay_set_positions (Ctx *c, uint32_t stream, const int32_t *x, const int32_t *y, uint32_t n);
 
 /* jobs.cu */
 void layout_spans (const Layout *L, std::vector<StageSpan> &out);

@@ -1046,15 +1046,12 @@ raw_px (const PrepareParams &p, int x, int y)
       + (size_t) (x - p.fx) * 4);
 }
 
-/* One thread per prepared element: a pixel (luma, packed), a chroma sample
- * (planar chroma) or a chroma pair (semi-planar chroma). */
-__global__ void __launch_bounds__ (256)
-ttmlblend_prepare_kernel (const PrepareParams p, int n_elems)
+/* One prepared element: a pixel (luma, packed), a chroma sample (planar chroma) or a chroma
+ * pair (semi-planar chroma), element i of prepared row r. The one definition of the prepare
+ * arithmetic for both prepare kernels. */
+__device__ __forceinline__ void
+prepare_elem (const PrepareParams &p, int i, int r)
 {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  const int r = blockIdx.y;
-  if (i >= n_elems || r >= p.rows)
-    return;
   const size_t orow = (size_t) r * p.out_pitch;
   const bool premul = p.premul != 0;
 
@@ -1228,6 +1225,43 @@ ttmlblend_prepare_kernel (const PrepareParams p, int n_elems)
   }
 }
 
+/* One thread per prepared element of one rectangle's plane(s). */
+__global__ void __launch_bounds__ (256)
+ttmlblend_prepare_kernel (const PrepareParams p, int n_elems)
+{
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const int r = blockIdx.y;
+  if (i >= n_elems || r >= p.rows)
+    return;
+  prepare_elem (p, i, r);
+}
+
+/* Every plane of every rectangle of one overlay_set_positions generation in one launch: a CTA
+ * finds its item by bisecting the items' first CTAs (prefix sums of their element counts in
+ * whole CTAs, uniform across the CTA), then takes elements row-major inside it. The items sit in
+ * the kernel parameters, or in device memory when there are more than fit there. */
+__global__ void __launch_bounds__ (256)
+ttmlblend_prepare_batch_kernel (const __grid_constant__ PrepareBatch B)
+{
+  const PrepareItem *items = B.items ? B.items : B.inl;
+  const uint32_t cta = blockIdx.x;
+  uint32_t lo = 0, hi = B.n_items;            /* the last item whose first CTA is <= cta */
+  while (hi - lo > 1) {
+    const uint32_t m = (lo + hi) / 2;
+    if (items[m].cta0 <= cta)
+      lo = m;
+    else
+      hi = m;
+  }
+  const PrepareItem &it = items[lo];
+  const int64_t e = (int64_t) (cta - it.cta0) * 256 + threadIdx.x;
+  const int n = it.n_elems;
+  if (e >= (int64_t) n * it.p.rows)
+    return;
+  const int r = (int) (e / n);
+  prepare_elem (it.p, (int) (e - (int64_t) r * n), r);
+}
+
 /* NON-PARITY option (fluc_ttmlblend_set_chroma_mode): each 4:2:0 chroma sample takes the
  * alpha-weighted mean colour and the mean alpha of its 2x2 luma pixels instead of the
  * pixel sited at (even x, even y). GStreamer does not do this (BLENDSPEC section 4), so the
@@ -1309,6 +1343,32 @@ launch_prepare (const PrepareParams &p, int n_elems, cudaStream_t stream)
     dim3 grid ((n_elems + 255) / 256, nr);
     ttmlblend_prepare_kernel<<<grid, 256, 0, stream>>> (q, n_elems);
   }
+  return cudaGetLastError ();
+}
+
+uint32_t
+prepare_batch_plan (PrepareItem *items, uint32_t n)
+{
+  uint32_t ctas = 0;
+  for (uint32_t k = 0; k < n; k++) {
+    items[k].cta0 = ctas;
+    ctas += (uint32_t) (((uint64_t) items[k].n_elems * (uint64_t) items[k].p.rows + 255) / 256);
+  }
+  return ctas;
+}
+
+cudaError_t
+launch_prepare_batch (const PrepareItem *items, uint32_t n, const PrepareItem *d_items, uint32_t ctas,
+    cudaStream_t stream)
+{
+  if (n == 0 || ctas == 0)
+    return cudaSuccess;
+  PrepareBatch B;
+  B.n_items = n;
+  B.items = n > kPrepareBatchInline ? d_items : nullptr;
+  if (!B.items)
+    memcpy (B.inl, items, n * sizeof (PrepareItem));
+  ttmlblend_prepare_batch_kernel<<<ctas, 256, 0, stream>>> (B);
   return cudaGetLastError ();
 }
 

@@ -216,6 +216,23 @@ enum PrepareMode : int32_t {
   PM_BGR24 = 16
 };
 
+/* One item of a batch prepare: one launch_prepare's work (n_elems elements per row, p.rows rows),
+ * starting at CTA cta0 of the batch launch. */
+struct alignas (16) PrepareItem {
+  PrepareParams p;
+  int32_t n_elems;
+  uint32_t cta0;
+};
+/* items kept in the kernel parameters (4 KB of them); more are read from device memory */
+constexpr uint32_t kPrepareBatchInline = 31;
+struct PrepareBatch {
+  const PrepareItem *items;     /* device copy of the items, or nullptr: inl */
+  uint32_t n_items;
+  uint32_t pad_[2];
+  PrepareItem inl[kPrepareBatchInline];
+};
+static_assert (sizeof (PrepareBatch) <= 4096, "batch prepare parameters");
+
 /* All jobs of one launch share one PlaneKind and one variant: fast (every
  * job 16-byte aligned with row_bytes % 16 == 0) or byte-granular. */
 /* d_coarse[i] = index of the job that holds chunk i << kCoarseShift. */
@@ -231,6 +248,13 @@ cudaError_t launch_group (GroupParams &P, int kind, int sync, cudaStream_t strea
 cudaError_t launch_multi (MultiParams &P, int kind, int sync, cudaStream_t stream);
 /* n_elems = prepared elements per row (see PrepareMode). */
 cudaError_t launch_prepare (const PrepareParams &p, int n_elems, cudaStream_t stream);
+/* Fills in every item's cta0 (items without elements get none) and returns the CTAs of the batch. */
+uint32_t prepare_batch_plan (PrepareItem *items, uint32_t n);
+/* One launch of ttmlblend_prepare_batch_kernel for items[0..n) (n >= 1, planned): in the kernel
+ * parameters when n <= kPrepareBatchInline, otherwise read from d_items, a device copy of them
+ * ordered before the launch on `stream`. */
+cudaError_t launch_prepare_batch (const PrepareItem *items, uint32_t n, const PrepareItem *d_items, uint32_t ctas,
+    cudaStream_t stream);
 cudaError_t launch_scrub (uint8_t *buf, size_t bytes, cudaStream_t stream);
 /* bench helper: reads and rewrites `bytes` (multiple of 16) of mapped host memory in place */
 cudaError_t launch_pcie_probe (uint8_t *buf, size_t bytes, cudaStream_t stream);

@@ -100,6 +100,8 @@ PROTOTYPES = {
     "fluc_ttmlblend_overlay_clear": (C.c_int, [C.c_void_p, C.c_uint32]),
     "fluc_ttmlblend_overlay_set_global_alpha": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_float),
                                                           C.c_uint32]),
+    "fluc_ttmlblend_overlay_set_positions": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_int32),
+                                                       C.POINTER(C.c_int32), C.c_uint32]),
     "fluc_ttmlblend_set_chroma_mode": (C.c_int, [C.c_void_p, C.c_int]),
     "fluc_ttmlblend_submit": (C.c_int, [C.c_void_p, C.c_uint32, C.c_int, C.c_int32, C.c_int32,
                                         C.c_uint32, C.POINTER(Frame), C.POINTER(Frame),
@@ -367,6 +369,18 @@ class TtmlBlend:
         arr = (C.c_float * max(1, len(vals)))(*vals)
         self._check(self.lib.fluc_ttmlblend_overlay_set_global_alpha(self.h, stream, arr, len(vals)),
                     "overlay_set_global_alpha")
+
+    def overlay_set_positions(self, stream: int, xs: Sequence[int], ys: Sequence[int]):
+        """gst_video_overlay_rectangle_set_render_rectangle for the position only: rectangle i of
+        the stream's overlay_set_rectangles list goes to (xs[i], ys[i]), without a new upload, scale
+        or scan. Frames submitted afterwards blend the rectangles at their new positions."""
+        xl, yl = [int(v) for v in xs], [int(v) for v in ys]
+        if len(xl) != len(yl):
+            raise ValueError("overlay_set_positions: xs and ys differ in length")
+        ax = (C.c_int32 * max(1, len(xl)))(*xl)
+        ay = (C.c_int32 * max(1, len(yl)))(*yl)
+        self._check(self.lib.fluc_ttmlblend_overlay_set_positions(self.h, stream, ax, ay, len(xl)),
+                    "overlay_set_positions")
 
     def set_chroma_mode(self, average: bool):
         """False (default): GStreamer's sited chroma, bit-exact. True: 2x2 mean, NOT bit-exact."""

@@ -224,7 +224,10 @@ FLUC_EXPORT int fluc_ttmlblend_overlay_set (FlucTtmlBlend *thiz, uint32_t stream
 FLUC_EXPORT int fluc_ttmlblend_overlay_update (FlucTtmlBlend *thiz, uint32_t stream,
     const uint8_t *bgra_premul, int32_t w, int32_t h, int32_t stride,
     const FlucTtmlBlendRect *changed_rects, uint32_t n_changed);
-/* GstVideoOverlayComposition form: independent rectangles, blended in order. */
+/* GstVideoOverlayComposition form: independent rectangles, blended in order. Each rectangle is
+ * kept whole on the device, also the part that lies above or left of the frame (or all of it),
+ * so that overlay_set_positions can move it in later: such rectangles count those pixels in
+ * h2d_bytes and cache_bytes. The blended frames do not depend on it. */
 FLUC_EXPORT int fluc_ttmlblend_overlay_set_rectangles (FlucTtmlBlend *thiz,
     uint32_t stream, const FlucTtmlBlendRectangle *rects, uint32_t n_rects);
 /* Region form (SURVEY.md section 8f rank 3): the overlay is composed on the GPU from region
@@ -268,6 +271,24 @@ FLUC_EXPORT int fluc_ttmlblend_overlay_clear (FlucTtmlBlend *thiz, uint32_t stre
  * a value outside [0, 1]. */
 FLUC_EXPORT int fluc_ttmlblend_overlay_set_global_alpha (FlucTtmlBlend *thiz, uint32_t stream,
     const float *global_alpha, uint32_t n);
+
+/* gst_video_overlay_rectangle_set_render_rectangle for the position only: rectangle i of the
+ * stream's overlay_set_rectangles list (in list order, including rectangles outside the frame)
+ * is placed at (x[i], y[i]). Nothing is uploaded, scaled or scanned again. The render size stays
+ * the one the rectangle was installed with. Frames submitted after the call (submit*,
+ * submit_many_after, blend_host*) are blended exactly as overlay_set_rectangles with the moved
+ * rectangles would blend them. Frames already submitted keep the old positions.
+ * The rectangles keep their current global alphas, and overlay_set_global_alpha after a move
+ * keeps the positions; overlay_set* / overlay_clear start again from the new cue. A move
+ * prepares the moved rectangles again from their resident pixels on the GPU, in one kernel
+ * launch per destination format and size the stream has been blended in (under
+ * FLUC_TTMLBLEND_CHROMA_AVERAGE, plus one launch per moved rectangle for its averaged chroma).
+ * Unchanged positions: nothing is done. Returns NOT_FOUND when the stream has no overlay,
+ * INVALID_ARGUMENT for NULL arrays, n different from the number of rectangles installed, an
+ * overlay installed by overlay_set, overlay_update or overlay_set_regions, or a position at which
+ * x + render width or y + render height overflows int32_t. */
+FLUC_EXPORT int fluc_ttmlblend_overlay_set_positions (FlucTtmlBlend *thiz, uint32_t stream,
+    const int32_t *x, const int32_t *y, uint32_t n);
 
 /* How the overlay reaches the chroma planes of 4:2:0 frames. SITED (default) is what
  * GStreamer does and the only bit-exact mode: a chroma sample takes the overlay pixel at
