@@ -6,6 +6,8 @@
  */
 #include "ttmlblend_internal.h"
 
+#include <numeric>
+
 namespace tbh {
 
 /* Frees device memory once everything already queued on any of the
@@ -54,15 +56,28 @@ Overlay::~Overlay ()
         take (b);
     }
     take (p->table_block);
-    if (p->ready)
-      cudaEventDestroy (p->ready);
   }
   if (ctx)
     free_deferred (ctx, ptrs);
 }
 
+Prepared::~Prepared ()
+{
+  if (ready)
+    cudaEventDestroy (ready);
+}
+
 /* ---------------------------------------------------------------------- */
 /* prepare: raw BGRA rectangle -> per-plane prepared overlay              */
+
+static std::shared_ptr<DevBlock>
+make_block (Ctx *c, void *ptr)
+{
+  std::shared_ptr<DevBlock> b (new DevBlock ());
+  b->ctx = c;
+  b->ptr = ptr;
+  return b;
+}
 
 /* a stream-ordered allocation on the upload stream */
 static int
@@ -70,10 +85,7 @@ dev_block (Ctx *c, size_t bytes, std::shared_ptr<DevBlock> *out)
 {
   void *ptr = nullptr;
   CU (c, cudaMallocFromPoolAsync (&ptr, std::max<size_t> (bytes, 16), c->mem_pool, c->up_stream));
-  std::shared_ptr<DevBlock> b (new DevBlock ());
-  b->ctx = c;
-  b->ptr = ptr;
-  *out = std::move (b);
+  *out = make_block (c, ptr);
   return 0;
 }
 
@@ -86,32 +98,6 @@ dev_alloc (Ctx *c, std::vector<std::shared_ptr<DevBlock>> *blocks, size_t bytes,
     return rc;
   *out = static_cast<uint8_t *> (b->ptr);
   blocks->push_back (std::move (b));
-  return 0;
-}
-
-static int prepare_build (Ctx *c, Overlay *ov, int format, int W, int H, std::unique_ptr<Prepared> &P);
-
-int
-prepare_overlay (Ctx *c, Overlay *ov, int format, int W, int H, Prepared **out)
-{
-  for (auto &p : ov->prepared)
-    if (p->format == format && p->W == W && p->H == H && p->chroma_average == c->chroma_average) {
-      *out = p.get ();
-      return 0;
-    }
-
-  NvtxRange nvtx ("ttmlblend.prepare_overlay");
-  TBLOG (2, "prepare overlay: format %d, %dx%d, %zu rectangle(s)", format, W, H, ov->rects.size ());
-  std::unique_ptr<Prepared> P (new Prepared ());
-  const int rc = prepare_build (c, ov, format, W, H, P);
-  if (rc) {
-    /* half-built (out of memory, too many rectangles): its blocks go back with it */
-    if (P->ready)
-      cudaEventDestroy (P->ready);
-    return rc;
-  }
-  *out = P.get ();
-  ov->prepared.push_back (std::move (P));
   return 0;
 }
 
@@ -156,10 +142,44 @@ rect_params (const RawRect &rr, int format, int W, int H, PrepareParams &pp)
   return true;
 }
 
+/* One plane group of a rectangle: n_planes planes (alpha first) over the byte columns [b0, b1)
+ * of a destination plane, widened to whole 16-byte vectors, and its rows [y0, y1), prepared in
+ * `mode` with elem_bytes bytes per kernel element. Their blocks go to `blocks`. `ref` gets the
+ * span, ga 255 and the first two planes; `planes` all of them. */
+static int
+prepare_planes (Ctx *c, PrepareParams &pp, int mode, int b0, int b1, int y0, int y1, int n_planes, int elem_bytes,
+    std::vector<std::shared_ptr<DevBlock>> *blocks, std::vector<PrepareItem> *batch, RectRef &ref, uint8_t *planes[3])
+{
+  ref = {};
+  ref.v0 = b0 / 16;
+  ref.v1 = ceil_div (b1, 16);
+  ref.y0 = y0;
+  ref.y1 = y1;
+  ref.pitch = (ref.v1 - ref.v0) * 16;
+  ref.ga = 255;
+  const size_t bytes = (size_t) ref.pitch * (y1 - y0);
+  for (int k = 0; k < 3; k++)
+    planes[k] = nullptr;
+  for (int k = 0; k < n_planes; k++) {
+    const int rc = dev_alloc (c, blocks, bytes, &planes[k]);
+    if (rc)
+      return rc;
+  }
+  ref.a = planes[0];
+  ref.c = planes[1];
+  pp.mode = mode;
+  pp.out_a = planes[0]; pp.out_c = planes[1]; pp.out_c2 = planes[2];
+  pp.out_pitch = ref.pitch;
+  pp.v0 = ref.v0;
+  pp.row0 = y0;
+  pp.rows = y1 - y0;
+  return issue_prepare (c, pp, ref.pitch / elem_bytes, batch);
+}
+
 /* The chroma planes of a planar / semi-planar YUV format: the samples sited on the even pixel
  * of each pair / the even line of each line pair, as far as the format subsamples (parity);
  * with the non-parity 2x2 average of 4:2:0 (avg) every sample with at least one covered pixel.
- * Their planes go to `blocks`. */
+ * Nothing for the one-plane formats. Their planes go to `blocks`. */
 static int
 prepare_chroma (Ctx *c, PrepareParams pp, int format, bool avg, std::vector<std::shared_ptr<DevBlock>> *blocks,
     PreparedRect &out, std::vector<PrepareItem> *batch)
@@ -171,59 +191,23 @@ prepare_chroma (Ctx *c, PrepareParams pp, int format, bool avg, std::vector<std:
   const int by0 = avg ? pp.cy0 / 2 : ceil_div (pp.cy0, sy), by1 = ceil_div (pp.cy1, sy);
   if (n_planes < 2 || bx1 <= bx0 || by1 <= by0)
     return 0;
+  RectRef ref;
+  uint8_t *planes[3];
+  int rc;
   if (n_planes == 3) {
-    RectRef ref = {};
-    ref.v0 = bx0 / 16;
-    ref.v1 = ceil_div (bx1, 16);
-    ref.y0 = by0;
-    ref.y1 = by1;
-    ref.pitch = (ref.v1 - ref.v0) * 16;
-    ref.ga = 255;
-    const size_t bytes = (size_t) ref.pitch * (by1 - by0);
-    uint8_t *a, *u, *v;
-    int rc;
-    if ((rc = dev_alloc (c, blocks, bytes, &a)) || (rc = dev_alloc (c, blocks, bytes, &u))
-        || (rc = dev_alloc (c, blocks, bytes, &v)))
-      return rc;
-    pp.mode = PM_CHROMA_PLANAR;
-    pp.out_a = a; pp.out_c = u; pp.out_c2 = v;
-    pp.out_pitch = ref.pitch;
-    pp.v0 = ref.v0;
-    pp.row0 = by0;
-    pp.rows = by1 - by0;
-    if ((rc = issue_prepare (c, pp, ref.pitch, batch)))
+    /* alpha, U, V: one byte per sample */
+    if ((rc = prepare_planes (c, pp, PM_CHROMA_PLANAR, bx0, bx1, by0, by1, 3, 1, blocks, batch, ref, planes)))
       return rc;
     const int pu = format == FLUC_TTMLBLEND_FORMAT_YV12 ? 2 : 1;
-    const int pv = 3 - pu;
-    ref.a = a;
-    ref.c = u;
     out.refs[out.n_refs++] = { pu, ref };
-    ref.c = v;
-    out.refs[out.n_refs++] = { pv, ref };
+    ref.c = planes[2];
+    out.refs[out.n_refs++] = { 3 - pu, ref };
   } else {
-    RectRef ref = {};
-    ref.v0 = (2 * bx0) / 16;
-    ref.v1 = ceil_div (2 * bx1, 16);
-    ref.y0 = by0;
-    ref.y1 = by1;
-    ref.pitch = (ref.v1 - ref.v0) * 16;
-    ref.ga = 255;
-    const size_t bytes = (size_t) ref.pitch * (by1 - by0);
-    uint8_t *a, *uv;
-    int rc;
-    if ((rc = dev_alloc (c, blocks, bytes, &a)) || (rc = dev_alloc (c, blocks, bytes, &uv)))
-      return rc;
-    pp.mode = (format == FLUC_TTMLBLEND_FORMAT_NV21 || format == FLUC_TTMLBLEND_FORMAT_NV61) ?
+    /* alpha pairs and interleaved U,V: two bytes per sample */
+    const int mode = (format == FLUC_TTMLBLEND_FORMAT_NV21 || format == FLUC_TTMLBLEND_FORMAT_NV61) ?
         PM_CHROMA_VU : PM_CHROMA_UV;
-    pp.out_a = a; pp.out_c = uv; pp.out_c2 = nullptr;
-    pp.out_pitch = ref.pitch;
-    pp.v0 = ref.v0;
-    pp.row0 = by0;
-    pp.rows = by1 - by0;
-    if ((rc = issue_prepare (c, pp, ref.pitch / 2, batch)))
+    if ((rc = prepare_planes (c, pp, mode, 2 * bx0, 2 * bx1, by0, by1, 2, 2, blocks, batch, ref, planes)))
       return rc;
-    ref.a = a;
-    ref.c = uv;
     out.refs[out.n_refs++] = { 1, ref };
   }
   return 0;
@@ -242,13 +226,36 @@ prepare_avg_chroma (Ctx *c, PrepareParams pp, int format, int ga, PreparedRect &
   return prepare_chroma (c, pp, format, true, &out.avg_blocks, out, nullptr);
 }
 
+/* the prepare mode of a format's first plane group: luma, the packed 4:2:2 / 3-byte 4:4:4
+ * bytes, or the pixel words */
+static int
+first_mode (int format)
+{
+  switch (format) {
+    case FLUC_TTMLBLEND_FORMAT_YUY2: return PM_YUY2;
+    case FLUC_TTMLBLEND_FORMAT_UYVY: return PM_UYVY;
+    case FLUC_TTMLBLEND_FORMAT_YVYU: return PM_YVYU;
+    case FLUC_TTMLBLEND_FORMAT_VYUY: return PM_VYUY;
+    case FLUC_TTMLBLEND_FORMAT_v308: return PM_V308;
+    case FLUC_TTMLBLEND_FORMAT_IYU2: return PM_IYU2;
+    case FLUC_TTMLBLEND_FORMAT_RGB: return PM_RGB24;
+    case FLUC_TTMLBLEND_FORMAT_BGR: return PM_BGR24;
+    case FLUC_TTMLBLEND_FORMAT_AYUV: return PM_PACKED_AYUV;
+    case FLUC_TTMLBLEND_FORMAT_ARGB: return PM_PACKED_ARGB;
+    case FLUC_TTMLBLEND_FORMAT_ABGR: return PM_PACKED_ABGR;
+    case FLUC_TTMLBLEND_FORMAT_RGBA: return PM_PACKED_RGBA;
+    case FLUC_TTMLBLEND_FORMAT_BGRA: return PM_PACKED_BGRA;
+    default: return PM_LUMA;
+  }
+}
+
 /* Prepares one rectangle for one destination format: allocates its planes, runs the prepare
  * kernel(s) on the upload stream (or adds them to `batch`, issue_prepare), and notes how each
  * destination plane sees it. ga_now is the current global alpha of its box, which only averaged
  * chroma folds in. */
 static int
 prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_average, int ga_now,
-    PreparedRect &out, std::vector<PrepareItem> *batch = nullptr)
+    PreparedRect &out, std::vector<PrepareItem> *batch)
 {
   const int kind = plane_kind (format);
   PrepareParams pp;
@@ -256,129 +263,50 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
     return 0;
   if (rr.ga == 0)
     return 0;                 /* asrc == 0 everywhere: blends nothing */
-  const int cx0 = pp.cx0, cy0 = pp.cy0, cx1 = pp.cx1, cy1 = pp.cy1;
-
-  if (kind == PK_PLANE8 && format_packed_422 (format)) {
+  const int cx0 = pp.cx0, cx1 = pp.cx1;
+  /* the first plane group's byte columns: a luma plane (byte == pixel), alpha + colour planes */
+  int b0 = cx0, b1 = cx1, n_planes = 2, elem_bytes = 1;
+  if (format_packed_422 (format)) {
     /* YUY2 / UYVY: one plane of macropixels, every byte gets its own alpha + colour */
-    RectRef ref = {};
-    ref.v0 = (4 * (cx0 / 2)) / 16;
-    ref.v1 = ceil_div (4 * ceil_div (cx1, 2), 16);
-    ref.y0 = cy0;
-    ref.y1 = cy1;
-    ref.pitch = (ref.v1 - ref.v0) * 16;
-    ref.ga = 255;
-    const size_t bytes = (size_t) ref.pitch * (cy1 - cy0);
-    uint8_t *a, *col;
-    int rc;
-    if ((rc = dev_alloc (c, &out.blocks, bytes, &a)) || (rc = dev_alloc (c, &out.blocks, bytes, &col)))
-      return rc;
-    ref.a = a;
-    ref.c = col;
-    pp.mode = format == FLUC_TTMLBLEND_FORMAT_YUY2 ? PM_YUY2 : format == FLUC_TTMLBLEND_FORMAT_UYVY ? PM_UYVY :
-        format == FLUC_TTMLBLEND_FORMAT_YVYU ? PM_YVYU : PM_VYUY;
-    pp.out_a = a; pp.out_c = col; pp.out_c2 = nullptr;
-    pp.out_pitch = ref.pitch;
-    pp.v0 = ref.v0;
-    pp.row0 = cy0;
-    pp.rows = cy1 - cy0;
-    if ((rc = issue_prepare (c, pp, ref.pitch / 4, batch)))
-      return rc;
-    out.refs[out.n_refs++] = { 0, ref };
-  } else if (kind == PK_PLANE8_RGB || (kind == PK_PLANE8 && format_packed_444_3 (format))) {
-    /* v308 / IYU2 / RGB / BGR: one plane, three bytes per pixel, every byte its own alpha +
-     * colour; the RGB pair keeps the source colours and the rectangle's flags for the blend */
-    RectRef ref = {};
-    ref.v0 = (3 * cx0) / 16;
-    ref.v1 = ceil_div (3 * cx1, 16);
-    ref.y0 = cy0;
-    ref.y1 = cy1;
-    ref.pitch = (ref.v1 - ref.v0) * 16;
-    ref.ga = 255;
-    const size_t bytes = (size_t) ref.pitch * (cy1 - cy0);
-    uint8_t *a, *col;
-    int rc;
-    if ((rc = dev_alloc (c, &out.blocks, bytes, &a)) || (rc = dev_alloc (c, &out.blocks, bytes, &col)))
-      return rc;
-    ref.a = a;
-    ref.c = col;
-    if (kind == PK_PLANE8_RGB) {
-      ref.ga = rr.ga;
-      ref.src_premul = rr.premul ? 1 : 0;
-    }
-    pp.mode = format == FLUC_TTMLBLEND_FORMAT_v308 ? PM_V308 : format == FLUC_TTMLBLEND_FORMAT_IYU2 ? PM_IYU2 :
-        format == FLUC_TTMLBLEND_FORMAT_RGB ? PM_RGB24 : PM_BGR24;
-    pp.out_a = a; pp.out_c = col; pp.out_c2 = nullptr;
-    pp.out_pitch = ref.pitch;
-    pp.v0 = ref.v0;
-    pp.row0 = cy0;
-    pp.rows = cy1 - cy0;
-    if ((rc = issue_prepare (c, pp, ref.pitch, batch)))
-      return rc;
-    out.refs[out.n_refs++] = { 0, ref };
-  } else if (kind == PK_PLANE8) {
-    /* luma plane: byte == pixel */
-    {
-      RectRef ref = {};
-      ref.v0 = cx0 / 16;
-      ref.v1 = ceil_div (cx1, 16);
-      ref.y0 = cy0;
-      ref.y1 = cy1;
-      ref.pitch = (ref.v1 - ref.v0) * 16;
-      ref.ga = 255;
-      const size_t bytes = (size_t) ref.pitch * (cy1 - cy0);
-      uint8_t *a, *y;
-      int rc;
-      if ((rc = dev_alloc (c, &out.blocks, bytes, &a)) || (rc = dev_alloc (c, &out.blocks, bytes, &y)))
-        return rc;
-      ref.a = a;
-      ref.c = y;
-      pp.mode = PM_LUMA;
-      pp.out_a = a; pp.out_c = y; pp.out_c2 = nullptr;
-      pp.out_pitch = ref.pitch;
-      pp.v0 = ref.v0;
-      pp.row0 = cy0;
-      pp.rows = cy1 - cy0;
-      if ((rc = issue_prepare (c, pp, ref.pitch, batch)))
-        return rc;
-      out.refs[out.n_refs++] = { 0, ref };
-    }
-    if (chroma_average && pp.sub_x == 2 && pp.sub_y == 2)
-      return prepare_avg_chroma (c, pp, format, ga_now, out);
-    return prepare_chroma (c, pp, format, false, &out.blocks, out, batch);
-  } else {
-    RectRef ref = {};
-    ref.v0 = cx0 / 4;
-    ref.v1 = ceil_div (cx1, 4);
-    ref.y0 = cy0;
-    ref.y1 = cy1;
-    ref.pitch = (ref.v1 - ref.v0) * 16;
-    ref.ga = rr.ga;
-    const bool yuv = format == FLUC_TTMLBLEND_FORMAT_AYUV;
-    ref.src_premul = (!yuv && rr.premul) ? 1 : 0;
-    const size_t bytes = (size_t) ref.pitch * (cy1 - cy0);
-    uint8_t *w;
-    int rc;
-    if ((rc = dev_alloc (c, &out.blocks, bytes, &w)))
-      return rc;
-    switch (format) {
-      case FLUC_TTMLBLEND_FORMAT_AYUV: pp.mode = PM_PACKED_AYUV; break;
-      case FLUC_TTMLBLEND_FORMAT_ARGB: pp.mode = PM_PACKED_ARGB; break;
-      case FLUC_TTMLBLEND_FORMAT_ABGR: pp.mode = PM_PACKED_ABGR; break;
-      case FLUC_TTMLBLEND_FORMAT_RGBA: pp.mode = PM_PACKED_RGBA; break;
-      default: pp.mode = PM_PACKED_BGRA; break;
-    }
-    pp.out_a = w; pp.out_c = nullptr; pp.out_c2 = nullptr;
-    pp.out_pitch = ref.pitch;
-    pp.v0 = ref.v0;
-    pp.row0 = cy0;
-    pp.rows = cy1 - cy0;
-    if ((rc = issue_prepare (c, pp, ref.pitch / 4, batch)))
-      return rc;
-    ref.a = w;
-    ref.c = nullptr;
-    out.refs[out.n_refs++] = { 0, ref };
+    b0 = 4 * (cx0 / 2);
+    b1 = 4 * ceil_div (cx1, 2);
+    elem_bytes = 4;
+  } else if (kind == PK_PLANE8_RGB || format_packed_444_3 (format)) {
+    /* v308 / IYU2 / RGB / BGR: one plane, three bytes per pixel, every byte its own alpha + colour */
+    b0 = 3 * cx0;
+    b1 = 3 * cx1;
+  } else if (kind != PK_PLANE8) {
+    /* one plane of pixel words */
+    b0 = 4 * cx0;
+    b1 = 4 * cx1;
+    n_planes = 1;
+    elem_bytes = 4;
   }
-  return 0;
+  RectRef ref;
+  uint8_t *planes[3];
+  const int rc = prepare_planes (c, pp, first_mode (format), b0, b1, pp.cy0, pp.cy1, n_planes, elem_bytes,
+      &out.blocks, batch, ref, planes);
+  if (rc)
+    return rc;
+  if (kind != PK_PLANE8) {
+    /* the RGB pair and the pixel words keep the source colours and the rectangle's flags for the
+     * blend (AYUV's colours are converted, so premultiplied ones are not) */
+    ref.ga = rr.ga;
+    ref.src_premul = (format != FLUC_TTMLBLEND_FORMAT_AYUV && rr.premul) ? 1 : 0;
+  }
+  out.refs[out.n_refs++] = { 0, ref };
+  if (chroma_average && pp.sub_x == 2 && pp.sub_y == 2)
+    return prepare_avg_chroma (c, pp, format, ga_now, out);
+  return prepare_chroma (c, pp, format, false, &out.blocks, out, batch);
+}
+
+/* the PLANE8 kinds fold a rectangle's global alpha into its prepared alpha bytes; the packed kinds
+ * give it to the blend */
+static bool
+folds_ga (int format)
+{
+  const int kind = plane_kind (format);
+  return kind == PK_PLANE8 || kind == PK_PLANE8_RGB;
 }
 
 /* The rectangle tables of P with every box's current global alpha: a box at 0 drops out (no
@@ -388,12 +316,12 @@ prepare_rect (Ctx *c, const RawRect &rr, int format, int W, int H, bool chroma_a
  * (overlay_set_positions) goes out here as one launch; when its items do not fit in the kernel
  * parameters they are uploaded in the tables' allocation, behind them. */
 static int
-prepare_assemble (Ctx *c, Prepared *P, const Overlay *ov, std::vector<PrepareItem> *batch = nullptr)
+prepare_assemble (Ctx *c, Prepared *P, const Overlay *ov, std::vector<PrepareItem> *batch)
 {
   for (int pl = 0; pl < 3; pl++)
     P->h_rects[pl].clear ();
   const int kind = plane_kind (P->format);
-  const bool planes = kind == PK_PLANE8 || kind == PK_PLANE8_RGB;
+  const bool planes = folds_ga (P->format);
   P->fade = false;
   for (const OverlayBox &b : ov->boxes)
     for (uint32_t i = b.first_rect; i < b.first_rect + b.n_rects; i++) {
@@ -486,21 +414,86 @@ declared_px (const Overlay *ov, int W, int H)
   return px;
 }
 
-static int
-prepare_build (Ctx *c, Overlay *ov, int format, int W, int H, std::unique_ptr<Prepared> &P)
+/* Can rectangle `now` use the planes prepared from `was`: equal in everything rect_params and
+ * prepare_rect read. The global alpha counts where the prepare folds it in (folds_ga); for the
+ * packed kinds only whether it is 0 (nothing prepared). */
+static bool
+same_prepare (const RawRect &now, const RawRect &was, bool folded)
 {
+  return now.dev == was.dev && now.pitch == was.pitch && now.w == was.w && now.h == was.h && now.x == was.x &&
+      now.y == was.y && now.premul == was.premul && (folded ? now.ga == was.ga : (now.ga == 0) == (was.ga == 0));
+}
+
+/* Builds the Prepared of nv for (format, W, H, chroma_average) and adds it to nv->prepared. For a
+ * new generation of an overlay (overlay_update, a fade, a move), `old` is the Prepared of the
+ * previous generation `prev` for the same four, and from_old[i] the rectangle of prev that
+ * rectangle i of nv comes from (-1: none). A rectangle keeps the planes of the one it comes from when the two
+ * are the same for the prepare (same_prepare), and its averaged chroma as well when that was
+ * prepared at its box's current global alpha; otherwise only the averaged chroma is prepared again
+ * at the new value. Every other rectangle is prepared from its raw pixels: with `batched`
+ * (overlay_set_positions) in one batch launch. */
+static int
+build_prepared (Ctx *c, Overlay *nv, int format, int W, int H, bool chroma_average, const Overlay *prev = nullptr,
+    const Prepared *old = nullptr, const std::vector<int> *from_old = nullptr, bool batched = false)
+{
+  std::unique_ptr<Prepared> P (new Prepared ());
   P->format = format;
   P->W = W;
   P->H = H;
-  P->chroma_average = c->chroma_average;
-  P->overlay_px = declared_px (ov, W, H);
-  P->per_rect.resize (ov->rects.size ());
-  for (size_t i = 0; i < ov->rects.size (); i++) {
-    const int rc = prepare_rect (c, ov->rects[i], format, W, H, P->chroma_average, box_ga (ov, i), P->per_rect[i]);
+  P->chroma_average = chroma_average;
+  P->overlay_px = declared_px (nv, W, H);
+  P->used = old ? old->used : false;
+  P->per_rect.resize (nv->rects.size ());
+  const bool folded = folds_ga (format);
+  std::vector<PrepareItem> items;
+  std::vector<PrepareItem> *batch = batched ? &items : nullptr;
+  for (size_t i = 0; i < nv->rects.size (); i++) {
+    const RawRect &rr = nv->rects[i];
+    const int j = old ? (*from_old)[i] : -1;
+    const PreparedRect *was = j >= 0 ? &old->per_rect[(size_t) j] : nullptr;
+    const int ga = box_ga (nv, i);
+    PreparedRect &pr = P->per_rect[i];
+    PrepareParams pp;
+    int rc = 0;
+    if (!was || !same_prepare (rr, prev->rects[(size_t) j], folded)) {
+      rc = prepare_rect (c, rr, format, W, H, chroma_average, ga, pr, batch);
+    } else if (was->avg_ga >= 0 && was->avg_ga != ga && rect_params (rr, format, W, H, pp)) {
+      /* the luma planes as they were, the averaged chroma at the new value */
+      pr.blocks = was->blocks;
+      for (int k = 0; k < was->n_refs; k++)
+        if (was->refs[k].plane == 0)
+          pr.refs[pr.n_refs++] = was->refs[k];
+      rc = prepare_avg_chroma (c, pp, format, ga, pr);
+    } else {
+      pr = *was;
+    }
     if (rc)
       return rc;
   }
-  return prepare_assemble (c, P.get (), ov);
+  const int rc = prepare_assemble (c, P.get (), nv, batch);
+  if (rc)
+    return rc;
+  nv->prepared.push_back (std::move (P));
+  return 0;
+}
+
+int
+prepare_overlay (Ctx *c, Overlay *ov, int format, int W, int H, Prepared **out)
+{
+  for (auto &p : ov->prepared)
+    if (p->format == format && p->W == W && p->H == H && p->chroma_average == c->chroma_average) {
+      *out = p.get ();
+      return 0;
+    }
+
+  NvtxRange nvtx ("ttmlblend.prepare_overlay");
+  TBLOG (2, "prepare overlay: format %d, %dx%d, %zu rectangle(s)", format, W, H, ov->rects.size ());
+  /* a half-built one (out of memory, too many rectangles) goes back with its blocks */
+  const int rc = build_prepared (c, ov, format, W, H, c->chroma_average);
+  if (rc)
+    return rc;
+  *out = ov->prepared.back ().get ();
+  return 0;
 }
 
 
@@ -587,15 +580,6 @@ crop_runs (const std::vector<int2> &spans, int min_gap, size_t max_runs, std::ve
     out.push_back ({ r.x0, r.y0, r.x1 - r.x0, r.y1 - r.y0 });
 }
 
-static std::shared_ptr<DevBlock>
-make_block (Ctx *c, void *ptr)
-{
-  std::shared_ptr<DevBlock> b (new DevBlock ());
-  b->ctx = c;
-  b->ptr = ptr;
-  return b;
-}
-
 /* A rectangle whose pixels already sit in device memory, on its way into an overlay. */
 struct Up {
   RawRect rr;
@@ -656,6 +640,35 @@ scan_rows (Ctx *c, std::unique_lock<std::mutex> &lk, Up &u)
   CUU (c, lk, cudaMemcpyAsync (u.raw.data (), sp, nb, cudaMemcpyDeviceToHost, c->up_stream));   /* one copy for both */
   CUU (c, lk, cudaFreeAsync (sp, c->up_stream));
   return 0;
+}
+
+/* Queues the upload of rr.w x rr.h BGRA pixels from `src` into a block of rr's own on the upload
+ * stream. cudaMemcpyDefault: the pixels may just as well be in device memory already (UVA tells);
+ * host pixels count into st.h2d_bytes. */
+static int
+upload_rect (Ctx *c, std::unique_lock<std::mutex> &lk, const uint8_t *src, int stride, RawRect &rr, InstallStats &st)
+{
+  rr.pitch = (int) align_up ((size_t) rr.w * 4, 256);
+  void *d = nullptr;
+  CUU (c, lk, cudaMallocFromPoolAsync (&d, (size_t) rr.pitch * rr.h, c->mem_pool, c->up_stream));
+  rr.block = make_block (c, d);
+  rr.dev = static_cast<uint8_t *> (d);
+  CUU (c, lk, cudaMemcpy2DAsync (rr.dev, rr.pitch, src, stride, (size_t) rr.w * 4, rr.h, cudaMemcpyDefault,
+          c->up_stream));
+  if (!on_device (src))
+    st.h2d_bytes += (uint64_t) rr.w * 4 * rr.h;
+  return 0;
+}
+
+/* Waits for what the install queued on the upload stream while unlocked -- the caller's pixels
+ * must be consumed and the row spans back before it returns -- and takes the context lock back. */
+static int
+wait_uploads (Ctx *c, std::unique_lock<std::mutex> &lk)
+{
+  CUU (c, lk, cudaStreamSynchronize (c->up_stream));
+  if (!lk.owns_lock ())
+    lk.lock ();
+  return c->sticky;
 }
 
 /* after the upload stream has been waited for: the scan's two arrays apart */
@@ -742,13 +755,9 @@ static int
 finish_install (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, std::shared_ptr<Overlay> ov,
     std::vector<Up> &ups, const InstallStats &st)
 {
-  /* the caller's pixels must be consumed (and the row spans back) before we return; the
-   * context stays unlocked while that takes its time */
-  CUU (c, lk, cudaStreamSynchronize (c->up_stream));
-  if (!lk.owns_lock ())
-    lk.lock ();
-  if (c->sticky)
-    return c->sticky;
+  int rc = wait_uploads (c, lk);
+  if (rc)
+    return rc;
   c->stats.h2d_bytes += st.h2d_bytes;
   c->stats.prepare_launches += st.launches;
   for (Up &u : ups)
@@ -765,8 +774,7 @@ finish_install (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, std::
       if (!p->used || p->chroma_average != c->chroma_average)
         continue;
       Prepared *unused = nullptr;
-      const int rc = prepare_overlay (c, ov.get (), p->format, p->W, p->H, &unused);
-      if (rc)
+      if ((rc = prepare_overlay (c, ov.get (), p->format, p->W, p->H, &unused)))
         return rc;
     }
   }
@@ -866,17 +874,10 @@ overlay_install (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, cons
     rr.ga = std::max (0, std::min (255, rr.ga));
     rr.premul = (r.flags & FLUC_TTMLBLEND_FLAG_PREMULTIPLIED_ALPHA) != 0;
     ov->declared.push_back ({ rr.x, rr.y, rr.w, rr.h });
+    int rc;
     if (!scaled) {
-      rr.pitch = (int) align_up ((size_t) rr.w * 4, 256);
-      void *d = nullptr;
-      CUU (c, lk, cudaMallocFromPoolAsync (&d, (size_t) rr.pitch * rr.h, c->mem_pool, c->up_stream));
-      rr.block = make_block (c, d);
-      rr.dev = static_cast<uint8_t *> (d);
-      /* cudaMemcpyDefault: the pixels may just as well be in device memory already (UVA tells) */
-      CUU (c, lk, cudaMemcpy2DAsync (rr.dev, rr.pitch, r.pixels + (size_t) yoff * r.stride + (size_t) xoff * 4,
-              r.stride, (size_t) rr.w * 4, rr.h, cudaMemcpyDefault, c->up_stream));
-      if (!on_device (r.pixels))
-        st.h2d_bytes += (uint64_t) rr.w * 4 * rr.h;
+      if ((rc = upload_rect (c, lk, r.pixels + (size_t) yoff * r.stride + (size_t) xoff * 4, r.stride, rr, st)))
+        return rc;
     } else {
       /* the whole source goes up, is scaled to the render size on the GPU, and the clipped
        * part of the scaled image is what gets blended */
@@ -902,8 +903,7 @@ overlay_install (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, cons
       CUU (c, lk, cudaFreeAsync (p, c->up_stream));
       rr.dev = static_cast<uint8_t *> (d) + (size_t) yoff * rr.pitch + (size_t) xoff * 4;
     }
-    int rc = scan_rows (c, lk, u);
-    if (rc)
+    if ((rc = scan_rows (c, lk, u)))
       return rc;
     ups.push_back (std::move (u));
   }
@@ -966,24 +966,14 @@ overlay_update_image (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream,
     rr.x = d.x; rr.y = d.y; rr.w = d.w; rr.h = d.h;
     rr.ga = 255;
     rr.premul = true;
-    rr.pitch = (int) align_up ((size_t) rr.w * 4, 256);
-    void *dev = nullptr;
-    CUU (c, lk, cudaMallocFromPoolAsync (&dev, (size_t) rr.pitch * rr.h, c->mem_pool, c->up_stream));
-    rr.block = make_block (c, dev);
-    rr.dev = static_cast<uint8_t *> (dev);
-    CUU (c, lk, cudaMemcpy2DAsync (rr.dev, rr.pitch, bgra + (size_t) d.y * stride + (size_t) d.x * 4, stride,
-            (size_t) rr.w * 4, rr.h, cudaMemcpyDefault, c->up_stream));
-    if (!on_device (bgra))
-      st.h2d_bytes += (uint64_t) rr.w * 4 * rr.h;
-    int rc = scan_rows (c, lk, ups[b]);
-    if (rc)
+    int rc;
+    if ((rc = upload_rect (c, lk, bgra + (size_t) d.y * stride + (size_t) d.x * 4, stride, rr, st)) ||
+        (rc = scan_rows (c, lk, ups[b])))
       return rc;
   }
-  CUU (c, lk, cudaStreamSynchronize (c->up_stream));
-  if (!lk.owns_lock ())
-    lk.lock ();
-  if (c->sticky)
-    return c->sticky;
+  int rc = wait_uploads (c, lk);
+  if (rc)
+    return rc;
   auto now = c->overlays.find (stream);
   if (now == c->overlays.end () || now->second != old)
     return FLUC_TTMLBLEND_ERROR_NOT_FOUND;      /* replaced meanwhile by another thread */
@@ -1023,36 +1013,50 @@ overlay_update_image (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream,
   /* prepared for the formats / sizes the stream's frames have been using: kept rectangles bring
    * their prepared planes along, the others are prepared now */
   for (auto &p : old->prepared) {
-    if (!p->used || p->chroma_average != c->chroma_average || p->per_rect.size () != old->rects.size ())
+    if (!p->used || p->chroma_average != c->chroma_average)
       continue;
-    std::unique_ptr<Prepared> P (new Prepared ());
-    P->format = p->format;
-    P->W = p->W;
-    P->H = p->H;
-    P->chroma_average = p->chroma_average;
-    P->overlay_px = p->overlay_px;
-    P->used = true;
-    P->per_rect.resize (nv->rects.size ());
-    int rc = 0;
-    for (size_t i = 0; i < nv->rects.size () && !rc; i++) {
-      if (from_old[i] >= 0)
-        P->per_rect[i] = p->per_rect[(size_t) from_old[i]];
-      else
-        rc = prepare_rect (c, nv->rects[i], P->format, P->W, P->H, P->chroma_average, box_ga (nv.get (), i),
-            P->per_rect[i]);
-    }
-    if (!rc)
-      rc = prepare_assemble (c, P.get (), nv.get ());
-    if (rc) {
-      if (P->ready)
-        cudaEventDestroy (P->ready);
+    if ((rc = build_prepared (c, nv.get (), p->format, p->W, p->H, p->chroma_average, old.get (), p.get (),
+             &from_old)))
       return rc;
-    }
-    nv->prepared.push_back (std::move (P));
   }
   c->overlays[stream] = nv;       /* frames already queued keep the old one */
   c->stats.overlays_set++;
   c->stats.overlays_updated++;
+  return 0;
+}
+
+/* A new generation of ov: the same rectangles, boxes and form, nothing prepared yet. */
+static std::shared_ptr<Overlay>
+next_generation (const Overlay *ov)
+{
+  std::shared_ptr<Overlay> nv (new Overlay ());
+  nv->ctx = ov->ctx;
+  nv->rects = ov->rects;
+  nv->boxes = ov->boxes;
+  nv->declared = ov->declared;
+  nv->image_w = ov->image_w;
+  nv->image_h = ov->image_h;
+  nv->updatable = ov->updatable;
+  nv->movable = ov->movable;
+  nv->n_alphas = ov->n_alphas;
+  return nv;
+}
+
+/* Prepares nv, a new generation of the stream's overlay `old` with its rectangles in the same
+ * order, for everything old was prepared for (build_prepared), and swaps it in. */
+static int
+install_generation (Ctx *c, uint32_t stream, const Overlay *old, const std::shared_ptr<Overlay> &nv, bool batched)
+{
+  decide_lazy (nv.get ());
+  std::vector<int> same (nv->rects.size ());
+  std::iota (same.begin (), same.end (), 0);
+  for (auto &p : old->prepared) {
+    const int rc = build_prepared (c, nv.get (), p->format, p->W, p->H, p->chroma_average, old, p.get (), &same,
+        batched);
+    if (rc)
+      return rc;
+  }
+  c->overlays[stream] = nv;       /* frames already queued keep the old one */
   return 0;
 }
 
@@ -1075,17 +1079,7 @@ overlay_set_alpha (Ctx *c, uint32_t stream, const int *ga, uint32_t n)
   const std::shared_ptr<Overlay> old = it->second;
   if (n != 1 && n != old->n_alphas)
     return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
-  std::shared_ptr<Overlay> nv (new Overlay ());
-  nv->ctx = c;
-  nv->rects = old->rects;
-  nv->boxes = old->boxes;
-  nv->declared = old->declared;
-  nv->image_w = old->image_w;
-  nv->image_h = old->image_h;
-  nv->updatable = old->updatable;
-  nv->movable = old->movable;
-  nv->n_alphas = old->n_alphas;
-  std::vector<bool> again (nv->rects.size (), false);   /* prepared once more, without a global alpha */
+  std::shared_ptr<Overlay> nv = next_generation (old.get ());
   bool changed = false;
   for (OverlayBox &b : nv->boxes) {
     const int v = ga[n == 1 ? 0 : b.slot];
@@ -1094,56 +1088,11 @@ overlay_set_alpha (Ctx *c, uint32_t stream, const int *ga, uint32_t n)
     changed = true;
     b.ga = v;
     for (uint32_t i = b.first_rect; i < b.first_rect + b.n_rects; i++)
-      if (nv->rects[i].ga != 255) {
-        again[i] = true;
-        nv->rects[i].ga = 255;
-      }
+      nv->rects[i].ga = 255;    /* from now on the blend applies it */
   }
   if (!changed)
     return 0;
-  decide_lazy (nv.get ());
-  for (auto &p : old->prepared) {
-    const int kind = plane_kind (p->format);
-    const bool planes = kind == PK_PLANE8 || kind == PK_PLANE8_RGB;
-    std::unique_ptr<Prepared> P (new Prepared ());
-    P->format = p->format;
-    P->W = p->W;
-    P->H = p->H;
-    P->chroma_average = p->chroma_average;
-    P->overlay_px = p->overlay_px;
-    P->used = p->used;
-    P->per_rect.resize (nv->rects.size ());
-    int rc = 0;
-    for (size_t i = 0; i < nv->rects.size () && !rc; i++) {
-      const PreparedRect &was = p->per_rect[i];
-      const int v = box_ga (nv.get (), i);
-      PrepareParams pp;
-      /* the packed kinds never fold the global alpha in; a rectangle installed at 0 was not prepared */
-      if (again[i] && (planes || old->rects[i].ga == 0)) {
-        rc = prepare_rect (c, nv->rects[i], P->format, P->W, P->H, P->chroma_average, v, P->per_rect[i]);
-      } else if (was.avg_ga >= 0 && was.avg_ga != v && rect_params (nv->rects[i], P->format, P->W, P->H, pp)) {
-        /* the luma planes as they were, the averaged chroma at the new value */
-        PreparedRect &pr = P->per_rect[i];
-        pr.blocks = was.blocks;
-        for (int k = 0; k < was.n_refs; k++)
-          if (was.refs[k].plane == 0)
-            pr.refs[pr.n_refs++] = was.refs[k];
-        rc = prepare_avg_chroma (c, pp, P->format, v, pr);
-      } else {
-        P->per_rect[i] = was;
-      }
-    }
-    if (!rc)
-      rc = prepare_assemble (c, P.get (), nv.get ());
-    if (rc) {
-      if (P->ready)
-        cudaEventDestroy (P->ready);
-      return rc;
-    }
-    nv->prepared.push_back (std::move (P));
-  }
-  c->overlays[stream] = nv;       /* frames already queued keep the old one */
-  return 0;
+  return install_generation (c, stream, old.get (), nv, false);
 }
 
 /* overlay_set_positions: a new generation of the stream's overlay whose boxes sit at (x[i], y[i])
@@ -1167,17 +1116,7 @@ overlay_set_positions (Ctx *c, uint32_t stream, const int32_t *x, const int32_t 
   for (const OverlayBox &b : old->boxes)
     if ((int64_t) x[b.slot] + b.declared.w > INT32_MAX || (int64_t) y[b.slot] + b.declared.h > INT32_MAX)
       return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
-  std::shared_ptr<Overlay> nv (new Overlay ());
-  nv->ctx = c;
-  nv->rects = old->rects;
-  nv->boxes = old->boxes;
-  nv->declared = old->declared;
-  nv->image_w = old->image_w;
-  nv->image_h = old->image_h;
-  nv->updatable = old->updatable;
-  nv->movable = old->movable;
-  nv->n_alphas = old->n_alphas;
-  std::vector<bool> moved (nv->rects.size (), false);
+  std::shared_ptr<Overlay> nv = next_generation (old.get ());
   bool changed = false;
   for (OverlayBox &b : nv->boxes) {
     const int bx = x[b.slot], by = y[b.slot];
@@ -1188,7 +1127,6 @@ overlay_set_positions (Ctx *c, uint32_t stream, const int32_t *x, const int32_t 
       RawRect &rr = nv->rects[i];
       rr.x = bx + (rr.x - b.declared.x);      /* the crop run's offset inside the rectangle */
       rr.y = by + (rr.y - b.declared.y);
-      moved[i] = true;
     }
     b.declared.x = bx;
     b.declared.y = by;
@@ -1196,36 +1134,7 @@ overlay_set_positions (Ctx *c, uint32_t stream, const int32_t *x, const int32_t 
   }
   if (!changed)
     return 0;
-  decide_lazy (nv.get ());
-  for (auto &p : old->prepared) {
-    std::unique_ptr<Prepared> P (new Prepared ());
-    P->format = p->format;
-    P->W = p->W;
-    P->H = p->H;
-    P->chroma_average = p->chroma_average;
-    P->overlay_px = declared_px (nv.get (), P->W, P->H);
-    P->used = p->used;
-    P->per_rect.resize (nv->rects.size ());
-    std::vector<PrepareItem> batch;
-    int rc = 0;
-    for (size_t i = 0; i < nv->rects.size () && !rc; i++) {
-      if (moved[i])
-        rc = prepare_rect (c, nv->rects[i], P->format, P->W, P->H, P->chroma_average, box_ga (nv.get (), i),
-            P->per_rect[i], &batch);
-      else
-        P->per_rect[i] = p->per_rect[i];
-    }
-    if (!rc)
-      rc = prepare_assemble (c, P.get (), nv.get (), &batch);
-    if (rc) {
-      if (P->ready)
-        cudaEventDestroy (P->ready);
-      return rc;
-    }
-    nv->prepared.push_back (std::move (P));
-  }
-  c->overlays[stream] = nv;       /* frames already queued keep the old one */
-  return 0;
+  return install_generation (c, stream, old.get (), nv, true);
 }
 
 /* Cairo's colour conversion: double components -> premultiplied 16-bit shorts

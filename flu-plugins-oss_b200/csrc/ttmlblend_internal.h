@@ -328,6 +328,7 @@ struct Prepared {
   bool blend_waited = false;           /* blend stream already ordered after `ready` */
   bool used = false;                   /* a frame has been blended with it (worth preparing the next cue for) */
   std::vector<std::unique_ptr<Layout>> layouts;
+  ~Prepared ();                        /* destroys `ready` when set */
 };
 
 /* One rectangle as it was handed in (a region box of ttmlrender's image): the unit a cue update
