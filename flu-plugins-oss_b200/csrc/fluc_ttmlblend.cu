@@ -468,6 +468,16 @@ fluc_ttmlblend_overlay_set_positions (FlucTtmlBlend *thiz, uint32_t stream, cons
 }
 
 int
+fluc_ttmlblend_overlay_set_render_rectangles (FlucTtmlBlend *thiz, uint32_t stream, const FlucTtmlBlendRect *render,
+    uint32_t n)
+{
+  ENTER (thiz);
+  if (!render)
+    return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
+  return overlay_set_render (c, lk, stream, render, n);
+}
+
+int
 fluc_ttmlblend_set_chroma_mode (FlucTtmlBlend *thiz, int mode)
 {
   ENTER (thiz);

@@ -48,6 +48,8 @@ Overlay::~Overlay ()
   };
   for (RawRect &r : rects)
     take (r.block);
+  for (OverlayBox &b : boxes)
+    take (b.src.block);
   for (auto &p : prepared) {
     for (PreparedRect &pr : p->per_rect) {
       for (auto &b : pr.blocks)
@@ -587,6 +589,7 @@ struct Up {
   std::vector<int> groups;      /* per row: 16-pixel groups with any alpha */
   std::vector<int> raw;         /* both as they come back from the GPU in one copy: h x int2, then h x int */
   uint32_t slot = 0;            /* OverlayBox::slot */
+  BoxSource src;                /* OverlayBox::src */
 };
 
 /* Is this pointer device memory (a cue produced on the GPU, or left there by a previous stage)? */
@@ -696,6 +699,7 @@ append_box (Ctx *c, Overlay *ov, Up &u, size_t n_boxes)
   box.first_rect = (uint32_t) ov->rects.size ();
   box.ga = u.rr.ga;
   box.slot = u.slot;
+  box.src = u.src;
   if (!c->autocrop) {
     ov->rects.push_back (u.rr);
   } else {
@@ -878,6 +882,8 @@ overlay_install (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, cons
     if (!scaled) {
       if ((rc = upload_rect (c, lk, r.pixels + (size_t) yoff * r.stride + (size_t) xoff * 4, r.stride, rr, st)))
         return rc;
+      if (ov->movable)
+        u.src = { rr.block, rr.dev, rr.pitch, rr.w, rr.h, rr.premul };
     } else {
       /* the whole source goes up, is scaled to the render size on the GPU, and the clipped
        * part of the scaled image is what gets blended */
@@ -899,7 +905,11 @@ overlay_install (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, cons
       CUU (c, lk, launch_scale (static_cast<const uint8_t *> (s), sp, static_cast<const int4 *> (p), x_inc,
               static_cast<uint8_t *> (d), rr.pitch, rw, rh, c->up_stream));
       st.launches++;
-      CUU (c, lk, cudaFreeAsync (s, c->up_stream));
+      /* the composition form keeps the source for overlay_set_render_rectangles */
+      if (ov->movable)
+        u.src = { make_block (c, s), static_cast<const uint8_t *> (s), sp, r.width, r.height, rr.premul };
+      else
+        CUU (c, lk, cudaFreeAsync (s, c->up_stream));
       CUU (c, lk, cudaFreeAsync (p, c->up_stream));
       rr.dev = static_cast<uint8_t *> (d) + (size_t) yoff * rr.pitch + (size_t) xoff * 4;
     }
@@ -1042,16 +1052,22 @@ next_generation (const Overlay *ov)
   return nv;
 }
 
-/* Prepares nv, a new generation of the stream's overlay `old` with its rectangles in the same
- * order, for everything old was prepared for (build_prepared), and swaps it in. */
+/* Prepares nv, a new generation of the stream's overlay `old`, for everything old was prepared
+ * for (build_prepared), and swaps it in. from_old maps nv's rectangles to old's (nullptr: the
+ * same rectangles in the same order). */
 static int
-install_generation (Ctx *c, uint32_t stream, const Overlay *old, const std::shared_ptr<Overlay> &nv, bool batched)
+install_generation (Ctx *c, uint32_t stream, const Overlay *old, const std::shared_ptr<Overlay> &nv, bool batched,
+    const std::vector<int> *from_old = nullptr)
 {
   decide_lazy (nv.get ());
-  std::vector<int> same (nv->rects.size ());
-  std::iota (same.begin (), same.end (), 0);
+  std::vector<int> same;
+  if (!from_old) {
+    same.resize (nv->rects.size ());
+    std::iota (same.begin (), same.end (), 0);
+    from_old = &same;
+  }
   for (auto &p : old->prepared) {
-    const int rc = build_prepared (c, nv.get (), p->format, p->W, p->H, p->chroma_average, old, p.get (), &same,
+    const int rc = build_prepared (c, nv.get (), p->format, p->W, p->H, p->chroma_average, old, p.get (), from_old,
         batched);
     if (rc)
       return rc;
@@ -1135,6 +1151,181 @@ overlay_set_positions (Ctx *c, uint32_t stream, const int32_t *x, const int32_t 
   if (!changed)
     return 0;
   return install_generation (c, stream, old.get (), nv, true);
+}
+
+/* overlay_set_render_rectangles: a new generation of the stream's overlay whose boxes sit at
+ * render[i] and are render[i].w x render[i].h (box i = rectangle i of overlay_set_rectangles; a
+ * side of 0: the pixel size). A box whose size stays is moved as overlay_set_positions moves it.
+ * A resized box is built again from its resident source (BoxSource): scaled into a new block of
+ * the render size, or the source itself at its pixel size, and cropped by a fresh row scan exactly
+ * as overlay_install crops -- every resized box in one launch of the scale-and-scan kernel, one
+ * upload of the row plans and one readback of the spans, waited for with the context unlocked.
+ * Its new pixels are prepared like a box an update touches (the box keeps its global alpha, the
+ * blend applies it), with the moved boxes in one batch launch per (format, size) the old generation
+ * was prepared for. */
+int
+overlay_set_render (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, const FlucTtmlBlendRect *render,
+    uint32_t n)
+{
+  NvtxRange nvtx ("ttmlblend.overlay_set_render_rectangles");
+  auto it = c->overlays.find (stream);
+  if (it == c->overlays.end ())
+    return FLUC_TTMLBLEND_ERROR_NOT_FOUND;
+  const std::shared_ptr<Overlay> old = it->second;
+  if (!old->movable || n != old->boxes.size ())
+    return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
+  /* the limits overlay_install applies to a scaled rectangle */
+  for (const OverlayBox &b : old->boxes) {
+    const FlucTtmlBlendRect &r = render[b.slot];
+    if (r.w < 0 || r.h < 0 || r.w > 32768 || r.h > 32768)
+      return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
+    const int w = r.w ? r.w : b.src.w, h = r.h ? r.h : b.src.h;
+    if ((w != b.src.w || h != b.src.h) && (b.src.w < 2 || b.src.h < 2 || b.src.w > 32768 || b.src.h > 32768))
+      return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
+    if ((int64_t) r.x + w > INT32_MAX || (int64_t) r.y + h > INT32_MAX)
+      return FLUC_TTMLBLEND_ERROR_INVALID_ARGUMENT;
+  }
+  /* which boxes change size, which only move */
+  std::vector<Up> ups (old->boxes.size ());
+  std::vector<bool> resized (old->boxes.size (), false);
+  bool changed = false;
+  std::vector<ScaleScanItem> items;
+  std::vector<size_t> item_box;             /* box of every item */
+  std::vector<int4> plans;
+  for (size_t k = 0; k < old->boxes.size (); k++) {
+    const OverlayBox &b = old->boxes[k];
+    const FlucTtmlBlendRect &r = render[b.slot];
+    const int w = r.w ? r.w : b.src.w, h = r.h ? r.h : b.src.h;
+    changed = changed || r.x != b.declared.x || r.y != b.declared.y;
+    if (w == b.declared.w && h == b.declared.h)
+      continue;
+    changed = true;
+    resized[k] = true;
+    RawRect &rr = ups[k].rr;
+    rr.x = r.x; rr.y = r.y; rr.w = w; rr.h = h;
+    rr.premul = b.src.premul;
+    ScaleScanItem si = {};
+    si.w = w;
+    si.h = h;
+    if (w == b.src.w && h == b.src.h) {
+      /* back at its pixel size: the source itself, scanned */
+      rr.block = b.src.block;
+      rr.dev = const_cast<uint8_t *> (b.src.dev);
+      rr.pitch = b.src.pitch;
+      si.src = b.src.dev;
+      si.src_pitch = b.src.pitch;
+      si.plan = -1;
+      if (!c->autocrop)
+        continue;
+    } else {
+      si.src = b.src.dev;
+      si.src_pitch = b.src.pitch;
+      si.plan = (int32_t) plans.size ();
+      const std::vector<int4> p = scale_row_plan (b.src.h, h);
+      plans.insert (plans.end (), p.begin (), p.end ());
+      si.x_inc = w == 1 ? 0 : ((b.src.w - 1) << 16) / (w - 1) - 1;
+      rr.pitch = (int) align_up ((size_t) w * 4, 256);
+      si.dst_pitch = rr.pitch;
+    }
+    items.push_back (si);
+    item_box.push_back (k);
+  }
+  if (!changed)
+    return 0;                   /* nothing changed */
+
+  if (!items.empty ()) {
+    /* one allocation: the row plans and (beyond the inline limit) the items, uploaded in one
+     * copy, then the spans and group counts of every row, read back in one copy */
+    const uint32_t n_items = (uint32_t) items.size ();
+    const uint32_t rows = scale_scan_batch_plan (items.data (), n_items);
+    const size_t plan_bytes = plans.size () * sizeof (int4);
+    const size_t item_bytes = n_items > kScaleScanBatchInline ? n_items * sizeof (ScaleScanItem) : 0;
+    const size_t scan_bytes = c->autocrop ? (size_t) rows * (sizeof (int2) + sizeof (int)) : 0;
+    std::vector<uint8_t> up (plan_bytes + item_bytes);
+    std::vector<uint8_t> back (scan_bytes);
+    lk.unlock ();               /* as in overlay_update_image: this call's blocks and the upload stream only */
+    for (size_t i = 0; i < items.size (); i++) {
+      if (items[i].plan < 0)
+        continue;
+      RawRect &rr = ups[item_box[i]].rr;
+      void *d = nullptr;
+      CUU (c, lk, cudaMallocFromPoolAsync (&d, (size_t) rr.pitch * rr.h, c->mem_pool, c->up_stream));
+      rr.block = make_block (c, d);
+      rr.dev = static_cast<uint8_t *> (d);
+      items[i].dst = rr.dev;
+    }
+    memcpy (up.data (), plans.data (), plan_bytes);
+    if (item_bytes)
+      memcpy (up.data () + plan_bytes, items.data (), item_bytes);
+    void *buf = nullptr;
+    CUU (c, lk, cudaMallocFromPoolAsync (&buf, std::max<size_t> (up.size () + scan_bytes, 16), c->mem_pool,
+            c->up_stream));
+    uint8_t *d = static_cast<uint8_t *> (buf);
+    if (!up.empty ())
+      CUU (c, lk, cudaMemcpyAsync (d, up.data (), up.size (), cudaMemcpyHostToDevice, c->up_stream));
+    int2 *d_spans = scan_bytes ? reinterpret_cast<int2 *> (d + up.size ()) : nullptr;
+    int *d_groups = scan_bytes ? reinterpret_cast<int *> (d_spans + rows) : nullptr;
+    CUU (c, lk, launch_scale_scan_batch (items.data (), n_items,
+            reinterpret_cast<const ScaleScanItem *> (d + plan_bytes), reinterpret_cast<const int4 *> (d), d_spans,
+            d_groups, rows, c->up_stream));
+    if (scan_bytes)
+      CUU (c, lk, cudaMemcpyAsync (back.data (), d_spans, scan_bytes, cudaMemcpyDeviceToHost, c->up_stream));
+    CUU (c, lk, cudaFreeAsync (buf, c->up_stream));
+    int rc = wait_uploads (c, lk);
+    if (rc)
+      return rc;
+    c->stats.prepare_launches++;
+    if (scan_bytes) {
+      const int2 *spans = reinterpret_cast<const int2 *> (back.data ());
+      const int *groups = reinterpret_cast<const int *> (spans + rows);
+      for (size_t i = 0; i < items.size (); i++) {
+        Up &u = ups[item_box[i]];
+        u.spans.assign (spans + items[i].row0, spans + items[i].row0 + items[i].h);
+        u.groups.assign (groups + items[i].row0, groups + items[i].row0 + items[i].h);
+      }
+    }
+    auto now = c->overlays.find (stream);
+    if (now == c->overlays.end () || now->second != old)
+      return FLUC_TTMLBLEND_ERROR_NOT_FOUND;    /* replaced meanwhile by another thread */
+  }
+
+  std::shared_ptr<Overlay> nv = next_generation (old.get ());
+  nv->rects.clear ();
+  nv->boxes.clear ();
+  std::vector<int> from_old;    /* new rectangle -> the old overlay's rectangle it is, or -1 */
+  for (size_t k = 0; k < old->boxes.size (); k++) {
+    const OverlayBox &b = old->boxes[k];
+    if (resized[k]) {
+      /* new pixels, prepared without a global alpha (but averaged chroma); the box keeps its current one */
+      Up &u = ups[k];
+      u.slot = b.slot;
+      u.src = b.src;
+      u.rr.ga = b.ga;
+      append_box (c, nv.get (), u, old->boxes.size ());
+      for (uint32_t i = nv->boxes.back ().first_rect; i < nv->rects.size (); i++)
+        nv->rects[i].ga = 255;
+      from_old.resize (nv->rects.size (), -1);
+    } else {
+      /* kept, or moved: the crop runs are offsets inside the rectangle (overlay_set_positions) */
+      const FlucTtmlBlendRect &r = render[b.slot];
+      OverlayBox box = b;
+      box.first_rect = (uint32_t) nv->rects.size ();
+      box.declared.x = r.x;
+      box.declared.y = r.y;
+      for (uint32_t i = b.first_rect; i < b.first_rect + b.n_rects; i++) {
+        RawRect rr = old->rects[i];
+        rr.x = r.x + (rr.x - b.declared.x);
+        rr.y = r.y + (rr.y - b.declared.y);
+        nv->rects.push_back (rr);
+        from_old.push_back ((int) i);
+      }
+      nv->boxes.push_back (box);
+    }
+    nv->declared[b.slot] = nv->boxes.back ().declared;
+  }
+  if (nv->rects.size () > FLUC_TTMLBLEND_MAX_RECTANGLES)
+    return FLUC_TTMLBLEND_ERROR_TOO_MANY_RECTANGLES;
+  return install_generation (c, stream, old.get (), nv, true, &from_old);
 }
 
 /* Cairo's colour conversion: double components -> premultiplied 16-bit shorts

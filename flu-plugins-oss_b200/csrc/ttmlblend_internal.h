@@ -331,6 +331,16 @@ struct Prepared {
   ~Prepared ();                        /* destroys `ready` when set */
 };
 
+/* The pixels a rectangle of the composition form was installed from, whole and at their pixel
+ * size: the rectangle's raw block when it was installed unscaled, its own block otherwise.
+ * overlay_set_render_rectangles scales (or scans) them again for a new render size. */
+struct BoxSource {
+  std::shared_ptr<DevBlock> block;
+  const uint8_t *dev = nullptr;
+  int pitch = 0, w = 0, h = 0;
+  bool premul = true;
+};
+
 /* One rectangle as it was handed in (a region box of ttmlrender's image): the unit a cue update
  * keeps or replaces. */
 struct OverlayBox {
@@ -339,6 +349,7 @@ struct OverlayBox {
   uint64_t groups_all = 0, groups_on = 0, groups_opaque = 0;   /* 16-pixel groups under them: all / some alpha / alpha 255 */
   int ga = 255;                        /* its current global alpha (overlay_set_global_alpha) */
   uint32_t slot = 0;                   /* which value of overlay_set_global_alpha's list is its own */
+  BoxSource src;                       /* composition form only; declared.w / h are its render size */
 };
 
 struct Overlay {
@@ -719,6 +730,10 @@ int overlay_install_regions (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t 
 int overlay_set_alpha (Ctx *c, uint32_t stream, const int *ga, uint32_t n);
 /* x, y: one position per box (n == the number of rectangles installed); mu held throughout */
 int overlay_set_positions (Ctx *c, uint32_t stream, const int32_t *x, const int32_t *y, uint32_t n);
+/* render: one rectangle per box (n == the number of rectangles installed); entered with the
+ * context lock held (lk), drops it while it waits for the scale and scan, returns with it held */
+int overlay_set_render (Ctx *c, std::unique_lock<std::mutex> &lk, uint32_t stream, const FlucTtmlBlendRect *render,
+    uint32_t n);
 
 /* jobs.cu */
 void layout_spans (const Layout *L, std::vector<StageSpan> &out);

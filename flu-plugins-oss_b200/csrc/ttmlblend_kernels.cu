@@ -16,6 +16,7 @@
  *   ttmlblend_prepare_kernel    once per cue: unpack, un-premultiply, BT.709, siting
  *   ttmlblend_prepare_chroma_avg_kernel   opt-in, non-parity 2x2 chroma mean
  *   ttmlblend_rowspan_kernel    once per cue: non-transparent span of every row
+ *   ttmlblend_scale_scan_batch_kernel  once per resize: scale + row spans of every resized rectangle
  *   ttmlblend_blur_kernel       textOutline blur (pixman convolution semantics)
  */
 #include "ttmlblend_kernels.cuh"
@@ -1375,47 +1376,66 @@ launch_prepare_batch (const PrepareItem *items, uint32_t n, const PrepareItem *d
 /* ---------------------------------------------------------------------- */
 /* once per cue: where is the rectangle not transparent?                   */
 
-/* One CTA per row: span[y] = (first x, last x) with alpha != 0, or (w, -1); groups[y] = how
- * many of the row's 16-pixel groups hold any alpha != 0, in the low half, and how many are
- * opaque all over (alpha 255), in the high half. How sparse / how opaque the cue is decides
- * whether in-place launches look at the overlay before touching the frame. */
+/* One row's span and group figures: span = (first x, last x) with alpha != 0, or (w, -1); groups =
+ * how many of the row's 16-pixel groups hold any alpha != 0, in the low half, and how many are
+ * opaque all over (alpha 255), in the high half. Each thread of a 128-thread CTA feeds it pixels
+ * x = base + threadIdx.x for base = 0, 128, ... (every lane of a warp at once: the ballots see
+ * two 16-pixel groups per warp), 0 past the row's end; rowscan_store reduces and writes it. */
+struct RowScan {
+  int lo, hi, ng;
+};
+
+__device__ __forceinline__ void
+rowscan_px (RowScan &s, int x, uint32_t a)
+{
+  const bool on = a != 0u;
+  if (on) {
+    s.lo = min (s.lo, x);
+    s.hi = max (s.hi, x);
+  }
+  const uint32_t b = __ballot_sync (0xffffffffu, on);      /* two groups of 16 pixels per warp */
+  const uint32_t q = __ballot_sync (0xffffffffu, a == 255u);
+  s.ng += ((b & 0xffffu) ? 1 : 0) + ((b >> 16) ? 1 : 0);
+  s.ng += (((q & 0xffffu) == 0xffffu) ? 0x10000 : 0) + (((q >> 16) == 0xffffu) ? 0x10000 : 0);
+}
+
+/* every thread of the CTA calls it; thread 0 writes */
+__device__ __forceinline__ void
+rowscan_store (RowScan s, int2 *__restrict__ span, int *__restrict__ groups)
+{
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    s.lo = min (s.lo, __shfl_xor_sync (0xffffffffu, s.lo, o));
+    s.hi = max (s.hi, __shfl_xor_sync (0xffffffffu, s.hi, o));
+  }
+  __shared__ int s_lo[4], s_hi[4], s_ng[4];
+  if ((threadIdx.x & 31) == 0) {
+    s_lo[threadIdx.x >> 5] = s.lo;
+    s_hi[threadIdx.x >> 5] = s.hi;
+    s_ng[threadIdx.x >> 5] = s.ng;      /* the same in every lane of a warp */
+  }
+  __syncthreads ();
+  if (threadIdx.x == 0) {
+    *span = make_int2 (min (min (s_lo[0], s_lo[1]), min (s_lo[2], s_lo[3])),
+        max (max (s_hi[0], s_hi[1]), max (s_hi[2], s_hi[3])));
+    *groups = s_ng[0] + s_ng[1] + s_ng[2] + s_ng[3];
+  }
+}
+
+/* One CTA per row (RowScan). How sparse / how opaque the cue is decides whether in-place
+ * launches look at the overlay before touching the frame. */
 __global__ void __launch_bounds__ (128)
 ttmlblend_rowspan_kernel (const uint8_t *__restrict__ raw, int pitch, int w, int2 *__restrict__ spans,
     int *__restrict__ groups)
 {
   const int y = blockIdx.x;
   const uint32_t *row = reinterpret_cast<const uint32_t *> (raw + (size_t) y * pitch);
-  int lo = w, hi = -1, ng = 0;
+  RowScan s = { w, -1, 0 };
   for (int base = 0; base < w; base += blockDim.x) {
     const int x = base + (int) threadIdx.x;
-    const uint32_t a = x < w ? row[x] >> 24 : 0u;
-    const bool on = a != 0u;
-    if (on) {
-      lo = min (lo, x);
-      hi = max (hi, x);
-    }
-    const uint32_t b = __ballot_sync (0xffffffffu, on);      /* two groups of 16 pixels per warp */
-    const uint32_t q = __ballot_sync (0xffffffffu, a == 255u);
-    ng += ((b & 0xffffu) ? 1 : 0) + ((b >> 16) ? 1 : 0);
-    ng += (((q & 0xffffu) == 0xffffu) ? 0x10000 : 0) + (((q >> 16) == 0xffffu) ? 0x10000 : 0);
+    rowscan_px (s, x, x < w ? row[x] >> 24 : 0u);
   }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    lo = min (lo, __shfl_xor_sync (0xffffffffu, lo, o));
-    hi = max (hi, __shfl_xor_sync (0xffffffffu, hi, o));
-  }
-  __shared__ int s_lo[4], s_hi[4], s_ng[4];
-  if ((threadIdx.x & 31) == 0) {
-    s_lo[threadIdx.x >> 5] = lo;
-    s_hi[threadIdx.x >> 5] = hi;
-    s_ng[threadIdx.x >> 5] = ng;        /* the same in every lane of a warp */
-  }
-  __syncthreads ();
-  if (threadIdx.x == 0) {
-    spans[y] = make_int2 (min (min (s_lo[0], s_lo[1]), min (s_lo[2], s_lo[3])),
-        max (max (s_hi[0], s_hi[1]), max (s_hi[2], s_hi[3])));
-    groups[y] = s_ng[0] + s_ng[1] + s_ng[2] + s_ng[3];
-  }
+  rowscan_store (s, spans + y, groups + y);
 }
 
 cudaError_t
@@ -1604,14 +1624,10 @@ scale_mix_h (uint32_t a, uint32_t b, uint32_t f)
   return (lo & 0x00ff00ffu) | ((hi & 0x00ff00ffu) << 8);
 }
 
-__global__ void __launch_bounds__ (256)
-ttmlblend_scale_kernel (const uint8_t *__restrict__ src, int src_pitch, const int4 *__restrict__ rows,
-    int x_inc, uint8_t *__restrict__ dst, int dst_pitch, int dw, int dh)
+/* destination pixel x of the row whose source rows and weight are r */
+__device__ __forceinline__ uint32_t
+scale_px (const uint8_t *__restrict__ src, int src_pitch, int4 r, int x_inc, int x)
 {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
-  if (x >= dw || y >= dh)
-    return;
-  const int4 r = __ldg (&rows[y]);                /* row a, row b, weight */
   const int tmp = x * x_inc;
   const int sx = tmp >> 16;
   const uint32_t f = (uint32_t) (tmp >> 8) & 0xffu;
@@ -1625,7 +1641,18 @@ ttmlblend_scale_kernel (const uint8_t *__restrict__ src, int src_pitch, const in
     const int ca = (int) ((a >> k) & 0xffu), cb = (int) ((b >> k) & 0xffu);
     out |= (uint32_t) ((ca + (((cb - ca) * r.z + 128) >> 8)) & 0xff) << k;
   }
-  reinterpret_cast<uint32_t *> (dst + (size_t) y * dst_pitch)[x] = out;
+  return out;
+}
+
+__global__ void __launch_bounds__ (256)
+ttmlblend_scale_kernel (const uint8_t *__restrict__ src, int src_pitch, const int4 *__restrict__ rows,
+    int x_inc, uint8_t *__restrict__ dst, int dst_pitch, int dw, int dh)
+{
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
+  if (x >= dw || y >= dh)
+    return;
+  const int4 r = __ldg (&rows[y]);                /* row a, row b, weight */
+  reinterpret_cast<uint32_t *> (dst + (size_t) y * dst_pitch)[x] = scale_px (src, src_pitch, r, x_inc, x);
 }
 
 cudaError_t
@@ -1634,6 +1661,82 @@ launch_scale (const uint8_t *src, int src_pitch, const int4 *rows, int x_inc, ui
 {
   dim3 grid ((unsigned) ((dw + 255) / 256), (unsigned) dh);
   ttmlblend_scale_kernel<<<grid, 256, 0, stream>>> (src, src_pitch, rows, x_inc, dst, dst_pitch, dw, dh);
+  return cudaGetLastError ();
+}
+
+/* Every rectangle of one overlay_set_render_rectangles call in one launch: one CTA per destination
+ * row of every item, which finds its item by bisecting the items' first rows (as
+ * ttmlblend_prepare_batch_kernel does). A scaled item's CTA computes its row's pixels from the
+ * resident source, stores them and, from the same registers, reduces the row's span and group
+ * figures (RowScan) -- the scaled image is not read back for the scan. An item without a row plan
+ * only scans its source. Without spans (no auto-crop) nothing is scanned. */
+__global__ void __launch_bounds__ (128)
+ttmlblend_scale_scan_batch_kernel (const __grid_constant__ ScaleScanBatch B)
+{
+  const ScaleScanItem *items = B.items ? B.items : B.inl;
+  const uint32_t cta = blockIdx.x;
+  uint32_t lo = 0, hi = B.n_items;            /* the last item whose first row is <= cta */
+  while (hi - lo > 1) {
+    const uint32_t m = (lo + hi) / 2;
+    if (items[m].row0 <= cta)
+      lo = m;
+    else
+      hi = m;
+  }
+  const ScaleScanItem &it = items[lo];
+  const int y = (int) (cta - it.row0), w = it.w;
+  const bool scan = B.spans != nullptr;
+  RowScan s = { w, -1, 0 };
+  if (it.plan >= 0) {
+    const int4 r = __ldg (&B.plans[it.plan + y]);
+    uint32_t *out = reinterpret_cast<uint32_t *> (it.dst + (size_t) y * it.dst_pitch);
+    for (int base = 0; base < w; base += blockDim.x) {
+      const int x = base + (int) threadIdx.x;
+      uint32_t px = 0u;
+      if (x < w) {
+        px = scale_px (it.src, it.src_pitch, r, it.x_inc, x);
+        out[x] = px;
+      }
+      if (scan)
+        rowscan_px (s, x, px >> 24);
+    }
+  } else if (scan) {
+    const uint32_t *row = reinterpret_cast<const uint32_t *> (it.src + (size_t) y * it.src_pitch);
+    for (int base = 0; base < w; base += blockDim.x) {
+      const int x = base + (int) threadIdx.x;
+      rowscan_px (s, x, x < w ? row[x] >> 24 : 0u);
+    }
+  }
+  if (scan)
+    rowscan_store (s, B.spans + cta, B.groups + cta);
+}
+
+uint32_t
+scale_scan_batch_plan (ScaleScanItem *items, uint32_t n)
+{
+  uint32_t rows = 0;
+  for (uint32_t k = 0; k < n; k++) {
+    items[k].row0 = rows;
+    rows += (uint32_t) items[k].h;
+  }
+  return rows;
+}
+
+cudaError_t
+launch_scale_scan_batch (const ScaleScanItem *items, uint32_t n, const ScaleScanItem *d_items, const int4 *plans,
+    int2 *spans, int *groups, uint32_t rows, cudaStream_t stream)
+{
+  if (n == 0 || rows == 0)
+    return cudaSuccess;
+  ScaleScanBatch B;
+  B.n_items = n;
+  B.items = n > kScaleScanBatchInline ? d_items : nullptr;
+  B.plans = plans;
+  B.spans = spans;
+  B.groups = groups;
+  if (!B.items)
+    memcpy (B.inl, items, n * sizeof (ScaleScanItem));
+  ttmlblend_scale_scan_batch_kernel<<<rows, 128, 0, stream>>> (B);
   return cudaGetLastError ();
 }
 

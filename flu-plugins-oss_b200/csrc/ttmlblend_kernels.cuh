@@ -284,5 +284,39 @@ cudaError_t launch_rowspan (const uint8_t *raw, int pitch, int w, int h, int2 *s
 cudaError_t launch_scale (const uint8_t *src, int src_pitch, const int4 *rows, int x_inc, uint8_t *dst,
     int dst_pitch, int dw, int dh, cudaStream_t stream);
 
+/* One rectangle of a resize (overlay_set_render_rectangles): scaled from its resident source to
+ * w x h with the row plan at ScaleScanBatch::plans[plan ...] and x_inc as launch_scale, and its
+ * rows scanned as launch_rowspan; plan < 0: the source is already w x h and is only scanned
+ * (dst unused). Its rows are rows row0.. of the batch's spans / groups, and CTAs row0.. of the
+ * launch. */
+struct alignas (16) ScaleScanItem {
+  const uint8_t *src;
+  uint8_t *dst;
+  int32_t src_pitch, dst_pitch;
+  int32_t plan, x_inc;
+  int32_t w, h;
+  uint32_t row0;
+  uint32_t pad_;
+};
+/* items kept in the kernel parameters; more are read from device memory */
+constexpr uint32_t kScaleScanBatchInline = 32;
+struct ScaleScanBatch {
+  const ScaleScanItem *items;   /* device copy of the items, or nullptr: inl */
+  const int4 *plans;            /* the row plans of every scaled item, back to back */
+  int2 *spans;                  /* one per row of the batch; nullptr: no scan (no auto-crop) */
+  int *groups;
+  uint32_t n_items;
+  uint32_t pad_[3];
+  ScaleScanItem inl[kScaleScanBatchInline];
+};
+static_assert (sizeof (ScaleScanBatch) <= 4096, "scale-and-scan batch parameters");
+/* Fills in every item's row0 and returns the rows (= CTAs) of the batch. */
+uint32_t scale_scan_batch_plan (ScaleScanItem *items, uint32_t n);
+/* One launch of ttmlblend_scale_scan_batch_kernel for items[0..n) (planned): in the kernel
+ * parameters when n <= kScaleScanBatchInline, otherwise read from d_items, a device copy of them
+ * ordered before the launch on `stream`. */
+cudaError_t launch_scale_scan_batch (const ScaleScanItem *items, uint32_t n, const ScaleScanItem *d_items,
+    const int4 *plans, int2 *spans, int *groups, uint32_t rows, cudaStream_t stream);
+
 }  // namespace tb
 #endif

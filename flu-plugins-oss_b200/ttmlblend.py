@@ -102,6 +102,8 @@ PROTOTYPES = {
                                                           C.c_uint32]),
     "fluc_ttmlblend_overlay_set_positions": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(C.c_int32),
                                                        C.POINTER(C.c_int32), C.c_uint32]),
+    "fluc_ttmlblend_overlay_set_render_rectangles": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(Rect),
+                                                               C.c_uint32]),
     "fluc_ttmlblend_set_chroma_mode": (C.c_int, [C.c_void_p, C.c_int]),
     "fluc_ttmlblend_submit": (C.c_int, [C.c_void_p, C.c_uint32, C.c_int, C.c_int32, C.c_int32,
                                         C.c_uint32, C.POINTER(Frame), C.POINTER(Frame),
@@ -381,6 +383,16 @@ class TtmlBlend:
         ay = (C.c_int32 * max(1, len(yl)))(*yl)
         self._check(self.lib.fluc_ttmlblend_overlay_set_positions(self.h, stream, ax, ay, len(xl)),
                     "overlay_set_positions")
+
+    def overlay_set_render_rectangles(self, stream: int, rects: Iterable[Sequence[int]]):
+        """gst_video_overlay_rectangle_set_render_rectangle: rectangle i of the stream's
+        overlay_set_rectangles list is placed at (x, y) of rects[i] = (x, y, w, h) and rendered at
+        w x h (0: its pixel size), scaled again on the GPU from its resident pixels, without a new
+        upload. Frames submitted afterwards blend the rectangles at their new render rectangles."""
+        rl = [tuple(int(v) for v in r) for r in rects]
+        arr = (Rect * max(1, len(rl)))(*[Rect(*r) for r in rl])
+        self._check(self.lib.fluc_ttmlblend_overlay_set_render_rectangles(self.h, stream, arr, len(rl)),
+                    "overlay_set_render_rectangles")
 
     def set_chroma_mode(self, average: bool):
         """False (default): GStreamer's sited chroma, bit-exact. True: 2x2 mean, NOT bit-exact."""

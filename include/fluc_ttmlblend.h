@@ -227,7 +227,9 @@ FLUC_EXPORT int fluc_ttmlblend_overlay_update (FlucTtmlBlend *thiz, uint32_t str
 /* GstVideoOverlayComposition form: independent rectangles, blended in order. Each rectangle is
  * kept whole on the device, also the part that lies above or left of the frame (or all of it),
  * so that overlay_set_positions can move it in later: such rectangles count those pixels in
- * h2d_bytes and cache_bytes. The blended frames do not depend on it. */
+ * h2d_bytes and cache_bytes. A rectangle with another render size also keeps its pixels at their
+ * own size, so that overlay_set_render_rectangles can scale it again: cache_bytes counts them
+ * besides the scaled image. The blended frames do not depend on it. */
 FLUC_EXPORT int fluc_ttmlblend_overlay_set_rectangles (FlucTtmlBlend *thiz,
     uint32_t stream, const FlucTtmlBlendRectangle *rects, uint32_t n_rects);
 /* Region form (SURVEY.md section 8f rank 3): the overlay is composed on the GPU from region
@@ -275,7 +277,7 @@ FLUC_EXPORT int fluc_ttmlblend_overlay_set_global_alpha (FlucTtmlBlend *thiz, ui
 /* gst_video_overlay_rectangle_set_render_rectangle for the position only: rectangle i of the
  * stream's overlay_set_rectangles list (in list order, including rectangles outside the frame)
  * is placed at (x[i], y[i]). Nothing is uploaded, scaled or scanned again. The render size stays
- * the one the rectangle was installed with. Frames submitted after the call (submit*,
+ * the one the rectangle was installed with (overlay_set_render_rectangles changes it). Frames submitted after the call (submit*,
  * submit_many_after, blend_host*) are blended exactly as overlay_set_rectangles with the moved
  * rectangles would blend them. Frames already submitted keep the old positions.
  * The rectangles keep their current global alphas, and overlay_set_global_alpha after a move
@@ -289,6 +291,30 @@ FLUC_EXPORT int fluc_ttmlblend_overlay_set_global_alpha (FlucTtmlBlend *thiz, ui
  * x + render width or y + render height overflows int32_t. */
 FLUC_EXPORT int fluc_ttmlblend_overlay_set_positions (FlucTtmlBlend *thiz, uint32_t stream,
     const int32_t *x, const int32_t *y, uint32_t n);
+
+/* gst_video_overlay_rectangle_set_render_rectangle, position and size: rectangle i of the
+ * stream's overlay_set_rectangles list (in list order, as for overlay_set_positions) is placed at
+ * (render[i].x, render[i].y) and rendered at render[i].w x render[i].h; a side of 0 means the pixel
+ * size, as render_width = 0 does at install. Nothing is uploaded: a rectangle whose size changes is
+ * scaled again on the GPU from the pixels it was installed with, exactly as overlay_set_rectangles
+ * scales (or, back at its pixel size, taken as it is), and cropped again to its non-transparent
+ * rows. Frames submitted after the call (submit*, submit_many_after, blend_host*) are blended
+ * exactly as overlay_set_rectangles with the same pixels, flags and current global alphas at the
+ * new render rectangles would blend them. Frames already submitted keep the old geometry.
+ * The rectangles keep their current global alphas; overlay_set_global_alpha and
+ * overlay_set_positions after a resize keep the new sizes. Cost: every resized rectangle is scaled
+ * and scanned in one kernel launch whose row spans the call waits for (one host wait per call),
+ * then prepared as a move prepares (one launch per destination format and size the stream has been
+ * blended in; under FLUC_TTMLBLEND_CHROMA_AVERAGE, plus one per resized rectangle). An entry whose
+ * size stays and whose position changes costs what overlay_set_positions costs; nothing changed:
+ * nothing is done. Returns NOT_FOUND when the stream has no overlay (or another thread replaced it
+ * while the call waited), INVALID_ARGUMENT for a NULL array, n different from the number of
+ * rectangles installed, an overlay installed by overlay_set, overlay_update or
+ * overlay_set_regions, a side below 0 or above 32768, a rectangle that would be scaled while its
+ * pixel size is below 2x2 or above 32768 on a side, or x + w or y + h overflowing int32_t. A
+ * refused call changes nothing. */
+FLUC_EXPORT int fluc_ttmlblend_overlay_set_render_rectangles (FlucTtmlBlend *thiz, uint32_t stream,
+    const FlucTtmlBlendRect *render, uint32_t n);
 
 /* How the overlay reaches the chroma planes of 4:2:0 frames. SITED (default) is what
  * GStreamer does and the only bit-exact mode: a chroma sample takes the overlay pixel at
