@@ -18,8 +18,8 @@ HOOKS = os.path.join(graft.PKG_DIR, "csrc", "libfluc_ttmlblend_testhooks.so")
 JC_COPY, JC_ONE, JC_GENERAL, JC_ONE_BULK = 0, 1, 2, 3
 JF_VECTOR, JF_INPLACE, JF_DST_PREMUL, JF_FAST = 1, 2, 4, 8
 ITEMS_PER_CHUNK = 1024
-FMT = {"I420": 0, "NV12": 1, "AYUV": 2, "RGBA": 3, "BGRA": 4, "Y42B": 13, "Y444": 14, "YUY2": 15,
-       "GRAY8": 17, "NV16": 18, "NV24": 19}
+FMT = {"I420": 0, "NV12": 1, "AYUV": 2, "RGBA": 3, "BGRA": 4, "ARGB": 7, "Y42B": 13, "Y444": 14, "YUY2": 15,
+       "GRAY8": 17, "NV16": 18, "NV24": 19, "v308": 23, "RGB": 25}
 
 
 class HookRect(C.Structure):
@@ -37,8 +37,7 @@ class Rect(C.Structure):
     _fields_ = [("x", C.c_int32), ("y", C.c_int32), ("w", C.c_int32), ("h", C.c_int32)]
 
 
-@pytest.fixture(scope="module")
-def hooks():
+def load_hooks():
     if not os.path.exists(HOOKS):
         graft.build()
     lib = C.CDLL(HOOKS)
@@ -62,6 +61,11 @@ def hooks():
     return lib
 
 
+@pytest.fixture(scope="module")
+def hooks():
+    return load_hooks()
+
+
 def plane_geometry(fmt, W, H):
     """[(row_bytes, rows)] per plane -- restated from the format table in docs/BLENDSPEC.md."""
     cw, ch = (W + 1) // 2, (H + 1) // 2
@@ -74,8 +78,30 @@ def plane_geometry(fmt, W, H):
         "NV24": [(W, H), (2 * W, H)],
         "YUY2": [(4 * cw, H)],
         "GRAY8": [(W, H)],
-        "AYUV": [(4 * W, H)], "RGBA": [(4 * W, H)], "BGRA": [(4 * W, H)],
+        "AYUV": [(4 * W, H)], "RGBA": [(4 * W, H)], "BGRA": [(4 * W, H)], "ARGB": [(4 * W, H)],
+        "RGB": [(3 * W, H)], "v308": [(3 * W, H)],
     }[fmt]
+
+
+def plane_rects(fmt, W, H, rects):
+    """Per plane, the (v0, v1, y0, y1) span the prepare gives each pixel rectangle (x, y, w, h) of
+    the composition form, clipped to the frame: its byte columns widened to whole vectors, and for
+    the chroma planes the samples it sites (restated from prepare_rect / prepare_chroma)."""
+    bpp = {"AYUV": 4, "RGBA": 4, "BGRA": 4, "ARGB": 4, "RGB": 3, "v308": 3}
+    sub = {"I420": (2, 2), "NV12": (2, 2), "Y444": (1, 1)}
+    out = [[] for _ in plane_geometry(fmt, W, H)]
+    cdiv = lambda a, b: -(-a // b)
+    for (x, y, w, h) in rects:
+        x0, y0, x1, y1 = max(x, 0), max(y, 0), min(x + w, W), min(y + h, H)
+        b = bpp.get(fmt, 1)
+        out[0].append((b * x0 // 16, cdiv(b * x1, 16), y0, y1))
+        if fmt in sub:
+            sx, sy = sub[fmt]
+            bx0, bx1, by0, by1 = cdiv(x0, sx), cdiv(x1, sx), cdiv(y0, sy), cdiv(y1, sy)
+            e = 2 if fmt == "NV12" else 1
+            for pl in range(1, len(out)):
+                out[pl].append((e * bx0 // 16, cdiv(e * bx1, 16), by0, by1))
+    return out
 
 
 def build(hooks, fmt, W, H, rects_per_plane, windowed=False, misalign=False):
@@ -250,6 +276,136 @@ def test_random_layouts_tile_every_plane_once(hooks, seed):
         check_tiling(fmt, W, H, rects, jobs, windowed)
         if not windowed:
             assert algo == 2 * sum(rb * r for rb, r in geo)
+
+
+def pieces(jobs, plane=0):
+    return [(j.win_v0, j.win_nv, j.win_y0, j.win_rows, j.cls, j.grouped) for j in jobs if j.plane == plane]
+
+
+# Frames above 4K (tests/test_gpu_geometry.py). push_window cuts a window into pieces of at most
+# max_rows rows so that umulhi (item, magic) stays exact, and make_groupable sends a layout to the
+# table kernel when a full group of frames would not divide exactly. These pin which pieces and
+# which kernel the GPU cases reach: a change to either function shows here first.
+
+def test_8k_packed_windows_are_cut_into_1344_row_pieces(hooks):
+    rects = [(0, 200, 7680, 1500), (2000, 1600, 1200, 600)]
+    for fmt in ("RGBA", "BGRA", "AYUV", "ARGB"):
+        rr = plane_rects(fmt, 7680, 4320, rects)
+        jobs, _, cpf = build(hooks, fmt, 7680, 4320, rr, windowed=True)
+        assert pieces(jobs) == [(0, 1920, 200, 1344, JC_ONE_BULK, 1), (0, 1920, 1544, 56, JC_ONE_BULK, 1),
+                                (0, 1920, 1600, 100, JC_GENERAL, 1), (500, 300, 1700, 500, JC_ONE_BULK, 1)]
+        jobs, _, cpf = build(hooks, fmt, 7680, 4320, rr)
+        assert cpf > 0 and all(j.grouped for j in jobs)
+        assert [(j.win_y0, j.win_rows) for j in jobs if j.win_nv == 1920] == [
+            (0, 200), (200, 1344), (1544, 56), (1600, 100), (2200, 1344), (3544, 776)]
+    check_tiling("BGRA", 7680, 4320, rr, jobs, False)
+    # the same frame with the tall rectangle moved by (3, 37): the pieces start elsewhere
+    moved = plane_rects("BGRA", 7680, 4320, [(3, 237, 7680, 1500), (2000, 1600, 1200, 600)])
+    jobs, _, _ = build(hooks, "BGRA", 7680, 4320, moved, windowed=True)
+    assert pieces(jobs)[:2] == [(0, 1920, 237, 1344, JC_ONE_BULK, 1), (0, 1920, 1581, 19, JC_ONE_BULK, 1)]
+    check_tiling("BGRA", 7680, 4320, moved, jobs, True)
+
+
+def test_8k_three_byte_windows_are_cut_into_2519_row_pieces(hooks):
+    rects = [(0, 200, 7680, 2700), (2000, 2800, 1200, 600)]
+    for fmt in ("RGB", "v308"):
+        rr = plane_rects(fmt, 7680, 4320, rects)
+        jobs, _, _ = build(hooks, fmt, 7680, 4320, rr, windowed=True)
+        assert pieces(jobs) == [(0, 1440, 200, 2519, JC_ONE_BULK, 1), (0, 1440, 2719, 81, JC_ONE_BULK, 1),
+                                (0, 1440, 2800, 100, JC_GENERAL, 1), (375, 225, 2900, 500, JC_ONE_BULK, 1)]
+        # out of place the chunk count makes a full group inexact: the table kernel
+        jobs, _, cpf = build(hooks, fmt, 7680, 4320, rr)
+        assert cpf == 0 and not any(j.grouped for j in jobs) and all(j.flags & JF_FAST for j in jobs)
+        assert [(j.win_y0, j.win_rows) for j in jobs if j.win_nv == 1440][:3] == [(0, 200), (200, 2519), (2719, 81)]
+    check_tiling("RGB", 7680, 4320, rr, jobs, False)
+
+
+def test_8k_planar_windows_are_not_cut(hooks):
+    rects = [(0, 200, 7680, 1500), (2000, 1600, 1200, 600)]
+    for fmt in ("NV12", "I420"):
+        rr = plane_rects(fmt, 7680, 4320, rects)
+        for windowed in (False, True):
+            jobs, _, cpf = build(hooks, fmt, 7680, 4320, rr, windowed=windowed)
+            assert cpf > 0 and all(j.grouped for j in jobs)
+            assert (0, 480, 200, 1400, JC_ONE_BULK, 1) in pieces(jobs)
+            assert all(j.win_rows < 2500 or j.cls == JC_COPY for j in jobs)
+
+
+def test_8k_rectangle_over_the_right_and_bottom_edges(hooks):
+    rr = plane_rects("BGRA", 7680, 4320, [(300, 2820, 7600, 1600)])
+    jobs, _, cpf = build(hooks, "BGRA", 7680, 4320, rr)
+    assert cpf == 0 and pieces(jobs) == [(0, 1920, 0, 1344, JC_COPY, 0), (0, 1920, 1344, 1344, JC_COPY, 0),
+                                         (0, 1920, 2688, 132, JC_COPY, 0), (0, 75, 2820, 1500, JC_COPY, 0),
+                                         (75, 1845, 2820, 1500, JC_ONE_BULK, 0)]
+    jobs, _, cpf = build(hooks, "BGRA", 7680, 4320, rr, windowed=True)
+    assert cpf > 0 and pieces(jobs) == [(75, 1845, 2820, 1500, JC_ONE_BULK, 1)]
+
+
+@pytest.mark.parametrize("fmt,W,x,w", [("RGBA", 8192, 3000, 1500), ("Y444", 8192, 3000, 1500), ("RGB", 7680, 0, 4096)])
+def test_8k_geometries_that_fall_back_to_the_table_kernel(hooks, fmt, W, x, w):
+    rr = plane_rects(fmt, W, 4320, [(x, 1080, w, 2160)])
+    jobs, _, cpf = build(hooks, fmt, W, 4320, rr)
+    assert cpf == 0 and not any(j.grouped for j in jobs) and all(j.flags & JF_FAST for j in jobs)
+    jobs, _, cpf = build(hooks, fmt, W, 4320, rr, windowed=True)
+    assert cpf > 0 and all(j.grouped for j in jobs)              # in place they stay grouped
+
+
+def test_near_the_width_limit(hooks):
+    # 32764 BGRA: 8191 vectors a row, 64-row pieces; 13 under rows 102-921. Out of place group bands,
+    # in place (fewer chunks a frame) the table kernel
+    rr = plane_rects("BGRA", 32764, 1024, [(0, 102, 32764, 819)])
+    jobs, _, cpf = build(hooks, "BGRA", 32764, 1024, rr)
+    under = [p for p in pieces(jobs) if p[4] == JC_ONE_BULK]
+    assert cpf > 0 and all(j.grouped for j in jobs) and len(under) == 13
+    assert [p[2:4] for p in under] == [(102 + 64 * k, 64) for k in range(12)] + [(870, 51)]
+    jobs, _, cpf = build(hooks, "BGRA", 32764, 1024, rr, windowed=True)
+    assert cpf == 0 and [p[2:] for p in pieces(jobs)] == [(102 + 64 * k, 64, JC_ONE_BULK, 0) for k in range(12)] + [
+        (870, 51, JC_ONE_BULK, 0)]
+    # 32764 AYUV under rows 102-358: four pieces, grouped both ways
+    rr = plane_rects("AYUV", 32764, 1024, [(0, 102, 32764, 256)])
+    for windowed in (False, True):
+        jobs, _, cpf = build(hooks, "AYUV", 32764, 1024, rr, windowed=windowed)
+        assert cpf > 0 and [p[2:4] for p in pieces(jobs) if p[4] == JC_ONE_BULK] == [(102, 64), (166, 64), (230, 64), (294, 64)]
+    # 32767 wide: 2047 whole vectors and a 15-byte tail column for the byte kernel
+    for fmt in ("GRAY8", "I420"):
+        rr = plane_rects(fmt, 32767, 512, [(0, 100, 32767, 300)])
+        for windowed in (False, True):
+            jobs, _, cpf = build(hooks, fmt, 32767, 512, rr, windowed=windowed)
+            tail = [j for j in jobs if j.win_v0 == 2047]
+            assert cpf > 0 and tail and all(j.plane == 0 and j.win_nv == 1 and not j.grouped and not (j.flags & JF_FAST)
+                                            for j in tail)
+            assert all(j.grouped for j in jobs if j.win_v0 != 2047)
+    # 15360 RGBA: 3840 vectors a row, 312-row pieces; out of place the table kernel
+    rr = plane_rects("RGBA", 15360, 8640, [(0, 2000, 15360, 1000)])
+    jobs, _, cpf = build(hooks, "RGBA", 15360, 8640, rr)
+    assert cpf == 0 and [p[2:4] for p in pieces(jobs) if p[4] == JC_ONE_BULK] == [(2000, 312), (2312, 312), (2624, 312), (2936, 64)]
+    jobs, _, cpf = build(hooks, "RGBA", 15360, 8640, rr, windowed=True)
+    assert cpf > 0 and [p[2:4] for p in pieces(jobs)] == [(2000, 312), (2312, 312), (2624, 312), (2936, 64)]
+    rr = plane_rects("RGBA", 15360, 8640, [(0, 2000, 15360, 4320)])
+    jobs, _, cpf = build(hooks, "RGBA", 15360, 8640, rr, windowed=True)
+    assert cpf == 0 and len(jobs) == 14
+
+
+@pytest.mark.parametrize("fmt,W,H,rects", [
+    ("BGRA", 7680, 4320, [(0, 200, 7680, 1500), (2000, 1600, 1200, 600)]),
+    ("RGB", 7680, 4320, [(0, 200, 7680, 2700), (2000, 2800, 1200, 600)]),
+    ("RGBA", 15360, 8640, [(0, 2000, 15360, 1000), (5000, 1500, 3000, 3000)]),
+    ("BGRA", 32764, 2048, [(0, 102, 32764, 1024), (100, 1500, 200, 300)]),
+])
+def test_large_frames_tile_and_divide_exactly(hooks, fmt, W, H, rects):
+    """check_tiling (every window once, classes, the umulhi probe over each window's items) on the
+    geometries above 4K; its cover arrays are too large at 32768 x 32768."""
+    rr = plane_rects(fmt, W, H, rects)
+    for windowed in (False, True):
+        jobs, _, _ = build(hooks, fmt, W, H, rr, windowed=windowed)
+        assert any(j.win_rows == max_rows_of(j.win_nv) for j in jobs)
+        check_tiling(fmt, W, H, rr, jobs, windowed)
+
+
+def max_rows_of(nv):
+    magic = ((1 << 32) + nv - 1) // nv
+    e = magic * nv - (1 << 32)
+    return max(1, min(min(((1 << 32) - 1) // e if e else 1 << 31, 1 << 31) // nv, 1 << 30))
 
 
 # ---------------------------------------------------------------------------------------------

@@ -2,7 +2,7 @@
 # Runs the parity tests with every alternative code path forced through its environment knob:
 # table kernel only, no multi-layout launches, in-place launches always / never lazy, no
 # auto-crop, register-staged instead of TMA-staged overlay, interleaved chunk order, and the
-# host-frame knobs; then the global-alpha, move, resize and operator-domain files under each knob. Every line
+# host-frame knobs; then the global-alpha, move, resize, geometry and operator-domain files under each knob. Every line
 # must end in "passed".
 #   gpurun -- bash tools/knob_matrix.sh
 K="rectangles_match_oracle or golden or fuzz or alpha_sweep or scaled_rectangles or regions or unaligned or chain or ping_pong or dependency or two_overlays or update or sparse_cues or host_path or host_dma"
@@ -22,4 +22,6 @@ for v in FLUC_TTMLBLEND_GROUPS=0 FLUC_TTMLBLEND_MULTI=0 FLUC_TTMLBLEND_LAZY=1 FL
   env $v timeout 600 python -m pytest tests/test_gpu_move.py -q -x 2>&1 | tail -1
   # overlay_set_render_rectangles (scale-and-scan batch, crop and lazy figures of the resized rectangles)
   env $v timeout 600 python -m pytest tests/test_gpu_resize.py -q -x 2>&1 | tail -1
+  # frames above 4K up to 32768 wide: row-split windows, table-kernel fallbacks, offsets past 4 GiB
+  env $v timeout 600 python -m pytest tests/test_gpu_geometry.py -q -x 2>&1 | tail -1
 done
